@@ -13,8 +13,13 @@ single-threaded) on a bounded sample; `configs` = every configuration of BASELIN
 own after the headline step (CUDA events, median of a few launches), sharded over the ranks with their
 collectives at N > 1.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the last timed step returned, so that two builds can be compared output for output on
+identical inputs: DIR/prox_l0box.npy, prox_lhalfbox.npy, iprox_l0box.npy (Float64; above 2^21 elements a fixed,
+seeded sample of up to 2^21 positions, the same in every run; at N > 1 one file per rank with a `_rank<r>` suffix,
+each sampling its own shard with 2^21 / N draws) and psi_prox_l0box.npy (the fused ψ(y), all-reduced at N > 1).
 """
 from __future__ import annotations
 
@@ -52,7 +57,12 @@ def parse():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
     ap.add_argument("--config-reps", type=int, default=5)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (see the module docstring)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def measured_peak():
@@ -178,7 +188,7 @@ def run_reference(args, rank):
         return
     from concurrent.futures import ThreadPoolExecutor
 
-    steps, warm = max(1, args.steps), args.warmup
+    steps, warm = args.steps, args.warmup
     cores = max(1, len(os.sched_getaffinity(0)))
     # each step = a bounded sample of the workload; keep the whole run within a few minutes
     n = 1 << 20
@@ -283,6 +293,29 @@ class ClockSampler(threading.Thread):
 
 
 # ------------------------------------------------------------------- GPU arm ---
+DUMP_SAMPLE = 1 << 21  # elements per operation over all ranks: 3 x 16 MiB of Float64
+
+
+def dump_outputs(dirname, outs, psi_val, rank, world):
+    """--dump-outputs: the three result vectors of the step (a fixed, seeded sample of positions when larger than
+    DUMP_SAMPLE / world) and the fused ψ(y), as .npy files in DIR."""
+    import numpy as np
+    import torch
+
+    os.makedirs(dirname, exist_ok=True)
+    n, m = outs[0].numel(), DUMP_SAMPLE // world
+    idx = None
+    if n > m:
+        idx = np.unique(np.random.default_rng(SEED).integers(0, n, m))
+        idx = torch.from_numpy(idx).to(outs[0].device)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, t in zip(OPS, outs):
+        a = t if idx is None else t.index_select(0, idx)
+        np.save(os.path.join(dirname, f"{name}{suffix}.npy"), a.cpu().numpy())
+    if rank == 0:
+        np.save(os.path.join(dirname, "psi_prox_l0box.npy"), np.array([psi_val], dtype=np.float64))
+
+
 def run_ours(args, rank, local_rank, world):
     import torch
 
@@ -326,28 +359,33 @@ def run_ours(args, rank, local_rank, world):
         shd.comm_init(dev)
         shd.reduce_scalars(True, dev)
 
-    def step(ev=None):
+    def step(ev=None, outs=(y, y, y)):
+        """One C2 step; the three results go to outs (one vector per operation) and the fused ψ(y) is returned."""
         if ev is not None:
             ev[0].record()
-        sp.prox_(y, psi_l0, q, SIGMA, want_value=True)  # fused ψ(y) (+ all-reduce of its scalar at N > 1)
+        _, psi_val = sp.prox_(outs[0], psi_l0, q, SIGMA, want_value=True)  # fused ψ(y) (+ all-reduce at N > 1)
         if ev is not None:
             ev[1].record()
-        sp.prox_(y, psi_lh, q, SIGMA)
+        sp.prox_(outs[1], psi_lh, q, SIGMA)
         if ev is not None:
             ev[2].record()
-        sp.iprox_(y, psi_l0, q, d)
+        sp.iprox_(outs[2], psi_l0, q, d)
         if ev is not None:
             ev[3].record()
+        return psi_val
 
     def barrier():
         if dist is not None:
             dist.barrier()
         torch.cuda.synchronize()
 
-    K, W = max(1, args.steps), max(3, args.warmup)
+    K, W = args.steps, max(3, args.warmup)
     for _ in range(W):
         step()
     barrier()
+    # every operation writes all of its output vector either way, so keeping the three results apart for
+    # --dump-outputs moves the same bytes as overwriting one vector
+    outs = (y, torch.empty_like(y), torch.empty_like(y)) if args.dump_outputs else (y, y, y)
     evs = [[torch.cuda.Event(enable_timing=True) for _ in range(4)] for _ in range(K)]
     sampler = ClockSampler(local_rank)
     sampler.start()
@@ -357,7 +395,7 @@ def run_ours(args, rank, local_rank, world):
     t_end = torch.cuda.Event(enable_timing=True)
     t_start.record()
     for k in range(K):
-        step(evs[k])
+        psi_val = step(evs[k], outs)
     t_end.record()
     # the K steps are queued and the GPU is still working through them: a few samples from this thread as well (on
     # some boxes the sampler thread gets a single NVML answer during a 140 ms region)
@@ -367,6 +405,9 @@ def run_ours(args, rank, local_rank, world):
     launches = sp.launch_count(dev) - launches0
     collectives = shd.comm_info(dev)[2] if world > 1 else 0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs, psi_val, rank, world)
+    del outs
     ms_total = t_start.elapsed_time(t_end)
     per_op_ms = {op: sum(evs[k][i].elapsed_time(evs[k][i + 1]) for k in range(K)) / K for i, op in enumerate(OPS)}
     if dist is not None:

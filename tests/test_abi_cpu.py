@@ -4,6 +4,7 @@ refuses to compute without one (no CPU fallback)."""
 import ctypes
 import os
 import re
+import shutil
 import subprocess
 
 import pytest
@@ -11,6 +12,8 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEADER = os.path.join(ROOT, "include", "shiftedprox.h")
 LIB = os.path.join(ROOT, "shiftedproximaloperators.jl_b200", "libshiftedprox.so")
+# the toolkit's bin directory need not be on PATH: the build itself calls nvcc by this location (csrc/Makefile)
+CUOBJDUMP = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
 
 
 def declared_symbols():
@@ -61,7 +64,7 @@ def test_version_and_scalar_helpers(lib):
 
 
 def test_library_is_sm100a_only():
-    out = subprocess.run(["cuobjdump", "--list-elf", LIB], capture_output=True, text=True).stdout
+    out = subprocess.run([CUOBJDUMP, "--list-elf", LIB], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs
 
@@ -110,20 +113,16 @@ def test_group_index_sets_must_be_contiguous_ranges():
 def test_library_holds_only_sm_100a_code_and_the_bulk_copy_kernels_use_tma():
     """The shipped library is sm_100a-only (no PTX fallback, no other architecture), and the CTA-per-group kernels of
     spx_group.cu stage their groups with bulk copies (UBLKCP in the SASS: cp.async.bulk completing on an mbarrier) --
-    checked on the built artefacts with cuobjdump (skipped when the toolkit is not on PATH)."""
-    import shutil
-    import subprocess
-
-    cuobjdump = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
-    if not os.path.exists(cuobjdump):
+    checked on the built artefacts with cuobjdump (skipped when the toolkit has none)."""
+    if not os.path.exists(CUOBJDUMP):
         pytest.skip("cuobjdump not available")
     pkg = os.path.join(ROOT, "shiftedproximaloperators.jl_b200")
-    elfs = subprocess.run([cuobjdump, "-lelf", os.path.join(pkg, "libshiftedprox.so")], capture_output=True, text=True).stdout
+    elfs = subprocess.run([CUOBJDUMP, "-lelf", os.path.join(pkg, "libshiftedprox.so")], capture_output=True, text=True).stdout
     names = [ln.split(":")[-1].strip() for ln in elfs.splitlines() if "ELF file" in ln]
     assert names and all(n.endswith(".sm_100a.cubin") for n in names), names
-    ptx = subprocess.run([cuobjdump, "-lptx", os.path.join(pkg, "libshiftedprox.so")], capture_output=True, text=True).stdout
+    ptx = subprocess.run([CUOBJDUMP, "-lptx", os.path.join(pkg, "libshiftedprox.so")], capture_output=True, text=True).stdout
     assert "PTX file" not in ptx
     obj = os.path.join(pkg, "csrc", "build", "spx_group.o")
     if os.path.exists(obj):
-        sass = subprocess.run([cuobjdump, "-sass", obj], capture_output=True, text=True).stdout
+        sass = subprocess.run([CUOBJDUMP, "-sass", obj], capture_output=True, text=True).stdout
         assert sass.count("UBLKCP") > 0 and "SYNCS" in sass  # bulk copy + mbarrier
