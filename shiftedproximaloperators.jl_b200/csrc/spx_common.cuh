@@ -210,6 +210,54 @@ __device__ __forceinline__ void st_stream(float* p, const Pack<float, 1>& o) {
   asm volatile("st.global.cs.f32 [%0], %1;" ::"l"(p), "f"(o.v[0]) : "memory");
 }
 
+// ------------------------------------------------- asynchronous copies to shared memory --
+// Per-thread 16-byte cp.async (LDGSTS), completed by cp.async.wait_group, and 16-byte shared loads.
+__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N> __device__ __forceinline__ void cp_async_wait() {
+  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
+}
+__device__ __forceinline__ void lds16(uint32_t a, Pack<double, 2>& o) {
+  asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(o.v[0]), "=d"(o.v[1]) : "r"(a) : "memory");
+}
+__device__ __forceinline__ void lds16(uint32_t a, Pack<float, 4>& o) {
+  asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];"
+               : "=f"(o.v[0]), "=f"(o.v[1]), "=f"(o.v[2]), "=f"(o.v[3])
+               : "r"(a)
+               : "memory");
+}
+
+// Bulk copies (cp.async.bulk, UBLKCP): one thread moves a contiguous run of 16-byte granules global -> shared, and
+// the copy completes on an mbarrier (expect_tx / complete_tx): no LSU instructions, no registers, any thread of the
+// CTA may read the run once the barrier's phase flips.
+__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
+  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
+  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+}
+__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
+  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
+               "l"(src), "r"(bytes), "r"(smem_u32(bar))
+               : "memory");
+}
+__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\tSPX_MBAR_WAIT:\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t@p bra SPX_MBAR_DONE;\n\t"
+      "bra SPX_MBAR_WAIT;\n\tSPX_MBAR_DONE:\n\t}" ::"r"(smem_u32(bar)),
+      "r"(parity)
+      : "memory");
+}
+// orders the CTA's earlier generic-proxy reads of a buffer before the async-proxy writes of the next bulk copy into it
+__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+
 // --------------------------------------------------------------- reductions --
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll

@@ -96,122 +96,19 @@ __global__ void __launch_bounds__(kEwThreads, MinBlocks<Op>::value)
   }
 }
 
-// ---------------------------------------------------------------- pipelined form --
-// Operators whose arithmetic is heavy enough that a warp spends as long computing as waiting (the
-// RootNormLhalfBox prox!, the Box iprox!) leave HBM idle in the form above: nothing is in flight for
-// a warp while it computes, and registers (the occupancy limit) are what bounds the loads in flight.
-// Here every thread keeps STAGES-1 tiles of ITS OWN operands in flight with 16-byte
-// cp.async.cg (LDGSTS, L1-bypassing) into a private shared-memory slot, and reads the slot back
-// after cp.async.wait_group: no barrier of any kind (a thread only ever reads what it copied), no
-// registers held by the prefetched tiles.  Shared memory per CTA = STAGES x NIN x 4 KiB.
-template <class Op, class = void> struct Stages { static constexpr int value = 0; };
-template <class Op> struct Stages<Op, std::void_t<decltype(Op::STAGES)>> { static constexpr int value = Op::STAGES; };
-
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
-__device__ __forceinline__ void lds16(uint32_t a, Pack<double, 2>& o) {
-  asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(o.v[0]), "=d"(o.v[1]) : "r"(a) : "memory");
-}
-__device__ __forceinline__ void lds16(uint32_t a, Pack<float, 4>& o) {
-  asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];"
-               : "=f"(o.v[0]), "=f"(o.v[1]), "=f"(o.v[2]), "=f"(o.v[3])
-               : "r"(a)
-               : "memory");
-}
-
-template <int VEC, class Op>
-__global__ void __launch_bounds__(kEwThreads, MinBlocks<Op>::value)
-    ew_pipe_kernel(const Op op, const long long n, const long long index_base, Partial* __restrict__ partials) {
-  using R = typename Op::Real;
-  constexpr int NIN = Op::NIN;
-  constexpr int ST = Stages<Op>::value;
-  static_assert(sizeof(R) * VEC == 16 && ST >= 2, "pipelined form moves 16-byte packets");
-  extern __shared__ __align__(16) unsigned char ew_smem[];
-  Partial acc;
-  acc.s = 0.0;
-  acc.s2 = 0.0;
-  acc.bad = -1;
-
-  const long long nvec = n / VEC;
-  const long long stride = (long long)gridDim.x * kEwThreads;
-  const uint32_t slot0 = (uint32_t)__cvta_generic_to_shared(ew_smem) + threadIdx.x * 16u;
-  constexpr uint32_t kPlane = kEwThreads * 16u;  // one operand of one stage
-  auto issue = [&](long long v, int stage) {
-    if (v < nvec) {
-#pragma unroll
-      for (int k = 0; k < NIN; ++k)
-        if (op.in[k] != nullptr) cp_async16(slot0 + (uint32_t)(stage * NIN + k) * kPlane, op.in[k] + v * VEC);
-    }
-    cp_async_commit();
-  };
-  long long v = (long long)blockIdx.x * kEwThreads + threadIdx.x;
-#pragma unroll
-  for (int s = 0; s < ST - 1; ++s) issue(v + s * stride, s);
-  int stage = 0;
-  for (long long base = (long long)blockIdx.x * kEwThreads; base < nvec; base += stride) {
-    int ahead = stage + (ST - 1);
-    ahead = ahead >= ST ? ahead - ST : ahead;
-    issue(v + (ST - 1) * stride, ahead);
-    cp_async_wait<ST - 1>();
-    if (v < nvec) {
-      Pack<R, VEC> reg[NIN];
-#pragma unroll
-      for (int k = 0; k < NIN; ++k) {
-        if (op.in[k] != nullptr) {
-          lds16(slot0 + (uint32_t)(stage * NIN + k) * kPlane, reg[k]);
-        } else {
-#pragma unroll
-          for (int e = 0; e < VEC; ++e) reg[k].v[e] = op.fill[k];
-        }
-      }
-      Pack<R, VEC> out;
-#pragma unroll
-      for (int e = 0; e < VEC; ++e) {
-        R x[NIN];
-#pragma unroll
-        for (int k = 0; k < NIN; ++k) x[k] = reg[k].v[e];
-        out.v[e] = op.apply(x, index_base + v * VEC + e, acc);
-      }
-      if (Op::OUT) st_stream(op.y + v * VEC, out);
-    }
-    v += stride;
-    stage = stage + 1 == ST ? 0 : stage + 1;
-  }
-  cp_async_wait<0>();
-  // scalar tail (n not a multiple of VEC): the last block's first threads
-  if (blockIdx.x == gridDim.x - 1) {
-    const long long i = nvec * VEC + threadIdx.x;
-    if (i < n) {
-      R x[NIN];
-#pragma unroll
-      for (int k = 0; k < NIN; ++k) x[k] = op.in[k] != nullptr ? op.in[k][i] : op.fill[k];
-      R o = op.apply(x, index_base + i, acc);
-      if (Op::OUT) op.y[i] = o;
-    }
-  }
-  if (Op::ACC) {
-    acc = block_fold<kEwThreads>(acc);
-    if (threadIdx.x == 0) partials[blockIdx.x] = acc;
-  }
-}
-
-template <int VEC, class Op> inline int ew_pipe_blocks_per_sm(size_t smem) {
-  static int cached = 0;  // per instantiation
-  if (cached == 0) {
-    int nb = 0;
-    cudaFuncSetAttribute(ew_pipe_kernel<VEC, Op>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, ew_pipe_kernel<VEC, Op>, kEwThreads, smem) != cudaSuccess ||
-        nb < 1)
-      nb = 1;
-    cached = nb;
-  }
-  return cached;
-}
+// ------------------------------------------------------------------ bulk-copy ring --
+// Operators that declare `static constexpr bool BULK = true` stream their operands through ew_bulk_kernel (spx_bulk.cuh)
+// when every operand is a 16-byte-aligned vector and n >= SPX_EWB_MIN_N.  The kernel and its launches live in their own
+// translation unit, spx_bulk.cu, which instantiates ew_bulk_launch for those operators: its dynamic shared memory
+// (`extern __shared__`) makes nvcc reserve 1 KiB of static shared memory in every kernel of the module it is in.
+#ifndef SPX_EWB_MIN_N
+#define SPX_EWB_MIN_N (1 << 20)  // elements: where the ring starts to beat ew_kernel (profiles/README.md, round 3)
+#endif
+template <class Op, class = void> struct Bulk { static constexpr bool value = false; };
+template <class Op> struct Bulk<Op, std::void_t<decltype(Op::BULK)>> { static constexpr bool value = Op::BULK; };
+template <class Op>
+int32_t ew_bulk_launch(spx_ctx* ctx, cudaStream_t stream, const Op& op, int64_t n, int64_t index_base, Partial* partials,
+                       int* nblocks_out);
 
 template <class Op> inline bool aligned16(const Op& op) {
   uintptr_t bits = 0;
@@ -253,22 +150,9 @@ int32_t ew_launch(spx_ctx* ctx, cudaStream_t stream, const Op& op, int64_t n, in
   if (nblocks_out) *nblocks_out = 0;
   if (n <= 0) return SPX_OK;
   const bool vec = aligned16(op);
-  if constexpr (Stages<Op>::value >= 2) {
-    if (vec) {
-      const size_t smem = (size_t)Stages<Op>::value * Op::NIN * kEwThreads * 16;
-      const long long nv = n / VECW;
-      long long want = (nv + kEwThreads - 1) / kEwThreads;
-      if (want < 1) want = 1;
-      long long cap = (long long)ctx->sm_count * ew_pipe_blocks_per_sm<VECW, Op>(smem);
-      if (cap > kMaxPartials) cap = kMaxPartials;
-      const int grid = (int)(want < cap ? want : cap);
-      ew_pipe_kernel<VECW, Op><<<grid, kEwThreads, smem, stream>>>(op, n, index_base, partials);
-      ctx->launches++;
-      if (nblocks_out) *nblocks_out = grid;
-      cudaError_t e = cudaGetLastError();
-      if (e != cudaSuccess) return cuda_fail(e, "ew_pipe_kernel launch");
-      return SPX_OK;
-    }
+  if constexpr (Bulk<Op>::value) {
+    if (vec && n >= SPX_EWB_MIN_N && leading_vectors(op) == Op::NIN)
+      return ew_bulk_launch(ctx, stream, op, n, index_base, partials, nblocks_out);
   }
   const long long nvec = vec ? n / VECW : n;
   const long long tile = (long long)kEwThreads * UNROLL;

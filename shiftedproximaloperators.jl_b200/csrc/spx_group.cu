@@ -393,30 +393,7 @@ __device__ __forceinline__ void stage_group_async(R* stage, const R* q, const R*
 // aligned addresses and sizes while a group starts on an element boundary: the copy starts at the 16-byte granule that
 // holds the first element and ends with the granule that holds the last one (the few neighbouring bytes of the same
 // granules are read and ignored -- a granule that holds a valid byte lies in the same page); `skip` elements of
-// padding result at the front of each plane, per operand.
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
-               "l"(src), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tSPX_MBAR_WAIT:\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t@p bra SPX_MBAR_DONE;\n\t"
-      "bra SPX_MBAR_WAIT;\n\tSPX_MBAR_DONE:\n\t}" ::"r"(smem_u32(bar)),
-      "r"(parity)
-      : "memory");
-}
-// orders the CTA's earlier generic-proxy reads of the planes before the async-proxy writes of the next bulk copy
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
+// padding result at the front of each plane, per operand.  The copy primitives (bulk_g2s, mbar_*) are in spx_common.cuh.
 template <class R> __device__ __forceinline__ int bulk_skip(const R* p) {  // elements of front padding in the plane
   return (int)(((uintptr_t)p & 15u) / sizeof(R));
 }
