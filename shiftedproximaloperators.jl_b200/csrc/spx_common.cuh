@@ -65,7 +65,8 @@ struct spx_ctx {
   cudaStream_t pipe_streams[3] = {nullptr, nullptr, nullptr};
   void* pipe_buf = nullptr;
   size_t pipe_bytes = 0;
-  cudaEvent_t pipe_events[16] = {};
+  // fork / join of side streams 0 and 1 by the group kernels (spx_group.cu): lazily created
+  cudaEvent_t pipe_events[3] = {};
   long long launches = 0;
   // multi-GPU (spx_comm.cu): an NCCL communicator bound to this context's device and stream
   void* comm = nullptr;  // ncclComm_t

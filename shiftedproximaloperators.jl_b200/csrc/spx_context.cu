@@ -306,8 +306,8 @@ int32_t spx_ctx_destroy(spx_ctx* c) {
   cudaStreamSynchronize(c->stream);
   for (int i = 0; i < 3; ++i)
     if (c->pipe_streams[i]) cudaStreamDestroy(c->pipe_streams[i]);
-  for (int i = 0; i < 16; ++i)
-    if (c->pipe_events[i]) cudaEventDestroy(c->pipe_events[i]);
+  for (cudaEvent_t ev : c->pipe_events)
+    if (ev) cudaEventDestroy(ev);
   if (c->pipe_buf) cudaFree(c->pipe_buf);
   if (c->d_scratch) cudaFree(c->d_scratch);
   spx_comm_peer_detach(c);

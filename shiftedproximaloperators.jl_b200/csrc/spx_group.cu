@@ -11,6 +11,7 @@
 // and the deeply batched loads a lone warp needs to hide latency do not share one register budget.  Sums of squares are accumulated in Float64 whatever R is; the butterfly order is fixed, so
 // results are deterministic.
 #include <algorithm>
+#include <cstddef>
 #include <cstdlib>
 
 #include "spx_elementwise.cuh"
@@ -107,14 +108,12 @@ __device__ __forceinline__ double sub_sum(double v, int L) {
 
 // Next task of a warp: round-robin (deterministic: required when ψ(y) partial sums ride along), or, when the
 // tasks are very unequal and heavy (the Binf root search on long groups) and nothing order-dependent is
-// accumulated, from a global counter in chunks of kTaskChunk consecutive tasks (one atomic per chunk).
-constexpr int kTaskChunk = 1;
+// accumulated, one task at a time from a global counter.
 __device__ __forceinline__ long long next_task(long long cur, long long nwarps, unsigned long long* counter,
                                                int lane) {
   if (counter == nullptr) return cur + nwarps;
-  if (cur >= 0 && ((cur + 1) % kTaskChunk) != 0) return cur + 1;  // still inside the claimed chunk
   unsigned long long t = 0;
-  if (lane == 0) t = atomicAdd(counter, (unsigned long long)kTaskChunk);
+  if (lane == 0) t = atomicAdd(counter, 1ull);
   return (long long)__shfl_sync(0xffffffffu, t, 0);
 }
 
@@ -358,35 +357,6 @@ __device__ __forceinline__ void prefetch_group_l2(const R* p0, const R* p1, cons
   }
 }
 
-// one element (8 or 4 bytes) global -> shared, asynchronously: group starts are only element-aligned
-template <class R> __device__ __forceinline__ void cp_async_elem(uint32_t dst, const R* src) {
-  if (sizeof(R) == 8)
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(dst), "l"(src) : "memory");
-  else
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src) : "memory");
-}
-// the CTA's copy of group [b, e) into the staging planes (thread t: elements b + t, b + T + t, ... into slots t, T + t,
-// ...: its own slots, which only it reads back, so cp.async.wait_group is the only synchronisation).  NP planes of PL
-// elements: q | xk | sj
-template <class R, int T, int EMAX, int PL, int NP>
-__device__ __forceinline__ void stage_group_async(R* stage, const R* q, const R* xk, const R* sj, long long b, long long e) {
-  const int t = threadIdx.x;
-  const uint32_t a0 = (uint32_t)__cvta_generic_to_shared(stage + t);
-#pragma unroll
-  for (int k = 0; k < EMAX; ++k) {
-    const long long i = b + (long long)k * T + t;
-    if (i < e) {
-      const uint32_t o = a0 + (uint32_t)(k * T * (int)sizeof(R));
-      cp_async_elem<R>(o, q + i);
-      if (NP > 1) {
-        cp_async_elem<R>(o + (uint32_t)(PL * (int)sizeof(R)), xk + i);
-        cp_async_elem<R>(o + (uint32_t)(2 * PL * (int)sizeof(R)), sj + i);
-      }
-    }
-  }
-  cp_async_commit();
-}
-
 // ---- TMA bulk copies (cp.async.bulk, one elected thread) for the CTA-per-group classes -------------------------------
 // A group is a contiguous run of each operand vector, so one thread moves it with three bulk copies that complete on an
 // mbarrier: no LSU instructions, no registers, any thread may read any element afterwards.  Bulk copies want 16-byte
@@ -440,13 +410,62 @@ __device__ __forceinline__ int list_class_groups(const long long* __restrict__ o
   return total;
 }
 
+// ST staging buffers of NP planes (PLS elements each) that take a chunk's listed groups in list order: listed group j
+// lands in buffer j % ST, and thread 0 refills that buffer with group j + ST once every thread holds group j.  `bar`
+// (ST mbarriers) and `buf` are the kernel's shared memory; the constructor initialises the mbarriers.
+template <class R, int NP, int PLS, int ST> struct StageRing {
+  uint64_t* bar;
+  R* buf;
+  uint32_t phases;  // bit s: the parity buffer s completes next
+  int cur;          // the buffer `wait` returned last
+  __device__ __forceinline__ StageRing(uint64_t* bar_, R* buf_) : bar(bar_), buf(buf_) {
+    if (threadIdx.x == 0)
+      for (int s = 0; s < ST; ++s) mbar_init(&bar[s], 1);
+    __syncthreads();
+    phases = 0;
+  }
+  // thread 0: the copies of the first ST listed groups
+  __device__ __forceinline__ void prime(const int* list, int nlisted, long long g0, const long long* __restrict__ offs,
+                                        const R* p0, const R* p1, const R* p2) {
+    if (threadIdx.x != 0) return;
+    fence_proxy_async();
+    for (int s = 0; s < ST && s < nlisted; ++s) {
+      const long long g = g0 + list[s];
+      stage_group_bulk<R, NP, PLS>(buf + s * NP * PLS, &bar[s], p0, p1, p2, offs[g], offs[g + 1]);
+    }
+  }
+  // the planes of listed group j, once its copies have landed
+  __device__ __forceinline__ R* wait(int j) {
+    cur = j % ST;
+    mbar_wait(&bar[cur], (phases >> cur) & 1u);
+    phases ^= 1u << cur;
+    return buf + cur * NP * PLS;
+  }
+  // [b, e) of listed group j + ST; false when the list ends before it
+  __device__ __forceinline__ bool ahead(const int* list, int nlisted, int j, long long g0,
+                                        const long long* __restrict__ offs, long long& b, long long& e) const {
+    if (j + ST >= nlisted) return false;
+    const long long g = g0 + list[j + ST];
+    b = offs[g];
+    e = offs[g + 1];
+    return true;
+  }
+  // thread 0, once every thread holds the group `wait` returned: its buffer takes group [b, e) (the one `ahead` gave)
+  __device__ __forceinline__ void refill(const R* p0, const R* p1, const R* p2, long long b, long long e) {
+    fence_proxy_async();
+    stage_group_bulk<R, NP, PLS>(buf + cur * NP * PLS, &bar[cur], p0, p1, p2, b, e);
+  }
+};
+
 // one group of a CTA-per-group class, E elements per thread (E T >= m); returns the group's ψ term.  The group has
-// been bulk-copied into staging buffer `stage`; once every thread holds its elements in registers (the barrier of the
-// first block sum) thread 0 refills the buffer with the group ST places further down the list, so that group's HBM
-// latency is spent under the work on the ST - 1 groups in between (ST = 1: under this group's scaling and stores).
-template <class R, bool PSI, bool SHIFTED, int E, int T, int PLS>
+// been bulk-copied into `stage`, the buffer of `ring` waited on last; once every thread holds its elements in registers (the
+// barrier of the first block sum) thread 0 refills the buffer with [nb, ne), the group ST places further down the list,
+// so that group's HBM latency is spent under the work on the ST - 1 groups in between (ST = 1: under this group's
+// scaling and stores).
+template <class R, bool PSI, bool SHIFTED, int E, int T, int PLS, class Ring>
 __device__ __forceinline__ double l2_big_group(R* y, const R* xk, const R* sj, const R* q, long long b, long long e, R lam,
-                                               R sigma, double* red, R* stage, uint64_t* bar, long long nb, long long ne) {
+                                               R sigma, double* red, const R* stage, Ring& ring, long long nb,
+                                               long long ne) {
   const int t = threadIdx.x;
   R sol[E], xs[E];
   double ss = 0.0;
@@ -466,10 +485,7 @@ __device__ __forceinline__ double l2_big_group(R* y, const R* xk, const R* sj, c
     }
   }
   ss = block_sum<T>(ss, red);
-  if (t == 0 && ne > nb) {
-    fence_proxy_async();
-    stage_group_bulk<R, SHIFTED ? 3 : 1, PLS>(stage, bar, q, xk, sj, nb, ne);
-  }
+  if (t == 0 && ne > nb) ring.refill(q, xk, sj, nb, ne);
   const R snorm = (R)sqrt(ss);
   const R alpha = jl_max(R(1) - sigma * lam / snorm, R(0));
   double vv = 0.0;
@@ -503,41 +519,24 @@ __global__ void __launch_bounds__(T, (sizeof(R) == 4 ? 3 : 2) * 256 / T)
   __shared__ double red[T / 32];
   __shared__ __align__(8) uint64_t bar[ST];
   extern __shared__ __align__(128) unsigned char l2_stage_raw[];
-  R* const stage0 = reinterpret_cast<R*>(l2_stage_raw);  // ST buffers of q | xk | sj, PLS elements each
   const int t = threadIdx.x;
-  if (t == 0)
-    for (int s = 0; s < ST; ++s) mbar_init(&bar[s], 1);
-  __syncthreads();
-  uint32_t phases = 0;  // bit s: the parity buffer s completes next
+  StageRing<R, NP, PLS, ST> ring(bar, reinterpret_cast<R*>(l2_stage_raw));  // q | xk | sj
   double psi = 0.0;
   for (long long g0 = (long long)blockIdx.x * T; g0 < ngroups; g0 += (long long)gridDim.x * T) {
     const int nbig = list_class_groups<T, LO, EB * T>(offs, g0, ngroups, list, wcount);
-    if (t == 0) {
-      fence_proxy_async();
-      for (int s = 0; s < ST && s < nbig; ++s) {
-        const long long gf = g0 + list[s];
-        stage_group_bulk<R, NP, PLS>(stage0 + s * NP * PLS, &bar[s], q, xk, sj, offs[gf], offs[gf + 1]);
-      }
-    }
+    ring.prime(list, nbig, g0, offs, q, xk, sj);
     for (int j = 0; j < nbig; ++j) {
-      const int sidx = j % ST;
       const long long g = g0 + list[j];
       const long long b = offs[g], e = offs[g + 1];
       const R lam = lambda_g[g];
       long long nb = 0, ne = 0;
-      if (j + ST < nbig) {
-        const long long gn = g0 + list[j + ST];
-        nb = offs[gn];
-        ne = offs[gn + 1];
-      }
-      mbar_wait(&bar[sidx], (phases >> sidx) & 1u);
-      phases ^= 1u << sidx;
-      R* const stage = stage0 + sidx * NP * PLS;
+      ring.ahead(list, nbig, j, g0, offs, nb, ne);
+      const R* const stage = ring.wait(j);
       double term;
       if (e - b <= EA * T)
-        term = l2_big_group<R, PSI, SHIFTED, EA, T, PLS>(y, xk, sj, q, b, e, lam, sigma, red, stage, &bar[sidx], nb, ne);
+        term = l2_big_group<R, PSI, SHIFTED, EA, T, PLS>(y, xk, sj, q, b, e, lam, sigma, red, stage, ring, nb, ne);
       else
-        term = l2_big_group<R, PSI, SHIFTED, EB, T, PLS>(y, xk, sj, q, b, e, lam, sigma, red, stage, &bar[sidx], nb, ne);
+        term = l2_big_group<R, PSI, SHIFTED, EB, T, PLS>(y, xk, sj, q, b, e, lam, sigma, red, stage, ring, nb, ne);
       if (PSI && t == 0) psi += term;
     }
   }
@@ -1715,33 +1714,15 @@ __global__ void __launch_bounds__(T, TPS / T)
   __shared__ __align__(8) uint64_t bar;
   extern __shared__ __align__(128) unsigned char big_stage_raw[];
   R* const stage = reinterpret_cast<R*>(big_stage_raw);  // three planes of PLS elements: q | xk | sj
+  // No StageRing here: the stage is the group's working memory (sol, then w) until the final pass, so it cannot take
+  // the next group early, and only one stage of 3 x 4096 elements fits per CTA.  The next group goes to L2 instead.
   const int t = threadIdx.x;
   if (t == 0) mbar_init(&bar, 1);
   __syncthreads();
   uint32_t phase = 0;
   int parity = 0, parity_f = 0;
   for (long long g0 = (long long)blockIdx.x * T; g0 < ngroups; g0 += (long long)gridDim.x * T) {
-    // index-ordered list of this chunk's groups of LO+1 .. EB T elements
-    int nbig;
-    {
-      const int lane = t & 31, w = t >> 5;
-      const long long g = g0 + t;
-      const long long mg = g < ngroups ? offs[g + 1] - offs[g] : 0;
-      const bool big = mg > LO && mg <= PL;
-      const unsigned bal = __ballot_sync(0xffffffffu, big);
-      __syncthreads();  // list / wcount reuse
-      if (lane == 0) wcount[w] = __popc(bal);
-      __syncthreads();
-      int base = 0;
-      nbig = 0;
-#pragma unroll
-      for (int ww = 0; ww < T / 32; ++ww) {
-        if (ww < w) base += wcount[ww];
-        nbig += wcount[ww];
-      }
-      if (big) list[base + __popc(bal & ((1u << lane) - 1u))] = t;
-      __syncthreads();
-    }
+    const int nbig = list_class_groups<T, LO, PL>(offs, g0, ngroups, list, wcount);
     for (int j = 0; j < nbig; ++j) {
       const long long g = g0 + list[j];
       const long long b = offs[g], e = offs[g + 1];
@@ -1860,32 +1841,19 @@ __global__ void __launch_bounds__(T, 512 / T)
   __shared__ double red[T / 32];
   __shared__ __align__(8) uint64_t bar[ST];
   extern __shared__ __align__(128) unsigned char val_stage_raw[];
-  R* const stage0 = reinterpret_cast<R*>(val_stage_raw);
   const int t = threadIdx.x;
-  if (t == 0)
-    for (int s = 0; s < ST; ++s) mbar_init(&bar[s], 1);
-  __syncthreads();
-  uint32_t phases = 0;
+  StageRing<R, 3, PLS, ST> ring(bar, reinterpret_cast<R*>(val_stage_raw));  // xk | sj | y
   Partial p;
   p.s = 0.0;
   p.s2 = 0.0;
   p.bad = -1;
   for (long long g0 = (long long)blockIdx.x * T; g0 < ngroups; g0 += (long long)gridDim.x * T) {
     const int nbig = list_class_groups<T, LO, EB * T>(offs, g0, ngroups, list, wcount);
-    if (t == 0) {
-      fence_proxy_async();
-      for (int s = 0; s < ST && s < nbig; ++s) {
-        const long long gf = g0 + list[s];
-        stage_group_bulk<R, 3, PLS>(stage0 + s * 3 * PLS, &bar[s], xk, sj, y, offs[gf], offs[gf + 1]);
-      }
-    }
+    ring.prime(list, nbig, g0, offs, xk, sj, y);
     for (int j = 0; j < nbig; ++j) {
-      const int sidx = j % ST;
       const long long g = g0 + list[j];
       const long long b = offs[g], e = offs[g + 1];
-      mbar_wait(&bar[sidx], (phases >> sidx) & 1u);
-      phases ^= 1u << sidx;
-      const R* stage = stage0 + sidx * 3 * PLS;
+      const R* stage = ring.wait(j);
       const R* px = stage + bulk_skip(xk + b) + t;
       const R* ps = stage + PLS + bulk_skip(sj + b) + t;
       const R* py = stage + 2 * PLS + bulk_skip(y + b) + t;
@@ -1909,11 +1877,8 @@ __global__ void __launch_bounds__(T, 512 / T)
       }
       ss = block_sum<T>(ss, red);
       if (t == 0) {
-        if (j + ST < nbig) {
-          const long long gn = g0 + list[j + ST];
-          fence_proxy_async();
-          stage_group_bulk<R, 3, PLS>(stage0 + sidx * 3 * PLS, &bar[sidx], xk, sj, y, offs[gn], offs[gn + 1]);
-        }
+        long long ahead_b, ahead_e;
+        if (ring.ahead(list, nbig, j, g0, offs, ahead_b, ahead_e)) ring.refill(xk, sj, y, ahead_b, ahead_e);
         p.s += (double)(lambda_g[g] * (R)sqrt(ss));  // λ_g ‖v_g‖  groupNormL2.jl:36
       }
     }
@@ -2020,45 +1985,69 @@ static int32_t prox_single_group(spx_ctx* ctx, int64_t n, R* y, const R* xk, con
   return ew_launch(ctx, ctx->stream, sc, n, 0, ctx->d_partials, &nb);
 }
 
-static int group_grid(spx_ctx* ctx, int64_t ngroups, const void* kernel) {
-  int per_sm = 1;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kGroupThreads, 0) != cudaSuccess || per_sm < 1)
-    per_sm = 1;
+// Grid of `want` CTAs, clamped to [1, cap].  A persistent (grid-stride) kernel is also held to the CTAs the device keeps
+// resident at once; a short-lived one (one CTA per chunk of work, cap kGridMax) is not.  Dynamic shared memory above
+// the default limit has to be allowed before the occupancy query and the launch.
+constexpr long long kGridMax = 1 << 20;
+static int32_t grid_for(spx_ctx* ctx, const void* kernel, int threads, size_t smem, long long want, long long cap,
+                        bool persistent, int* grid) {
+  if (smem > 0) SPX_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  if (persistent) {
+    int per_sm = 1;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem) != cudaSuccess || per_sm < 1)
+      per_sm = 1;
+    cap = std::min(cap, (long long)ctx->sm_count * per_sm);
+  }
+  *grid = (int)std::max(1LL, std::min(want, cap));
+  return SPX_OK;
+}
+// CTAs of a warp kernel (256 threads, one warp per task of kTask groups) that give every warp one task
+static long long warp_kernel_ctas(int64_t ngroups) {
   const long long ntasks = (ngroups + kTask - 1) / kTask;
-  long long want = (ntasks + (kGroupThreads / 32) - 1) / (kGroupThreads / 32);
-  long long cap = (long long)ctx->sm_count * per_sm;
-  if (cap > kMaxPartials) cap = kMaxPartials;
-  if (want < 1) want = 1;
-  return (int)(want < cap ? want : cap);
+  return (ntasks + (kGroupThreads / 32) - 1) / (kGroupThreads / 32);
+}
+// grid of a persistent warp kernel: one task per warp, at most the resident CTAs and kMaxPartials
+static int32_t group_grid(spx_ctx* ctx, int64_t ngroups, const void* kernel, int* grid) {
+  return grid_for(ctx, kernel, kGroupThreads, 0, warp_kernel_ctas(ngroups), kMaxPartials, true, grid);
 }
 
-// classes to launch for this layout: what spx_group_validate_offsets recorded, both when the layout is unknown
-static unsigned census_classes(const spx_ctx* ctx, const void* offs, int64_t ngroups, int64_t n) {
+// what spx_group_validate_offsets recorded for this layout, or nullptr
+static const spx_ctx::GroupCensus* find_census(const spx_ctx* ctx, const void* offs, int64_t ngroups, int64_t n) {
   for (const auto& c : ctx->census)
-    if (c.offs == offs && c.ngroups == (long long)ngroups && c.n == (long long)n) return c.classes & 3u;
-  return 3u;
+    if (c.offs == offs && c.ngroups == (long long)ngroups && c.n == (long long)n) return &c;
+  return nullptr;
 }
-// a validated layout whose groups all have <= 256 elements (the packed warp rounds hold every group)
-static bool census_short_only(const spx_ctx* ctx, const void* offs, int64_t ngroups, int64_t n) {
-  for (const auto& c : ctx->census)
-    if (c.offs == offs && c.ngroups == (long long)ngroups && c.n == (long long)n) return c.classes == 0u;
-  return false;
+// classes to launch for this layout: what the census recorded, both when the layout is unknown
+static unsigned census_classes(const spx_ctx* ctx, const void* offs, int64_t ngroups, int64_t n) {
+  const spx_ctx::GroupCensus* c = find_census(ctx, offs, ngroups, n);
+  return c ? c->classes & 3u : 3u;
+}
+
+// The context's side streams 0 and 1 and three events, created on first use: fork_side_streams makes both streams wait
+// for the work enqueued so far on ctx->stream, join_side_streams makes ctx->stream wait for both.
+static int32_t fork_side_streams(spx_ctx* ctx) {
+  for (int i = 0; i < 2; ++i)
+    if (!ctx->pipe_streams[i]) SPX_CUDA(cudaStreamCreateWithFlags(&ctx->pipe_streams[i], cudaStreamNonBlocking));
+  for (cudaEvent_t& ev : ctx->pipe_events)
+    if (!ev) SPX_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+  SPX_CUDA(cudaEventRecord(ctx->pipe_events[0], ctx->stream));
+  for (int i = 0; i < 2; ++i) SPX_CUDA(cudaStreamWaitEvent(ctx->pipe_streams[i], ctx->pipe_events[0], 0));
+  return SPX_OK;
+}
+static int32_t join_side_streams(spx_ctx* ctx) {
+  for (int i = 0; i < 2; ++i) {
+    SPX_CUDA(cudaEventRecord(ctx->pipe_events[1 + i], ctx->pipe_streams[i]));
+    SPX_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->pipe_events[1 + i], 0));
+  }
+  return SPX_OK;
 }
 
 #ifndef SPX_L2_MID_STAGES
 #define SPX_L2_MID_STAGES 2
 #endif
-// grid of a CTA-per-group kernel: one CTA per chunk of `threads` groups, at most the resident CTAs
-static int big_grid(spx_ctx* ctx, int64_t ngroups, const void* kernel, int threads, size_t stage_bytes) {
-  int per_sm = 1;
-  cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)stage_bytes);
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, stage_bytes) != cudaSuccess || per_sm < 1)
-    per_sm = 1;
-  long long want = (ngroups + threads - 1) / threads;
-  long long cap = (long long)ctx->sm_count * per_sm;
-  if (cap > kMaxPartials / 4) cap = kMaxPartials / 4;
-  if (want < 1) want = 1;
-  return (int)(want < cap ? want : cap);
+// grid of a persistent CTA-per-group kernel: one CTA per chunk of `threads` groups, at most the resident CTAs
+static int32_t big_grid(spx_ctx* ctx, int64_t ngroups, const void* kernel, int threads, size_t stage_bytes, int* grid) {
+  return grid_for(ctx, kernel, threads, stage_bytes, (ngroups + threads - 1) / threads, kMaxPartials / 4, true, grid);
 }
 
 template <class R>
@@ -2089,8 +2078,9 @@ int32_t value_group_binf(spx_ctx* ctx, int64_t n, const R* xk, const R* sj, cons
     return SPX_OK;
   }
   const double rad = 1.1 * (double)(R)delta;
-  const int grid0 = group_grid(ctx, ngroups, (const void*)group_value_kernel<R, 0>);
-  const int grid1 = group_grid(ctx, ngroups, (const void*)group_value_kernel<R, 1>);
+  int grid0 = 0, grid1 = 0, grid2 = 0, grid3 = 0;
+  int32_t st = group_grid(ctx, ngroups, (const void*)group_value_kernel<R, 0>, &grid0);
+  if (st == SPX_OK) st = group_grid(ctx, ngroups, (const void*)group_value_kernel<R, 1>, &grid1);
   // the classes (256, 1024] and (1024, 4096]: CTA per group, operands by bulk copies (as in launch_group_l2)
   constexpr int kMidT = 128;
   auto big_val = group_value_big_kernel<R, kGroupThreads, (int)kBigMin, kBigE / 2, kBigE, 1>;
@@ -2098,8 +2088,9 @@ int32_t value_group_binf(spx_ctx* ctx, int64_t n, const R* xk, const R* sj, cons
   const size_t big_bytes = 3 * (size_t)bulk_plane<R>((int)kBigMax) * sizeof(R);
   const size_t mid_bytes = SPX_L2_MID_STAGES * 3 * (size_t)bulk_plane<R>((int)kBigMin) * sizeof(R);
   const unsigned classes = census_classes(ctx, offs, ngroups, n);
-  const int grid2 = (classes & 2u) ? big_grid(ctx, ngroups, (const void*)big_val, kGroupThreads, big_bytes) : 0;
-  const int grid3 = (classes & 1u) ? big_grid(ctx, ngroups, (const void*)mid_val, kMidT, mid_bytes) : 0;
+  if (st == SPX_OK && (classes & 2u)) st = big_grid(ctx, ngroups, (const void*)big_val, kGroupThreads, big_bytes, &grid2);
+  if (st == SPX_OK && (classes & 1u)) st = big_grid(ctx, ngroups, (const void*)mid_val, kMidT, mid_bytes, &grid3);
+  if (st != SPX_OK) return st;
   group_value_kernel<R, 0><<<grid0, kGroupThreads, 0, ctx->stream>>>(xk, sj, y, ngroups, (const long long*)offs, lambda_g,
                                                                     binf, rad, classes, ctx->d_partials);
   group_value_kernel<R, 1><<<grid1, kGroupThreads, 0, ctx->stream>>>(xk, sj, y, ngroups, (const long long*)offs, lambda_g,
@@ -2112,8 +2103,7 @@ int32_t value_group_binf(spx_ctx* ctx, int64_t n, const R* xk, const R* sj, cons
                                                      ctx->d_partials + grid0 + grid1 + grid2);
   ctx->launches += 2 + (grid2 > 0) + (grid3 > 0);
   SPX_CUDA(cudaGetLastError());
-  const int grid = grid0 + grid1 + grid2 + grid3;
-  int32_t st = finalize_partials(ctx, grid, 1, false);
+  st = finalize_partials(ctx, grid0 + grid1 + grid2 + grid3, 1, false);
   if (st != SPX_OK) return st;
   // the reference accumulates sum_c in R; one rounding to R here
   *out = ctx->h_result[0].bad > 0 ? std::numeric_limits<double>::infinity() : (double)(R)ctx->h_result[0].s;
@@ -2139,10 +2129,12 @@ static int32_t launch_group_l2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const
   auto mid_psi = group_l2_big_kernel<R, true, SHIFTED, kMidT, (int)kMidMin, 4, 8, kMidStages>;
   auto mid_run = group_l2_big_kernel<R, false, SHIFTED, kMidT, (int)kMidMin, 4, 8, kMidStages>;
   if (psi_out) {
-    const int grid0 = group_grid(ctx, ngroups, (const void*)group_l2_kernel<R, true, 0, SHIFTED>);
-    const int grid1 = group_grid(ctx, ngroups, (const void*)group_l2_kernel<R, true, 1, SHIFTED>);
-    const int grid2 = (classes & 2u) ? big_grid(ctx, ngroups, (const void*)big_psi, kGroupThreads, big_bytes) : 0;
-    const int grid3 = (classes & 1u) ? big_grid(ctx, ngroups, (const void*)mid_psi, kMidT, mid_bytes) : 0;
+    int grid0 = 0, grid1 = 0, grid2 = 0, grid3 = 0;
+    int32_t st = group_grid(ctx, ngroups, (const void*)group_l2_kernel<R, true, 0, SHIFTED>, &grid0);
+    if (st == SPX_OK) st = group_grid(ctx, ngroups, (const void*)group_l2_kernel<R, true, 1, SHIFTED>, &grid1);
+    if (st == SPX_OK && (classes & 2u)) st = big_grid(ctx, ngroups, (const void*)big_psi, kGroupThreads, big_bytes, &grid2);
+    if (st == SPX_OK && (classes & 1u)) st = big_grid(ctx, ngroups, (const void*)mid_psi, kMidT, mid_bytes, &grid3);
+    if (st != SPX_OK) return st;
     group_l2_kernel<R, true, 0, SHIFTED><<<grid0, kGroupThreads, 0, ctx->stream>>>(
         y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma, classes, ctx->d_partials);
     group_l2_kernel<R, true, 1, SHIFTED><<<grid1, kGroupThreads, 0, ctx->stream>>>(
@@ -2155,7 +2147,7 @@ static int32_t launch_group_l2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const
                                                        ctx->d_partials + grid0 + grid1 + grid2);
     ctx->launches += 2 + (grid2 > 0) + (grid3 > 0);
     SPX_CUDA(cudaGetLastError());
-    int32_t st = finalize_partials(ctx, grid0 + grid1 + grid2 + grid3, 1, false);
+    st = finalize_partials(ctx, grid0 + grid1 + grid2 + grid3, 1, false);
     if (st != SPX_OK) return st;
     *psi_out = (double)(R)ctx->h_result[0].s;
     return SPX_OK;
@@ -2163,87 +2155,89 @@ static int32_t launch_group_l2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const
   // The size classes are independent: they run CONCURRENTLY on the context's side streams (fork / join by events on
   // the caller's stream), with one short-lived CTA per chunk of work instead of a persistent grid, so the block
   // scheduler interleaves the kernels as resources free up (the short-group class waits on its per-group arithmetic).
-  for (int i = 0; i < 2; ++i)
-    if (!ctx->pipe_streams[i]) SPX_CUDA(cudaStreamCreateWithFlags(&ctx->pipe_streams[i], cudaStreamNonBlocking));
-  for (int i = 13; i < 16; ++i)
-    if (!ctx->pipe_events[i]) SPX_CUDA(cudaEventCreateWithFlags(&ctx->pipe_events[i], cudaEventDisableTiming));
-  const long long ntasks = (ngroups + kTask - 1) / kTask;
-  const long long warps_per_cta = kGroupThreads / 32;
-  const int grid0 = (int)std::max<long long>(1, std::min<long long>((ntasks + warps_per_cta - 1) / warps_per_cta, 1 << 20));
-  const int grid2s = (int)std::max<long long>(1, std::min<long long>((ngroups + kGroupThreads - 1) / kGroupThreads, 1 << 20));
-  const int grid3s = (int)std::max<long long>(1, std::min<long long>((ngroups + kMidT - 1) / kMidT, 1 << 20));
+  int grid0 = 0, grid2 = 0, grid3 = 0;
+  int32_t st = grid_for(ctx, (const void*)group_l2_kernel<R, false, 0, SHIFTED>, kGroupThreads, 0,
+                        warp_kernel_ctas(ngroups), kGridMax, false, &grid0);
   // A class the layout is known not to hold (census of spx_group_validate_offsets) is not launched: its CTAs would
   // only scan the offsets, but their shared-memory carve-out keeps the warp kernel off the SMs they pass through
   // (uniform groups of 64: 2.21 ms with the two empty launches, 1.44 ms without).
-  SPX_CUDA(cudaEventRecord(ctx->pipe_events[13], ctx->stream));
-  if (classes & 2u) {
-    SPX_CUDA(cudaFuncSetAttribute((const void*)big_run, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)big_bytes));
-    big_run<<<grid2s, kGroupThreads, big_bytes, ctx->stream>>>(y, xk, sj, q, ngroups, (const long long*)offs, lambda_g,
-                                                              sigma, ctx->d_partials);
+  if (st == SPX_OK && (classes & 2u))
+    st = grid_for(ctx, (const void*)big_run, kGroupThreads, big_bytes, (ngroups + kGroupThreads - 1) / kGroupThreads,
+                  kGridMax, false, &grid2);
+  if (st == SPX_OK && (classes & 1u))
+    st = grid_for(ctx, (const void*)mid_run, kMidT, mid_bytes, (ngroups + kMidT - 1) / kMidT, kGridMax, false, &grid3);
+  if (st == SPX_OK) st = fork_side_streams(ctx);
+  if (st != SPX_OK) return st;
+  if (grid2 > 0) {
+    big_run<<<grid2, kGroupThreads, big_bytes, ctx->stream>>>(y, xk, sj, q, ngroups, (const long long*)offs, lambda_g,
+                                                             sigma, ctx->d_partials);
     ctx->launches++;
   }
-  if (classes & 1u) {
-    SPX_CUDA(cudaFuncSetAttribute((const void*)mid_run, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mid_bytes));
-    SPX_CUDA(cudaStreamWaitEvent(ctx->pipe_streams[0], ctx->pipe_events[13], 0));
-    mid_run<<<grid3s, kMidT, mid_bytes, ctx->pipe_streams[0]>>>(y, xk, sj, q, ngroups, (const long long*)offs, lambda_g,
-                                                               sigma, ctx->d_partials);
-    SPX_CUDA(cudaEventRecord(ctx->pipe_events[14], ctx->pipe_streams[0]));
+  if (grid3 > 0) {
+    mid_run<<<grid3, kMidT, mid_bytes, ctx->pipe_streams[0]>>>(y, xk, sj, q, ngroups, (const long long*)offs, lambda_g,
+                                                              sigma, ctx->d_partials);
     ctx->launches++;
   }
   // groups above 4096 elements (and those of a class not launched): the warp path, whose CTAs exit at once when there
   // are none -- on the side stream, under the short-group kernel
-  SPX_CUDA(cudaStreamWaitEvent(ctx->pipe_streams[1], ctx->pipe_events[13], 0));
   group_l2_kernel<R, false, 1, SHIFTED><<<grid0, kGroupThreads, 0, ctx->pipe_streams[1]>>>(
       y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma, classes, ctx->d_partials);
-  if (classes == 0u) {
-    group_l2_kernel<R, false, 0, SHIFTED><<<grid0, kGroupThreads, 0, ctx->stream>>>(
-        y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma, classes, ctx->d_partials);
-  } else {
-    group_l2_kernel<R, false, 0, SHIFTED><<<grid0, kGroupThreads, 0, ctx->pipe_streams[1]>>>(
-        y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma, classes, ctx->d_partials);
-  }
+  group_l2_kernel<R, false, 0, SHIFTED><<<grid0, kGroupThreads, 0, classes == 0u ? ctx->stream : ctx->pipe_streams[1]>>>(
+      y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma, classes, ctx->d_partials);
   ctx->launches += 2;
   SPX_CUDA(cudaGetLastError());
-  SPX_CUDA(cudaEventRecord(ctx->pipe_events[15], ctx->pipe_streams[1]));
-  if (classes & 1u) SPX_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->pipe_events[14], 0));
-  SPX_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->pipe_events[15], 0));
-  return SPX_OK;
+  return join_side_streams(ctx);
 }
 
 template <class R, int L>
-static void launch_uniform_binf_L(spx_ctx* ctx, R* y, const R* xk, const R* sj, const R* q, int64_t ngroups,
-                                  const R* lambda_g, R sigma, R delta, UDiv<R> by_sigma, const unsigned* uniform_flag,
-                                  unsigned* wl_count, unsigned* wl_rounds) {
+static int32_t launch_uniform_binf_L(spx_ctx* ctx, R* y, const R* xk, const R* sj, const R* q, int64_t ngroups,
+                                     const R* lambda_g, R sigma, R delta, UDiv<R> by_sigma, const unsigned* uniform_flag,
+                                     unsigned* wl_count, unsigned* wl_rounds) {
   const long long nrounds = (ngroups + (32 / L) - 1) / (32 / L);
   const long long want = (nrounds + (kGroupThreads / 32) - 1) / (kGroupThreads / 32);
-  auto grid_of = [&](const void* k, size_t smem_bytes) {
-    int per_sm = 1;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, kGroupThreads, smem_bytes) != cudaSuccess || per_sm < 1) per_sm = 1;
-    const long long cap = (long long)ctx->sm_count * per_sm;
-    return (int)std::max<long long>(1, std::min(want, cap));
-  };
   const size_t smem = (size_t)(kGroupThreads / 32) * UTile<R, L>::kWarpBytes;
-  cudaFuncSetAttribute((const void*)group_l2binf_uniform_kernel<R, L, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  cudaFuncSetAttribute((const void*)group_l2binf_uniform_kernel<R, L, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  group_l2binf_uniform_kernel<R, L, true>
-      <<<grid_of((const void*)group_l2binf_uniform_kernel<R, L, true>, smem), kGroupThreads, smem, ctx->stream>>>(
-          y, xk, sj, q, ngroups, lambda_g, sigma, delta, by_sigma, uniform_flag, wl_count, wl_rounds);
-  group_l2binf_uniform_kernel<R, L, false>
-      <<<grid_of((const void*)group_l2binf_uniform_kernel<R, L, false>, smem), kGroupThreads, smem, ctx->stream>>>(
-          y, xk, sj, q, ngroups, lambda_g, sigma, delta, by_sigma, uniform_flag, wl_count, wl_rounds);
+  int grid_fast = 0, grid_list = 0;
+  int32_t st = grid_for(ctx, (const void*)group_l2binf_uniform_kernel<R, L, true>, kGroupThreads, smem, want, kGridMax,
+                        true, &grid_fast);
+  if (st == SPX_OK)
+    st = grid_for(ctx, (const void*)group_l2binf_uniform_kernel<R, L, false>, kGroupThreads, smem, want, kGridMax, true,
+                  &grid_list);
+  if (st != SPX_OK) return st;
+  group_l2binf_uniform_kernel<R, L, true><<<grid_fast, kGroupThreads, smem, ctx->stream>>>(
+      y, xk, sj, q, ngroups, lambda_g, sigma, delta, by_sigma, uniform_flag, wl_count, wl_rounds);
+  group_l2binf_uniform_kernel<R, L, false><<<grid_list, kGroupThreads, smem, ctx->stream>>>(
+      y, xk, sj, q, ngroups, lambda_g, sigma, delta, by_sigma, uniform_flag, wl_count, wl_rounds);
+  return SPX_OK;
 }
 template <class R>
-static void launch_uniform_binf(spx_ctx* ctx, int L, R* y, const R* xk, const R* sj, const R* q, int64_t ngroups,
-                                const R* lambda_g, R sigma, R delta, UDiv<R> by_sigma, const unsigned* uniform_flag,
-                                unsigned* wl_count, unsigned* wl_rounds) {
+static int32_t launch_uniform_binf(spx_ctx* ctx, int L, R* y, const R* xk, const R* sj, const R* q, int64_t ngroups,
+                                   const R* lambda_g, R sigma, R delta, UDiv<R> by_sigma, const unsigned* uniform_flag,
+                                   unsigned* wl_count, unsigned* wl_rounds) {
   switch (L) {
 #define SPX_UL(LL) \
-  case LL: launch_uniform_binf_L<R, LL>(ctx, y, xk, sj, q, ngroups, lambda_g, sigma, delta, by_sigma, uniform_flag, wl_count, wl_rounds); break;
+  case LL: return launch_uniform_binf_L<R, LL>(ctx, y, xk, sj, q, ngroups, lambda_g, sigma, delta, by_sigma, uniform_flag, wl_count, wl_rounds);
     SPX_UL(2) SPX_UL(4) SPX_UL(8) SPX_UL(16) SPX_UL(32)
 #undef SPX_UL
-    default: break;
+    default: return SPX_OK;
   }
 }
+
+// ctx->d_scratch during a GroupNormL2Binf prox!: a head that every call clears, the work list of the uniform kernels at
+// 4 KiB, then `done` (one byte per group) on the next 256-byte boundary behind the list
+struct BinfScratch {
+  struct alignas(32) Head {
+    unsigned long long counter;  // task hand-out of the long groups (group_l2binf_kernel<R, 1>)
+    unsigned long_flag;          // some task holds a group of more than 256 elements
+    unsigned uniform_flag;       // offs is {0, m, 2m, ...}: the uniform kernels own the call
+    unsigned wl_count;           // rounds in wl_rounds
+  } head;
+  unsigned char unused[4096 - sizeof(Head)];
+  unsigned wl_rounds[1];  // one entry per round of the uniform layout
+  static size_t done_offset(int64_t nrounds) {
+    return offsetof(BinfScratch, wl_rounds) + (((size_t)nrounds * sizeof(unsigned) + 255) & ~(size_t)255);
+  }
+};
+static_assert(sizeof(BinfScratch::Head) == 32 && offsetof(BinfScratch, wl_rounds) == 4096, "Binf scratch layout");
 
 template <class R>
 static int32_t prox_group(spx_ctx* ctx, bool binf, int64_t n, R* y, const R* xk, const R* sj, const R* q,
@@ -2263,8 +2257,10 @@ static int32_t prox_group(spx_ctx* ctx, bool binf, int64_t n, R* y, const R* xk,
     }
     UDiv<R> by_sigma;
     by_sigma.set((R)sigma);
-    const int grid0 = group_grid(ctx, ngroups, (const void*)group_l2binf_kernel<R, 0>);
-    const int grid1 = group_grid(ctx, ngroups, (const void*)group_l2binf_kernel<R, 1>);
+    int grid0 = 0, grid1 = 0;
+    int32_t st = group_grid(ctx, ngroups, (const void*)group_l2binf_kernel<R, 0>, &grid0);
+    if (st == SPX_OK) st = group_grid(ctx, ngroups, (const void*)group_l2binf_kernel<R, 1>, &grid1);
+    if (st != SPX_OK) return st;
     // uniform layout candidate: n == ngroups m, m = 8 L, 16-byte aligned vectors.  Whether offs really is
     // {0, m, 2m, ...} is checked on the device; the flag gates the uniform kernels and the generic ones.
     const int64_t m = ngroups > 0 && n % ngroups == 0 ? n / ngroups : 0;
@@ -2273,22 +2269,19 @@ static int32_t prox_group(spx_ctx* ctx, bool binf, int64_t n, R* y, const R* xk,
     const bool sigma_ok = std::isfinite(sigma) && std::fabs(sigma) > 1e-30 && std::fabs(sigma) < 1e30 &&
                           std::isfinite(delta) && std::fabs(delta) < 1e30;
     const bool uni = sigma_ok && aligned && (m == 16 || m == 32 || m == 64 || m == 128 || m == 256) && n < (int64_t(1) << 39);
-    const int64_t nrounds = uni ? (n + kRoundElems - 1) / kRoundElems : 0;
-    const size_t done_off = 4096 + (((size_t)nrounds * sizeof(unsigned) + 255) & ~(size_t)255);
-    int32_t st0 = ensure_scratch(ctx, done_off + (size_t)ngroups + 256);
-    if (st0 != SPX_OK) return st0;
-    unsigned long long* counter = (unsigned long long*)ctx->d_scratch;  // long groups: dynamic task hand-out
-    unsigned* long_flag = (unsigned*)((char*)ctx->d_scratch + 8);
-    unsigned* uniform_flag = (unsigned*)((char*)ctx->d_scratch + 12);
-    unsigned* wl_count = (unsigned*)((char*)ctx->d_scratch + 16);
-    unsigned* wl_rounds = (unsigned*)((char*)ctx->d_scratch + 4096);
-    SPX_CUDA(cudaMemsetAsync(ctx->d_scratch, 0, 32, ctx->stream));
+    const size_t done_off = BinfScratch::done_offset(uni ? (n + kRoundElems - 1) / kRoundElems : 0);
+    st = ensure_scratch(ctx, done_off + (size_t)ngroups + 256);
+    if (st != SPX_OK) return st;
+    BinfScratch* const scratch = (BinfScratch*)ctx->d_scratch;
+    unsigned* const uniform_flag = &scratch->head.uniform_flag;
+    SPX_CUDA(cudaMemsetAsync(&scratch->head, 0, sizeof(BinfScratch::Head), ctx->stream));
     if (uni) {
       SPX_CUDA(cudaMemsetAsync(uniform_flag, 1, sizeof(unsigned), ctx->stream));
       const int cgrid = (int)std::min<int64_t>((ngroups + 256) / 256, (int64_t)ctx->sm_count * 8);
       group_uniform_check_kernel<<<cgrid, 256, 0, ctx->stream>>>((const long long*)offs, ngroups, m, uniform_flag);
-      launch_uniform_binf<R>(ctx, (int)(m / kEPL), y, xk, sj, q, ngroups, lambda_g, (R)sigma, (R)delta, by_sigma,
-                             uniform_flag, wl_count, wl_rounds);
+      st = launch_uniform_binf<R>(ctx, (int)(m / kEPL), y, xk, sj, q, ngroups, lambda_g, (R)sigma, (R)delta, by_sigma,
+                                  uniform_flag, &scratch->head.wl_count, scratch->wl_rounds);
+      if (st != SPX_OK) return st;
       ctx->launches += 3;
     }
     // Fast kernels first, each marking the groups it has written in `done`: groups of <= 256 elements on the planner's
@@ -2299,92 +2292,75 @@ static int32_t prox_group(spx_ctx* ctx, bool binf, int64_t n, R* y, const R* xk,
     // overlaps an input partially (a group's y would land on another group's inputs) or σ, Δ are outside the range of
     // the branch-free quotient.
     unsigned char* done = nullptr;
-    {
-      const char *y0 = (const char*)y, *y1 = y0 + (size_t)n * sizeof(R);
-      auto overlaps = [&](const R* p) {
-        return p != y && (const char*)p < y1 && (const char*)p + (size_t)n * sizeof(R) > y0;
+    const char *y0 = (const char*)y, *y1 = y0 + (size_t)n * sizeof(R);
+    auto overlaps = [&](const R* p) {
+      return p != y && (const char*)p < y1 && (const char*)p + (size_t)n * sizeof(R) > y0;
+    };
+    if (sigma_ok && !(overlaps(xk) || overlaps(sj) || overlaps(q))) {
+      done = (unsigned char*)ctx->d_scratch + done_off;
+      SPX_CUDA(cudaMemsetAsync(done, 0, (size_t)ngroups, ctx->stream));
+      // a class the layout is known not to hold is not launched (whatever is not marked done goes to the bracketing
+      // search anyway, so the census is only a hint here as well)
+      const unsigned classes = census_classes(ctx, offs, ngroups, n);
+      // With CTA-per-group classes present the fast kernels run CONCURRENTLY (short groups and the 128-thread classes on
+      // the context's side streams, as in launch_group_l2), each with one short-lived CTA per chunk of groups instead of
+      // a persistent grid: the block scheduler then mixes CTAs of the kernels on an SM, and the barrier-separated phases
+      // of one kernel leave their idle issue slots to the others.
+      const bool fork = classes != 0u;
+      if (fork) {
+        st = fork_side_streams(ctx);
+        if (st != SPX_OK) return st;
+      }
+      auto launch_class = [&](auto kern, int threads, size_t stage_bytes, cudaStream_t stream) -> int32_t {
+        int grid = 0;
+        const int32_t s2 = grid_for(ctx, (const void*)kern, threads, stage_bytes, (ngroups + threads - 1) / threads,
+                                    kGridMax, false, &grid);
+        if (s2 != SPX_OK) return s2;
+        kern<<<grid, threads, stage_bytes, stream>>>(y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, (R)sigma,
+                                                     (R)delta, by_sigma, uni ? uniform_flag : nullptr, done);
+        ctx->launches++;
+        return SPX_OK;
       };
-      if (sigma_ok && !(overlaps(xk) || overlaps(sj) || overlaps(q)) && std::getenv("SPX_BINF_NOBIG") == nullptr) {
-        done = (unsigned char*)ctx->d_scratch + done_off;
-        SPX_CUDA(cudaMemsetAsync(done, 0, (size_t)ngroups, ctx->stream));
-        // a class the layout is known not to hold is not launched (whatever is not marked done goes to the bracketing
-        // search anyway, so the census is only a hint here as well)
-        const unsigned classes = census_classes(ctx, offs, ngroups, n);
-        // With CTA-per-group classes present the fast kernels run CONCURRENTLY (short groups and the 128-thread classes on
-        // the context's side streams, fork / join by events as in launch_group_l2), each with one short-lived CTA per
-        // chunk of groups instead of a persistent grid: the block scheduler then mixes CTAs of the kernels on an SM, and
-        // the barrier-separated phases of one kernel leave their idle issue slots to the others.
-        const bool fork = classes != 0u && std::getenv("SPX_BINF_SERIAL") == nullptr;
-        cudaStream_t s_small = ctx->stream, s_mid = ctx->stream;
-        if (fork) {
-          for (int i = 0; i < 2; ++i)
-            if (!ctx->pipe_streams[i]) SPX_CUDA(cudaStreamCreateWithFlags(&ctx->pipe_streams[i], cudaStreamNonBlocking));
-          for (int i = 13; i < 16; ++i)
-            if (!ctx->pipe_events[i]) SPX_CUDA(cudaEventCreateWithFlags(&ctx->pipe_events[i], cudaEventDisableTiming));
-          s_mid = ctx->pipe_streams[0];
-          s_small = ctx->pipe_streams[1];
-          SPX_CUDA(cudaEventRecord(ctx->pipe_events[13], ctx->stream));
-          SPX_CUDA(cudaStreamWaitEvent(s_mid, ctx->pipe_events[13], 0));
-          SPX_CUDA(cudaStreamWaitEvent(s_small, ctx->pipe_events[13], 0));
-        }
-        auto launch_class = [&](auto kern, int threads, size_t stage_bytes, cudaStream_t stream) -> int32_t {
-          int per_sm = 1;
-          SPX_CUDA(cudaFuncSetAttribute((const void*)kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)stage_bytes));
-          if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)kern, threads, stage_bytes) != cudaSuccess ||
-              per_sm < 1)
-            per_sm = 1;
-          const int64_t chunks = (ngroups + threads - 1) / threads;
-          const int grid = (int)std::max<int64_t>(
-              1, std::min<int64_t>(chunks, fork ? (int64_t)(1 << 20) : (int64_t)ctx->sm_count * per_sm));
-          kern<<<grid, threads, stage_bytes, stream>>>(y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, (R)sigma,
-                                                      (R)delta, by_sigma, uni ? uniform_flag : nullptr, done);
-          ctx->launches++;
-          return SPX_OK;
-        };
-        int32_t stc = SPX_OK;
-        // (1024, 4096]: 256 threads x 8 or 16 elements, two CTAs per SM in 128 registers (measured at 2^28 Float64,
-        // ragged layout: 2.8 ms; split into 512 x 8 and 256 x 8 at 64 registers and 1024 threads per SM: 3.4 ms;
-        // three CTAs per SM in 80 registers with sj read from global memory instead of staged: 3.3 ms -- more
-        // resident CTAs do not help this class).
-        // (256, 1024]: two shapes of 128 threads, 8 and 4 elements, 64 registers (0.77 ms; one shape of 4 or 8
-        // elements at 128 registers: 0.94 ms).
-        if (classes & 2u) {
-          stc = launch_class(group_l2binf_big_kernel<R, kBinfBigThreads, 1024, 8, 16, 512>, kBinfBigThreads,
-                             3 * (size_t)bulk_plane<R>(16 * kBinfBigThreads) * sizeof(R), ctx->stream);
-          if (stc != SPX_OK) return stc;
-        }
-        if ((classes & 1u) && std::getenv("SPX_BINF_NOMID") == nullptr) {
-          stc = launch_class(group_l2binf_big_kernel<R, kBinfMidThreads, 512, 8, 8, 1024>, kBinfMidThreads,
-                             3 * (size_t)bulk_plane<R>(8 * kBinfMidThreads) * sizeof(R), s_mid);
-          if (stc != SPX_OK) return stc;
-          stc = launch_class(group_l2binf_big_kernel<R, kBinfMidThreads, 256, 4, 4, 1024>, kBinfMidThreads,
-                             3 * (size_t)bulk_plane<R>(4 * kBinfMidThreads) * sizeof(R), s_mid);
-          if (stc != SPX_OK) return stc;
-        }
-        // the short groups last: the class (1024, 4096] is the long pole and should get the SMs first
-        if (std::getenv("SPX_BINF_NOSMALL") == nullptr) {
-          const long long ntasks = (ngroups + kTask - 1) / kTask;
-          const int grids = fork ? (int)std::max<long long>(1, std::min<long long>((ntasks + 7) / 8, 1 << 20))
-                                 : group_grid(ctx, ngroups, (const void*)group_l2binf_small_fast_kernel<R>);
-          group_l2binf_small_fast_kernel<R><<<grids, kGroupThreads, 0, s_small>>>(
-              y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, (R)sigma, (R)delta, by_sigma,
-              uni ? uniform_flag : nullptr, done);
-          ctx->launches++;
-        }
-        if (fork) {
-          SPX_CUDA(cudaEventRecord(ctx->pipe_events[14], s_mid));
-          SPX_CUDA(cudaEventRecord(ctx->pipe_events[15], s_small));
-          SPX_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->pipe_events[14], 0));
-          SPX_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->pipe_events[15], 0));
-        }
+      // (1024, 4096]: 256 threads x 8 or 16 elements, two CTAs per SM in 128 registers (measured at 2^28 Float64,
+      // ragged layout: 2.8 ms; split into 512 x 8 and 256 x 8 at 64 registers and 1024 threads per SM: 3.4 ms;
+      // three CTAs per SM in 80 registers with sj read from global memory instead of staged: 3.3 ms -- more
+      // resident CTAs do not help this class).
+      // (256, 1024]: two shapes of 128 threads, 8 and 4 elements, 64 registers (0.77 ms; one shape of 4 or 8
+      // elements at 128 registers: 0.94 ms).
+      if (classes & 2u) {
+        st = launch_class(group_l2binf_big_kernel<R, kBinfBigThreads, 1024, 8, 16, 512>, kBinfBigThreads,
+                          3 * (size_t)bulk_plane<R>(16 * kBinfBigThreads) * sizeof(R), ctx->stream);
+        if (st != SPX_OK) return st;
+      }
+      if (classes & 1u) {
+        st = launch_class(group_l2binf_big_kernel<R, kBinfMidThreads, 512, 8, 8, 1024>, kBinfMidThreads,
+                          3 * (size_t)bulk_plane<R>(8 * kBinfMidThreads) * sizeof(R), ctx->pipe_streams[0]);
+        if (st != SPX_OK) return st;
+        st = launch_class(group_l2binf_big_kernel<R, kBinfMidThreads, 256, 4, 4, 1024>, kBinfMidThreads,
+                          3 * (size_t)bulk_plane<R>(4 * kBinfMidThreads) * sizeof(R), ctx->pipe_streams[0]);
+        if (st != SPX_OK) return st;
+      }
+      // the short groups last: the class (1024, 4096] is the long pole and should get the SMs first.  Alone (no class
+      // present) they take a persistent grid on ctx->stream.
+      int grids = 0;
+      st = grid_for(ctx, (const void*)group_l2binf_small_fast_kernel<R>, kGroupThreads, 0, warp_kernel_ctas(ngroups),
+                    fork ? kGridMax : kMaxPartials, !fork, &grids);
+      if (st != SPX_OK) return st;
+      group_l2binf_small_fast_kernel<R><<<grids, kGroupThreads, 0, fork ? ctx->pipe_streams[1] : ctx->stream>>>(
+          y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, (R)sigma, (R)delta, by_sigma,
+          uni ? uniform_flag : nullptr, done);
+      ctx->launches++;
+      if (fork) {
+        st = join_side_streams(ctx);
+        if (st != SPX_OK) return st;
       }
     }
     group_l2binf_kernel<R, 0><<<grid0, kGroupThreads, 0, ctx->stream>>>(
-        y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, (R)sigma, (R)delta, by_sigma, nullptr, long_flag,
-        uni ? uniform_flag : nullptr, done);
+        y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, (R)sigma, (R)delta, by_sigma, nullptr,
+        &scratch->head.long_flag, uni ? uniform_flag : nullptr, done);
     group_l2binf_kernel<R, 1><<<grid1, kGroupThreads, 0, ctx->stream>>>(
-        y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, (R)sigma, (R)delta, by_sigma, counter, long_flag,
-        uni ? uniform_flag : nullptr, done);
+        y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, (R)sigma, (R)delta, by_sigma, &scratch->head.counter,
+        &scratch->head.long_flag, uni ? uniform_flag : nullptr, done);
     ctx->launches += 2;
     SPX_CUDA(cudaGetLastError());
   }
@@ -2506,13 +2482,18 @@ static int32_t step_groupl2(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, 
   DeviceGuard g(ctx->device);
   out3[0] = out3[1] = out3[2] = 0.0;
   if (ngroups == 0 || n == 0) return SPX_OK;
-  if (ngroups > 1 && census_short_only(ctx, offs, ngroups, n) && std::getenv("SPX_STEP_COMPOSED") == nullptr) {
-    const int grid = std::min(group_grid(ctx, ngroups, (const void*)group_l2_step_kernel<R>), kMaxPartials / 2);
+  const spx_ctx::GroupCensus* census = find_census(ctx, offs, ngroups, n);
+  // a validated layout whose groups all have <= 256 elements (the packed warp rounds hold every group)
+  if (ngroups > 1 && census && census->classes == 0u && std::getenv("SPX_STEP_COMPOSED") == nullptr) {
+    int grid = 0;
+    int32_t st = grid_for(ctx, (const void*)group_l2_step_kernel<R>, kGroupThreads, 0, warp_kernel_ctas(ngroups),
+                          kMaxPartials / 2, true, &grid);
+    if (st != SPX_OK) return st;
     group_l2_step_kernel<R><<<grid, kGroupThreads, 0, ctx->stream>>>(s, xsy, xk, sj, grad, ngroups, (const long long*)offs,
                                                                     lambda_g, (R)nu, -(R)nu, ctx->d_partials);
     ctx->launches++;
     SPX_CUDA(cudaGetLastError());
-    int32_t st = finalize_partials(ctx, grid, 2, false);
+    st = finalize_partials(ctx, grid, 2, false);
     if (st != SPX_OK) return st;
     if (ctx->h_result[0].bad <= 0) {
       out3[0] = (double)(R)ctx->h_result[0].s;

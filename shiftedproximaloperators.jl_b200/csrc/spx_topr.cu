@@ -1247,7 +1247,7 @@ static int32_t topr_stream_launch(spx_ctx* ctx, int64_t nprob, int64_t n, R* y, 
   const size_t key_bytes = (size_t)n * sizeof(unsigned short);
   // keys in shared memory while 2 n bytes fit next to the static state of a CTA: one 1024-thread CTA per SM above
   // 72 KiB of keys, two 512-thread CTAs down to 36 KiB, four 256-thread CTAs below
-  const bool smem_keys = key_bytes <= 200 * 1024 && std::getenv("SPX_TOPR_L2KEYS") == nullptr;
+  const bool smem_keys = key_bytes <= 200 * 1024;
   int32_t st = SPX_OK;
   unsigned char* flags = nullptr;
   auto go = [&](auto kern, int threads, size_t dyn, bool scratch_keys) -> int32_t {
@@ -1307,8 +1307,7 @@ static int32_t prox_indballl0(spx_ctx* ctx, int64_t nprob, int64_t n, R* y, cons
     const char *y0 = (const char*)y, *y1 = y0 + (size_t)nprob * n * sizeof(R);
     auto overlaps = [&](const R* p) { return (const char*)p < y1 && (const char*)p + (size_t)nprob * n * sizeof(R) > y0; };
     const bool alias = overlaps(xk) || overlaps(sj) || overlaps(q);
-    if (vec && !alias && n % 8 == 0 && n >= 4096 && r > 0 && r < n && nprob >= 2 * (int64_t)ctx->sm_count &&
-        std::getenv("SPX_TOPR_CLUSTER") == nullptr) {
+    if (vec && !alias && n % 8 == 0 && n >= 4096 && r > 0 && r < n && nprob >= 2 * (int64_t)ctx->sm_count) {
       return binf ? topr_stream_launch<R, true>(ctx, nprob, n, y, xk, sj, q, r, (R)delta)
                   : topr_stream_launch<R, false>(ctx, nprob, n, y, xk, sj, q, r, (R)delta);
     }
