@@ -352,6 +352,30 @@ typedef struct spx_box_job_f32 {
   int32_t spx_step_box_##SUF(spx_ctx* ctx, int32_t op, int64_t n, R* s, R* xsy, const R* xk,     \
                              const R* sj, const R* grad, const spx_bound* l, const spx_bound* u, \
                              const spx_sel* sel, double lambda, double nu, double* out3_host);   \
+  /* The fused step around iprox! (diagonal model: the R2DH / TRDH iterations of               */ \
+  /* RegularizedOptimization.jl), in the one pass of the iprox! itself:                          */ \
+  /*   d = D .+ dshift                          [rounded to R like the caller's broadcast]       */ \
+  /*   iprox!(s, ψ, grad, d)                    [shiftedNormL1.jl:60-75, shiftedNormL0.jl:61-80, */ \
+  /*                                             shiftedNormL1Box.jl:131-225,                    */ \
+  /*                                             shiftedNormL0Box.jl:137-231]                    */ \
+  /*   xsy = (xk + sj) + s                      [xsy == NULL: not written]                       */ \
+  /*   out4_host[0] = ψ(s)                      [ShiftedProximalOperators.jl:51-54; Box forms    */ \
+  /*                                             shiftedNormL1Box.jl:70-82: Inf outside the box] */ \
+  /*   out4_host[1] = Σ s_i², out4_host[2] = Σ grad_i s_i, out4_host[3] = Σ d_i s_i² (Float64)   */ \
+  /* s is bit-identical to spx_iprox_*(g = grad, d = D .+ dshift rounded to R).  sj == NULL: ψ    */ \
+  /* shifted once (sj = 0).  kind = SPX_H_L1, _L0 (no iprox! for _LHALF: SPX_E_INVALID).  The     */ \
+  /* `@assert d[i] > 0` of the unboxed forms applies to d: SPX_E_ASSERT_D and *first_bad_d (may   */ \
+  /* be NULL) as for spx_iprox_l1; s is written in full either way.  s may be grad and xsy may be */ \
+  /* xk (each element's operands are read before its results are written).  The call            */ \
+  /* synchronises; the four sums are all-reduced when the context reduces scalars.               */ \
+  int32_t spx_istep_sep_##SUF(spx_ctx* ctx, int32_t kind, int64_t n, R* s, R* xsy, const R* xk,  \
+                              const R* sj, const R* grad, const R* D, double dshift,             \
+                              double lambda, int64_t* first_bad_d, double* out4_host);           \
+  /* the same step for the Box forms; op: 0 L1Box, 1 L0Box (2 LhalfBox: SPX_E_INVALID) */        \
+  int32_t spx_istep_box_##SUF(spx_ctx* ctx, int32_t op, int64_t n, R* s, R* xsy, const R* xk,    \
+                              const R* sj, const R* grad, const R* D, double dshift,             \
+                              const spx_bound* l, const spx_bound* u, const spx_sel* sel,        \
+                              double lambda, double* out4_host);                                 \
   /* The step around a prox! that is not one streaming pass (groups, top-r, ShiftedNormL1B2): the    */ \
   /* caller's sweeps as two passes around the operator's own entry point --                          */ \
   /*   spx_step_pre:   q = (-nu) .* grad (rounded to R), written where s will be;                    */ \

@@ -78,13 +78,7 @@ static int32_t iprox_sep(spx_ctx* ctx, int kind, int64_t n, R* y, const R* xk, c
   SPX_CHECK_VEC3(ctx, n, y, xk, sj, g);
   SPX_REQUIRE(n == 0 || d != nullptr, "null d");
   const R lam = (R)lambda;
-  auto setup = [&](auto& op) {
-    set3(op, xk, sj, g);
-    op.in[3] = d;
-    op.fill[3] = R(1);
-    op.y = y;
-    op.lambda = lam;
-  };
+  auto setup = [&](auto& op) { set_iprox(op, y, xk, sj, g, d, lam); };
   int nb = 0;
   int32_t st;
   if (psi_out) {
@@ -139,15 +133,11 @@ static int32_t launch_box_t(spx_ctx* ctx, cudaStream_t stream, int opc, bool inv
   } else {
     if (opc == BOX_L1) {
       IproxL1Box<R, PSI> op;
-      set_box(op, xk, sj, qg, d, lvec, lval, uvec, uval);
-      op.y = y; op.sel = sel; op.lambda = lambda;
-      op.lam_ok = lambda == R(0) || (std::fabs((double)lambda) > 1e-100 && std::fabs((double)lambda) < 1e100);
+      set_iprox_box(op, y, xk, sj, qg, d, lvec, lval, uvec, uval, sel, lambda);
       return ew_launch(ctx, stream, op, n, base, partials, nb);
     } else if (opc == BOX_L0) {
       IproxL0Box<R, PSI> op;
-      set_box(op, xk, sj, qg, d, lvec, lval, uvec, uval);
-      op.y = y; op.sel = sel; op.lambda = lambda;
-      op.lam_ok = lambda == R(0) || (std::fabs((double)lambda) > 1e-150 && std::fabs((double)lambda) < 1e150);
+      set_iprox_box(op, y, xk, sj, qg, d, lvec, lval, uvec, uval, sel, lambda);
       return ew_launch(ctx, stream, op, n, base, partials, nb);
     }
   }

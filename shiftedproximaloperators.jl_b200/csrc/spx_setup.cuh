@@ -26,6 +26,37 @@ static inline void set_box(Op& op, const R* xk, const R* sj, const R* qg, const 
   op.in[k] = uvec; op.fill[k++] = uval;
 }
 
+// operands and λ of the iprox! functors, shared by iprox! (spx_elementwise.cu) and the fused istep (spx_step.cu).
+// Unboxed (IproxL1 / IproxL0): xk, sj, g, d (d's fill is never read: d must be a vector)
+template <class Op, class R>
+static inline void set_iprox(Op& op, R* y, const R* xk, const R* sj, const R* g, const R* d, R lambda) {
+  set3(op, xk, sj, g);
+  op.in[3] = d;
+  op.fill[3] = R(1);
+  op.y = y;
+  op.lambda = lambda;
+}
+// Box (IproxL1Box / IproxL0Box): set_box, the selection, λ and lam_ok -- λ is 0 or a normal number far enough from
+// the range limits for the one-reciprocal quotients (quot4 / quot3 in spx_ops.cuh)
+static inline bool lam_within(double lambda, double lo, double hi) {
+  return lambda == 0.0 || (std::fabs(lambda) > lo && std::fabs(lambda) < hi);
+}
+template <class R, bool PSI> static inline void set_lam_ok(IproxL1Box<R, PSI>& op) {
+  op.lam_ok = lam_within((double)op.lambda, 1e-100, 1e100);
+}
+template <class R, bool PSI> static inline void set_lam_ok(IproxL0Box<R, PSI>& op) {
+  op.lam_ok = lam_within((double)op.lambda, 1e-150, 1e150);
+}
+template <class Op, class R>
+static inline void set_iprox_box(Op& op, R* y, const R* xk, const R* sj, const R* g, const R* d, const R* lvec, R lval,
+                                 const R* uvec, R uval, DevSel sel, R lambda) {
+  set_box(op, xk, sj, g, d, lvec, lval, uvec, uval);
+  op.y = y;
+  op.sel = sel;
+  op.lambda = lambda;
+  set_lam_ok(op);
+}
+
 // λ·Σ in R, returned as double (NormL1/NormL0/RootNormLhalf value functors)
 template <class R> static inline double scale_value(int kind, R lambda, double sum, int64_t r) {
   if (kind == SPX_H_INDBALLL0) return sum <= (double)r ? 0.0 : kInf;

@@ -12,6 +12,12 @@
 // Same streaming structure as ew_kernel (spx_elementwise.cuh): 128-bit loads of every operand, UNROLL
 // independent requests per stream before the first use, streaming stores, one partial slot per CTA folded
 // in fixed order.
+//
+// The diagonal quasi-Newton iterations (R2DH, TRDH) wrap iprox!(s, ψ, ∇f, D .+ σ) in the same sweeps plus the model's
+// quadratic term; the iprox! form of the kernel (IPROX) does that step in the same pass:
+//     d_i   = D_i + σ                        (rounded to R like the caller's broadcast)
+//     s_i   = iprox!(ψ, ∇f, d)_i             IproxL1/L0 and their Box forms, bit for bit the stand-alone iprox!
+//     xsy_i, ψ(s), Σ s_i², Σ ∇f_i s_i        as above,  and  Σ d_i s_i²  in Float64
 #include "spx_elementwise.cuh"
 #include "spx_ops.cuh"
 #include "spx_setup.cuh"
@@ -23,13 +29,22 @@ namespace spx {
 #ifndef SPX_STEP_MINB
 #define SPX_STEP_MINB 3
 #endif
-template <class Op> struct StepBlocks {
-  static constexpr int value = MinBlocks<Op>::value > SPX_STEP_MINB ? SPX_STEP_MINB : MinBlocks<Op>::value;
+// The iprox! form also keeps d, ∇f and Σ d s² live.  Under the 84 registers of 3 CTAs the Float64 IproxL0Box instance
+// spills 36 bytes, so that form alone gets 2 CTAs = 128 registers.  The other Box forms keep 3: on a B200 at n = 2^28
+// Float64 / 2^29 Float32 they ran about 3 % faster there than at 2 (profiles/r05_istep_ops_ctas.txt).
+template <class Op> struct IstepTwoCtas : std::false_type {};
+template <bool PSI> struct IstepTwoCtas<IproxL0Box<double, PSI>> : std::true_type {};
+template <class Op, bool IPROX = false> struct StepBlocks {
+  static constexpr int cap = IPROX && IstepTwoCtas<Op>::value ? 2 : SPX_STEP_MINB;
+  static constexpr int value = MinBlocks<Op>::value > cap ? cap : MinBlocks<Op>::value;
 };
 
-template <int VEC, int UNROLL, class Op>
-__global__ void __launch_bounds__(kEwThreads, StepBlocks<Op>::value)
-    step_kernel(const Op op, const typename Op::Real mnu, typename Op::Real* xsy, const long long n,
+// IPROX = false: the step around prox!, c = -ν scales ∇f into q.
+// IPROX = true:  the step around iprox!, ∇f goes to the functor as loaded, c = σ shifts the diagonal (x[3]) into
+//                d = D + σ, and Σ d s² is summed as well.
+template <int VEC, int UNROLL, class Op, bool IPROX = false>
+__global__ void __launch_bounds__(kEwThreads, StepBlocks<Op, IPROX>::value)
+    step_kernel(const Op op, const typename Op::Real c, typename Op::Real* xsy, const long long n,
                 Partial* __restrict__ partials) {
   using R = typename Op::Real;
   constexpr int NIN = Op::NIN;
@@ -37,14 +52,18 @@ __global__ void __launch_bounds__(kEwThreads, StepBlocks<Op>::value)
   acc.s = 0.0;
   acc.s2 = 0.0;
   acc.bad = -1;
-  double dot = 0.0;
+  double dot = 0.0, sds = 0.0;
   auto element = [&](R (&x)[NIN], long long i, R& s, R& v) {
     const R g = x[2];
-    x[2] = mnu * g;  // q = -ν ∇f
+    if constexpr (IPROX)
+      x[3] = x[3] + c;  // d = D + σ
+    else
+      x[2] = c * g;  // q = -ν ∇f
     s = op.apply(x, i, acc);
     v = (x[0] + x[1]) + s;
     acc.s2 = __fma_rn((double)s, (double)s, acc.s2);
     dot = __fma_rn((double)g, (double)s, dot);
+    if constexpr (IPROX) sds = __fma_rn((double)x[3] * (double)s, (double)s, sds);
   };
 
   const long long nvec = n / VEC;
@@ -95,7 +114,7 @@ __global__ void __launch_bounds__(kEwThreads, StepBlocks<Op>::value)
   acc = block_fold<kEwThreads>(acc);
   Partial second;
   second.s = dot;
-  second.s2 = 0.0;
+  second.s2 = sds;
   second.bad = -1;
   second = block_fold<kEwThreads>(second);
   if (threadIdx.x == 0) {
@@ -104,11 +123,12 @@ __global__ void __launch_bounds__(kEwThreads, StepBlocks<Op>::value)
   }
 }
 
-template <int VEC, int UNROLL, class Op> static int step_blocks_per_sm() {
+template <int VEC, int UNROLL, class Op, bool IPROX> static int step_blocks_per_sm() {
   static int cached = 0;  // per instantiation
   if (cached == 0) {
     int nb = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, step_kernel<VEC, UNROLL, Op>, kEwThreads, 0) != cudaSuccess ||
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, step_kernel<VEC, UNROLL, Op, IPROX>, kEwThreads, 0) !=
+            cudaSuccess ||
         nb < 1)
       nb = 1;
     cached = nb;
@@ -116,9 +136,9 @@ template <int VEC, int UNROLL, class Op> static int step_blocks_per_sm() {
   return cached;
 }
 
-// launch, fold the two slots, hand back (ψ(s), Σs², Σ∇f·s)
-template <class Op, class R>
-static int32_t step_run(spx_ctx* ctx, const Op& op, R nu, R* xsy, int64_t n, int kind, R lambda, double* out3) {
+// launch and fold the two slots into ctx->h_result: [0] = (ψ sum, Σs², flag), [1] = (Σ∇f·s, Σ d s² or 0)
+template <bool IPROX, class Op, class R>
+static int32_t step_launch(spx_ctx* ctx, const Op& op, R c, R* xsy, int64_t n) {
   constexpr int VECW = 16 / (int)sizeof(R);
   constexpr int UNROLL = Op::UNROLL;
   int nb = 0;
@@ -128,20 +148,25 @@ static int32_t step_run(spx_ctx* ctx, const Op& op, R nu, R* xsy, int64_t n, int
     const long long tile = (long long)kEwThreads * UNROLL;
     long long want = (nvec + tile - 1) / tile;
     if (want < 1) want = 1;
-    long long cap = (long long)ctx->sm_count *
-                    (vec ? step_blocks_per_sm<VECW, UNROLL, Op>() : step_blocks_per_sm<1, UNROLL, Op>());
+    long long cap = (long long)ctx->sm_count * (vec ? step_blocks_per_sm<VECW, UNROLL, Op, IPROX>()
+                                                    : step_blocks_per_sm<1, UNROLL, Op, IPROX>());
     if (cap > kMaxPartials) cap = kMaxPartials;
     nb = (int)(want < cap ? want : cap);
-    const R mnu = -nu;
     if (vec)
-      step_kernel<VECW, UNROLL, Op><<<nb, kEwThreads, 0, ctx->stream>>>(op, mnu, xsy, n, ctx->d_partials);
+      step_kernel<VECW, UNROLL, Op, IPROX><<<nb, kEwThreads, 0, ctx->stream>>>(op, c, xsy, n, ctx->d_partials);
     else
-      step_kernel<1, UNROLL, Op><<<nb, kEwThreads, 0, ctx->stream>>>(op, mnu, xsy, n, ctx->d_partials);
+      step_kernel<1, UNROLL, Op, IPROX><<<nb, kEwThreads, 0, ctx->stream>>>(op, c, xsy, n, ctx->d_partials);
     ctx->launches++;
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "step_kernel launch");
   }
-  int32_t st = finalize_partials(ctx, nb, 2, false);
+  return finalize_partials(ctx, nb, 2, false);
+}
+
+// the step around prox!: hand back (ψ(s), Σs², Σ∇f·s)
+template <class Op, class R>
+static int32_t step_run(spx_ctx* ctx, const Op& op, R nu, R* xsy, int64_t n, int kind, R lambda, double* out3) {
+  int32_t st = step_launch<false>(ctx, op, -nu, xsy, n);
   if (st != SPX_OK) return st;
   out3[0] = ctx->h_result[0].bad > 0 ? kInf : scale_value<R>(kind, lambda, ctx->h_result[0].s, 0);
   out3[1] = ctx->h_result[0].s2;
@@ -196,6 +221,72 @@ static int32_t step_box(spx_ctx* ctx, int32_t opc, int64_t n, R* s, R* xsy, cons
   if (opc == BOX_LHALF) return go(ProxLhalfBox<R, true>{});
   set_error("spx_step_box: unknown Box operator %d", (int)opc);
   return SPX_E_INVALID;
+}
+
+// ---- the step around iprox! (diagonal model: R2DH, TRDH) --------------------------------------------------------
+// The same pass with the iprox! functors: d = D + σ in R, s = iprox!(ψ, ∇f, d), and out4 = (ψ(s), Σs², Σ∇f·s, Σ d s²).
+#define SPX_ISTEP_COMMON_CHECKS()                                                  \
+  SPX_REQUIRE(ctx != nullptr, "null context");                                     \
+  SPX_REQUIRE(n >= 0, "n < 0");                                                    \
+  SPX_REQUIRE(out4 != nullptr, "null result array");                               \
+  SPX_REQUIRE(n == 0 || (s && xk && grad && D), "null device vector");             \
+  DeviceGuard guard__(ctx->device)
+
+static void istep_sums(const spx_ctx* ctx, double* out4) {
+  out4[1] = ctx->h_result[0].s2;
+  out4[2] = ctx->h_result[1].s;
+  out4[3] = ctx->h_result[1].s2;
+}
+
+template <class R>
+static int32_t istep_sep(spx_ctx* ctx, int32_t kind, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad,
+                         const R* D, double dshift, double lambda, int64_t* first_bad_d, double* out4) {
+  SPX_ISTEP_COMMON_CHECKS();
+  const R lam = (R)lambda;
+  auto go = [&](auto op) {
+    set_iprox(op, s, xk, sj, grad, D, lam);
+    int32_t st = step_launch<true>(ctx, op, (R)dshift, xsy, n);
+    if (st != SPX_OK) return st;
+    out4[0] = scale_value<R>(kind, lam, ctx->h_result[0].s, 0);
+    istep_sums(ctx, out4);
+    const long long bad = ctx->h_result[0].bad;  // first d[i] <= 0, as in iprox_sep (spx_elementwise.cu)
+    const long long idx = bad < 0 ? -1 : ((1ll << 62) - bad);
+    if (first_bad_d) *first_bad_d = idx;
+    if (idx >= 0) {
+      set_error("AssertionError: d[%lld] > 0", idx);
+      return SPX_E_ASSERT_D;
+    }
+    return SPX_OK;
+  };
+  if (kind == SPX_H_L1) return go(IproxL1<R, true>{});
+  if (kind == SPX_H_L0) return go(IproxL0<R, true>{});
+  set_error("spx_istep_sep: h kind %d has no iprox!", (int)kind);
+  return SPX_E_INVALID;
+}
+
+template <class R>
+static int32_t istep_box(spx_ctx* ctx, int32_t opc, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad,
+                         const R* D, double dshift, const spx_bound* l, const spx_bound* u, const spx_sel* sel,
+                         double lambda, double* out4) {
+  SPX_ISTEP_COMMON_CHECKS();
+  SPX_REQUIRE(l && u, "null bounds");
+  if (opc != BOX_L1 && opc != BOX_L0) {
+    set_error("spx_istep_box: Box operator %d has no iprox!", (int)opc);
+    return SPX_E_INVALID;
+  }
+  DevSel ds;
+  int32_t st = make_sel(sel, n, &ds);
+  if (st != SPX_OK) return st;
+  const R lam = (R)lambda;
+  auto go = [&](auto op) {
+    set_iprox_box(op, s, xk, sj, grad, D, (const R*)l->vec, (R)l->val, (const R*)u->vec, (R)u->val, ds, lam);
+    int32_t st = step_launch<true>(ctx, op, (R)dshift, xsy, n);
+    if (st != SPX_OK) return st;
+    out4[0] = ctx->h_result[0].bad > 0 ? kInf : scale_value<R>(box_kind(opc), lam, ctx->h_result[0].s, 0);
+    istep_sums(ctx, out4);
+    return SPX_OK;
+  };
+  return opc == BOX_L1 ? go(IproxL1Box<R, true>{}) : go(IproxL0Box<R, true>{});
 }
 
 // ---- the step around a prox! that is not one streaming pass (groups, top-r, ShiftedNormL1B2) ----------------------
@@ -290,6 +381,16 @@ using namespace spx;
   extern "C" int32_t spx_step_post_##SUF(spx_ctx* ctx, int64_t n, R* xsy, const R* xk, const R* sj, const R* s,       \
                                          const R* grad, double* out2) {                                               \
     return step_post<R>(ctx, n, xsy, xk, sj, s, grad, out2);                                                          \
+  }                                                                                                                   \
+  extern "C" int32_t spx_istep_sep_##SUF(spx_ctx* ctx, int32_t kind, int64_t n, R* s, R* xsy, const R* xk,            \
+                                         const R* sj, const R* grad, const R* D, double dshift, double lambda,        \
+                                         int64_t* first_bad_d, double* out4) {                                        \
+    return istep_sep<R>(ctx, kind, n, s, xsy, xk, sj, grad, D, dshift, lambda, first_bad_d, out4);                    \
+  }                                                                                                                   \
+  extern "C" int32_t spx_istep_box_##SUF(spx_ctx* ctx, int32_t op, int64_t n, R* s, R* xsy, const R* xk, const R* sj, \
+                                         const R* grad, const R* D, double dshift, const spx_bound* l,                \
+                                         const spx_bound* u, const spx_sel* sel, double lambda, double* out4) {       \
+    return istep_box<R>(ctx, op, n, s, xsy, xk, sj, grad, D, dshift, l, u, sel, lambda, out4);                        \
   }
 
 SPX_DEFINE_STEP(f64, double)

@@ -38,7 +38,7 @@ __all__ = [
     "ShiftedNormL0Box", "ShiftedRootNormLhalfBox", "ShiftedNormL1B2", "ShiftedIndBallL0", "ShiftedIndBallL0BInf",
     "ShiftedGroupNormL2", "ShiftedGroupNormL2Binf",
     "shifted", "shift_", "set_radius_", "set_bounds_", "prox_", "prox", "iprox_", "iprox", "prox_zero",
-    "iprox_zero", "step_", "StepResult", "context", "launch_count",
+    "iprox_zero", "step_", "StepResult", "istep_", "IStepResult", "context", "launch_count",
 ]
 
 _SUF = {torch.float64: "f64", torch.float32: "f32"}
@@ -296,6 +296,25 @@ class ShiftedProximableFunction:
                    _p(grad), C.c_double(self.h.lam), C.c_double(nu), out)
         return s, StepResult(out[0], math.sqrt(out[1]), out[2])
 
+    def istep_(self, s, grad, d, dshift=0.0, xsy=None):
+        raise NotImplementedError(f"iprox! is not defined for {type(self).__name__}")
+
+    def _istep_check(self, s, grad, d, xsy):
+        self._check(s, grad, ("s", "grad"))
+        _vec(d, self.xk, "d")
+        if xsy is not None:
+            _vec(xsy, self.xk, "xsy")
+
+    def _istep_sep(self, s, grad, d, dshift, xsy):
+        # spx_istep_sep_*: D + σ, iprox!, ψ(s), xk+sj+s, Σs², Σ∇f·s, Σ d s² in the one pass of the iprox!
+        self._istep_check(s, grad, d, xsy)
+        out = (C.c_double * 4)()
+        bad = C.c_int64()
+        sj = self.sj if self.shifted_twice else None  # ψ shifted once: NULL reads zeros (see _step_sep)
+        self._call("istep_sep", C.c_int32(self._H_KIND), C.c_int64(self.n), _p(s), _p(xsy), _p(self.xk), _p(sj),
+                   _p(grad), _p(d), C.c_double(dshift), C.c_double(self.h.lam), C.byref(bad), out)
+        return s, IStepResult(out[0], math.sqrt(out[1]), out[2], out[3])
+
     def __repr__(self):  # Base.show  (ShiftedProximalOperators.jl:123-133)
         return f"{type(self).__name__}(n={self.n}, dtype={self.xk.dtype}, shifted_twice={self.shifted_twice})"
 
@@ -312,6 +331,19 @@ class StepResult(tuple):
     gdots = property(lambda self: self[2])
 
 
+class IStepResult(tuple):
+    """(ψ(s), ‖s‖₂, ∇f·s, sᵀ(D + σ)s) of a fused solver step around iprox!."""
+    __slots__ = ()
+
+    def __new__(cls, psi, snorm, gdots, sds):
+        return super().__new__(cls, (psi, snorm, gdots, sds))
+
+    psi = property(lambda self: self[0])
+    snorm = property(lambda self: self[1])
+    gdots = property(lambda self: self[2])
+    sds = property(lambda self: self[3])
+
+
 def _psi_arg(want_value):
     out = C.c_double() if want_value else None
     return out, (C.byref(out) if want_value else None)
@@ -326,6 +358,9 @@ class ShiftedNormL1(ShiftedProximableFunction):
 
     def step_(self, s, grad, nu, xsy=None):
         return self._step_sep(s, grad, nu, xsy)
+
+    def istep_(self, s, grad, d, dshift=0.0, xsy=None):
+        return self._istep_sep(s, grad, d, dshift, xsy)
 
     def prox_(self, y, q, sigma, want_value=False):  # shiftedNormL1.jl:40-54
         self._check(y, q)
@@ -353,6 +388,9 @@ class ShiftedNormL0(ShiftedProximableFunction):
 
     def step_(self, s, grad, nu, xsy=None):
         return self._step_sep(s, grad, nu, xsy)
+
+    def istep_(self, s, grad, d, dshift=0.0, xsy=None):
+        return self._istep_sep(s, grad, d, dshift, xsy)
 
     def prox_(self, y, q, sigma, want_value=False):  # shiftedNormL0.jl:38-55
         self._check(y, q)
@@ -468,6 +506,17 @@ class _BoxBase(ShiftedProximableFunction):
                    _p(self.sj), _p(grad), C.byref(lb), C.byref(ub), self._sel.ref(), C.c_double(self.h.lam),
                    C.c_double(nu), out)
         return s, StepResult(out[0], math.sqrt(out[1]), out[2])
+
+    def istep_(self, s, grad, d, dshift=0.0, xsy=None):
+        if self._BOX_NAME == "lhalfbox":
+            raise NotImplementedError("iprox! is not defined for ShiftedRootNormLhalfBox")
+        self._istep_check(s, grad, d, xsy)
+        lb, ub = self._bounds()
+        out = (C.c_double * 4)()
+        self._call("istep_box", C.c_int32(_BOX_OP[self._BOX_NAME]), C.c_int64(self.n), _p(s), _p(xsy), _p(self.xk),
+                   _p(self.sj), _p(grad), _p(d), C.c_double(dshift), C.byref(lb), C.byref(ub), self._sel.ref(),
+                   C.c_double(self.h.lam), out)
+        return s, IStepResult(out[0], math.sqrt(out[1]), out[2], out[3])
 
     def __call__(self, y):  # shiftedNormL1Box.jl:70-82
         _vec(y, self.xk, "y")
@@ -802,6 +851,19 @@ def step_(s, psi, grad, nu, xsy=None):
     ShiftedNormL1 / L0 / RootNormLhalf and their Box / BInf forms; for the group, top-r and L1B2 types the sweeps are
     two passes around the type's own prox! (ShiftedProximableFunction.step_)."""
     return psi.step_(s, grad, nu, xsy)
+
+
+def istep_(s, psi, grad, d, dshift=0.0, xsy=None):
+    """Fused solver step around iprox! (extension): what an iteration of a diagonal quasi-Newton solver (R2DH, TRDH
+    of RegularizedOptimization.jl) wraps around its iprox!, in the one pass of the iprox! itself --
+
+        d = D .+ σ;  iprox!(s, ψ, ∇f, d);  xsy .= xk .+ sj .+ s (if given);  ψ(s);  ‖s‖₂;  ∇f's;  sᵀ d s
+
+    with D = `d` and σ = `dshift`.  Returns (s, IStepResult(psi, snorm, gdots, sds)).  `s` is bit-identical to
+    iprox_(s, ψ, grad, D + σ) with D + σ rounded to the vector's type; the sums are in Float64.  ShiftedNormL1 /
+    ShiftedNormL0 raise AssertionError on a d[i] <= 0, as their iprox! does.  Defined for the types with an iprox!:
+    ShiftedNormL1, ShiftedNormL0, ShiftedNormL1Box, ShiftedNormL0Box.  `s` may be `grad` and `xsy` may be ψ.xk."""
+    return psi.istep_(s, grad, d, dshift, xsy)
 
 
 def prox_zero(q, l, u):

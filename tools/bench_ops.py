@@ -129,6 +129,36 @@ def main():
             torch.add(xk, y, out=xsy)
             return v, float(torch.linalg.vector_norm(y)), float(torch.dot(q, y))
         timeit("step_l1_once_unfused", unfused, 4 * R, note="prox! + ψ(s) + 4 BLAS-1 sweeps, same result")
+    # fused step around iprox! (diagonal model: R2DH / TRDH): D + σ, iprox!, ψ(s), xk+sj+s, ‖s‖, ∇f's, sᵀ(D+σ)s in one
+    # pass; σ = `sigma`, D = dpos for the unboxed forms (their iprox! asserts d > 0), the C2 mix d for the Box forms
+    istep_names = ["istep_l1_once", "istep_l1", "istep_l0box_vec", "istep_l1box_scalar", "istep_l0box_vec_unfused"]
+    if any(re.search(args.only, nm) for nm in istep_names):
+        xsy = torch.empty(n, dtype=tdt, device=dev)
+        once = sp.shifted(sp.NormL1(lam), xk)
+        timeit("istep_l1_once", lambda: sp.istep_(y, once, q, dpos, sigma, xsy=xsy), 5 * R,
+               note="ψ shifted once: 3 reads + 2 writes")
+        timeit("istep_l1", lambda psi=two(sp.NormL1(lam)): sp.istep_(y, psi, q, dpos, sigma, xsy=xsy), 6 * R)
+        l0box = two(sp.NormL0(lam), l, u)
+        timeit("istep_l0box_vec", lambda: sp.istep_(y, l0box, q, d, sigma, xsy=xsy), 8 * R)
+        timeit("istep_l1box_scalar", lambda psi=two(sp.NormL1(lam), -1.0, 1.0): sp.istep_(y, psi, q, d, sigma, xsy=xsy),
+               6 * R)
+
+        def iunfused(s=y, out=xsy):  # the same step as separate sweeps (torch for the BLAS-1 parts)
+            dd = d + sigma
+            sp.iprox_(s, l0box, q, dd)
+            v = l0box(s)
+            torch.add(xk, sj, out=out)
+            out.add_(s)
+            return v, float(torch.linalg.vector_norm(s)), float(torch.dot(q, s)), float(torch.dot(dd * s, s))
+        if re.search(args.only, "istep_l0box_vec_unfused"):
+            y2, xsy2 = torch.empty_like(y), torch.empty_like(y)
+            _, r = sp.istep_(y, l0box, q, d, sigma, xsy=xsy)
+            r2 = iunfused(y2, xsy2)
+            same = torch.equal(y, y2) and torch.equal(xsy, xsy2)
+            print(f"istep_l0box_vec vs unfused: s and xsy bit-identical: {same}; scalars {tuple(r)} vs {r2}", flush=True)
+            del y2, xsy2
+        timeit("istep_l0box_vec_unfused", iunfused, 8 * R,
+               note="D+σ, iprox!, ψ(s), xk+sj+s, ‖s‖, ∇f's, sᵀds as separate sweeps, same result")
     # L1B2 (ball active: Δ = half the unconstrained norm)
     if re.search(args.only, "prox_l1b2"):
         psi0 = two(sp.NormL1(lam), 1e30, sp.NormL2(1.0))
