@@ -391,6 +391,17 @@ typedef struct spx_box_job_f32 {
   int32_t spx_step_groupl2_##SUF(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj,    \
                                  const R* grad, int64_t ngroups, const int64_t* offs,                \
                                  const R* lambda_g, double nu, double* out3_host);                   \
+  /* The whole step of ShiftedGroupNormL2Binf (shiftedGroupNormL2Binf.jl:67-119) in one call: ONE   */ \
+  /* pass when the layout is uniform (n == ngroups m, m in {16, 32, 64, 128, 256}, offs == {0, m,    */ \
+  /* 2m, ...}, ngroups > 1, 16-byte aligned vectors), the three calls above otherwise.  s is bit for */ \
+  /* bit prox!(s, ψ, (-nu) .* grad, nu).  out3_host = {ψ(s) of shiftedGroupNormL2Binf.jl:34-39 (Inf  */ \
+  /* when sj + s leaves the ball of 1.1 delta), Σ s², Σ grad·s}, the sums in Float64.  Contract as   */ \
+  /* for spx_step_groupl2; the call synchronises, the scalars are all-reduced when the context       */ \
+  /* reduces scalars.                                                                                */ \
+  int32_t spx_step_groupl2binf_##SUF(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk,             \
+                                     const R* sj, const R* grad, int64_t ngroups,                    \
+                                     const int64_t* offs, const R* lambda_g, double nu,              \
+                                     double delta, double* out3_host);                               \
   int32_t spx_step_post_##SUF(spx_ctx* ctx, int64_t n, R* xsy, const R* xk, const R* sj, const R* s, \
                               const R* grad, double* out2_host);                                     \
   /* ------------------------------ host-buffer entry points (end-to-end path) */              \

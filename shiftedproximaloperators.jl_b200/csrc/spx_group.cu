@@ -976,8 +976,11 @@ template <class R, int L> struct UTile {
     }
     cp_async_commit();
   }
-  // the round whose copies were enqueued last
-  __device__ __forceinline__ void take(long long round, long long ngroups, int lane, uint32_t sbase, int sjbuf) {
+  // the round whose copies were enqueued last.  STEP: the q plane holds ∇f, and q = (-ν) ∇f is formed here in R,
+  // as spx_step_pre writes it
+  template <bool STEP = false>
+  __device__ __forceinline__ void take(long long round, long long ngroups, int lane, uint32_t sbase, int sjbuf,
+                                       R mnu = R(0)) {
     cp_async_wait<0>();
     valid = lane_valid(round, ngroups, lane);
     base = lane_base(round, lane);
@@ -998,6 +1001,7 @@ template <class R, int L> struct UTile {
     for (int c = 0; c < NCH; ++c)
 #pragma unroll
       for (int e = 0; e < VEC; ++e) {
+        if constexpr (STEP) pq[c].v[e] = mnu * pq[c].v[e];
         sol[c * VEC + e] = (pq[c].v[e] + px[c].v[e]) + ps[c].v[e];  // :80
         xkr[c * VEC + e] = px[c].v[e];
       }
@@ -1245,31 +1249,69 @@ __device__ __forceinline__ bool binf_fast_search_entry(const UTile<float, L>& t,
   return binf_fast_search<float, L>(t.sol, t.xkr, t.sol, t.xkr, t.valid, lam, sigma, delta, n_out, fp_out, zero_out);
 }
 
+// the first round among i, i + stride, i + 2 stride, ... (below nrounds) that `declined` marks; nrounds when there is none
+__device__ __forceinline__ long long first_declined(const unsigned char* declined, long long i, long long stride,
+                                                    long long nrounds, int lane) {
+  for (; i < nrounds; i += 32 * stride) {
+    const long long r = i + lane * stride;
+    const unsigned hit = __ballot_sync(0xffffffffu, r < nrounds && declined[r] != 0);
+    if (hit != 0u) return i + (long long)(__ffs(hit) - 1) * stride;
+  }
+  return nrounds;
+}
+
 #ifndef SPX_GU_MINB
 #define SPX_GU_MINB 3
 #endif
 // FAST: rounds grid-stride, failures appended to the work list.  !FAST: the listed rounds, bracketing search.
-template <class R, int L, bool FAST>
-__global__ void __launch_bounds__(kGroupThreads, FAST ? SPX_GU_MINB : 2)
+// STEP (spx_step_groupl2binf): y = s, q = ∇f; the store loop also writes xsy = (xk + sj) + s and sums ψ(s), Σ s² and
+// Σ ∇f·s per CTA into part0[blockIdx.x] = {ψ, Σ s², infeasible} and part1[blockIdx.x] = {Σ ∇f·s, 0, redo}.  The FAST
+// form also marks its declined rounds in `declined`, and the !FAST form walks those in round order on the same static
+// round-to-warp map as the FAST one (not in the order of the work list, which is the order of atomicAdd), so that the
+// sums come out the same on every call.  With the uniform flag at 0 both only raise `redo`.
+// The Float64 STEP forms hold 8 more doubles per lane through the store loop and run with one CTA per SM fewer than
+// the prox! forms (3 -> 2 and 2 -> 1), the occupancy at which they do not spill.
+template <class R, int L, bool FAST, bool STEP = false>
+__global__ void __launch_bounds__(kGroupThreads, (FAST ? SPX_GU_MINB : 2) - (STEP && sizeof(R) == 8 ? 1 : 0))
     group_l2binf_uniform_kernel(R* y, const R* xk, const R* sj, const R* q, long long ngroups,
                                 const R* __restrict__ lambda_g, R sigma, R delta, UDiv<R> by_sigma,
-                                const unsigned* __restrict__ uniform_flag, unsigned* wl_count, unsigned* wl_rounds) {
-  if (*uniform_flag == 0u) return;
+                                const unsigned* __restrict__ uniform_flag, unsigned* wl_count, unsigned* wl_rounds,
+                                R* xsy, R mnu, double rad, unsigned char* declined, Partial* part0, Partial* part1) {
+  if (*uniform_flag == 0u) {
+    if constexpr (STEP) {
+      if (threadIdx.x == 0) {
+        part0[blockIdx.x] = Partial{0.0, 0.0, -1};
+        part1[blockIdx.x] = Partial{0.0, 0.0, 1};
+      }
+    }
+    return;
+  }
   constexpr int GPW = 32 / L;
   constexpr int VEC = UVec<R>::VEC, NCH = UVec<R>::NCH;
+  constexpr bool SCAN = STEP && !FAST;  // walk the declined rounds of the static map
   const int lane = threadIdx.x & 31;
   const long long warp = ((long long)blockIdx.x * kGroupThreads + threadIdx.x) >> 5;
   const long long nwarps = ((long long)gridDim.x * kGroupThreads) >> 5;
-  const long long nrounds = FAST ? (ngroups + GPW - 1) / GPW : (long long)*wl_count;
+  const long long nrounds = FAST ? (ngroups + GPW - 1) / GPW
+                            : SCAN ? (*wl_count == 0u ? 0 : (ngroups + GPW - 1) / GPW)
+                                   : (long long)*wl_count;
   extern __shared__ __align__(16) unsigned char uni_smem[];
   const uint32_t sbase = (uint32_t)__cvta_generic_to_shared(uni_smem) + (uint32_t)(threadIdx.x >> 5) * UTile<R, L>::kWarpBytes;
-  auto round_of = [&](long long i) -> long long { return FAST ? i : (long long)wl_rounds[i]; };
+  auto round_of = [&](long long i) -> long long { return FAST || SCAN ? i : (long long)wl_rounds[i]; };
+  // STEP: each thread's running ψ, Σ s² and Σ ∇f·s wait in shared memory between rounds, so that the search keeps
+  // its registers
+  __shared__ double uni_acc[STEP ? 3 : 1][STEP ? kGroupThreads : 1];
+  if constexpr (STEP) uni_acc[0][threadIdx.x] = uni_acc[1][threadIdx.x] = uni_acc[2][threadIdx.x] = 0.0;
+  bool infeasible = false;
   int sjbuf = 0;
-  if (warp < nrounds) UTile<R, L>::prefetch(round_of(warp), ngroups, lane, xk, sj, q, sbase, 0);
-  for (long long it = warp; it < nrounds; it += nwarps, sjbuf ^= 1) {
+  long long first = warp;
+  if constexpr (SCAN) first = first_declined(declined, warp, nwarps, nrounds, lane);
+  if (first < nrounds) UTile<R, L>::prefetch(round_of(first), ngroups, lane, xk, sj, q, sbase, 0);
+  for (long long it = first; it < nrounds; it += nwarps, sjbuf ^= 1) {
     const long long round = round_of(it);
+    if constexpr (SCAN) it = first_declined(declined, it + nwarps, nwarps, nrounds, lane) - nwarps;  // the next round taken is it + nwarps
     UTile<R, L> t;
-    t.take(round, ngroups, lane, sbase, sjbuf);
+    t.template take<STEP>(round, ngroups, lane, sbase, sjbuf, mnu);
     // the next round's copies go out now and land while this one is solved (q and xk planes are free again: their
     // contents sit in registers; sj goes to the other sj plane)
     if (it + nwarps < nrounds) UTile<R, L>::prefetch(round_of(it + nwarps), ngroups, lane, xk, sj, q, sbase, sjbuf ^ 1);
@@ -1281,7 +1323,10 @@ __global__ void __launch_bounds__(kGroupThreads, FAST ? SPX_GU_MINB : 2)
     if constexpr (FAST) {
       const bool ok = binf_fast_search_entry<L>(t, lam, sigma, delta, nroot, fp, zero_out);
       if (__any_sync(0xffffffffu, !ok)) {
-        if (lane == 0) wl_rounds[atomicAdd(wl_count, 1u)] = (unsigned)round;
+        if (lane == 0) {
+          wl_rounds[atomicAdd(wl_count, 1u)] = (unsigned)round;
+          if constexpr (STEP) declined[round] = 1;
+        }
         continue;
       }
     } else {
@@ -1315,11 +1360,49 @@ __global__ void __launch_bounds__(kGroupThreads, FAST ? SPX_GU_MINB : 2)
       const R ulps = jl_max(R(2), jl_min(R(16), gap * (R)(1.0 / (double)sl)));
       const bool accepted = zero_out || !t.valid || (jl_abs(res) <= ulps * Eps<R>::value * nroot * (R)fp);
       if (__any_sync(0xffffffffu, !accepted)) {
-        if (lane == 0) wl_rounds[atomicAdd(wl_count, 1u)] = (unsigned)round;
+        if (lane == 0) {
+          wl_rounds[atomicAdd(wl_count, 1u)] = (unsigned)round;
+          if constexpr (STEP) declined[round] = 1;
+        }
         continue;
       }
     }
-    if (t.valid) {
+    if constexpr (STEP) {
+      // ∇f of this round again for Σ ∇f·s: its q plane already holds the next round, and the copy of one round
+      // ago left it in L2
+      double vv = 0.0, ss2 = 0.0, dot = 0.0;
+      if (t.valid) {
+        Pack<R, VEC> pg[NCH];
+#pragma unroll
+        for (int c = 0; c < NCH; ++c) ld_stream(q + t.base + c * (L * VEC), pg[c]);
+#pragma unroll
+        for (int c = 0; c < NCH; ++c) {
+          Pack<R, VEC> ps, po, px;
+          lds16(sbase + (2u + (uint32_t)sjbuf) * UTile<R, L>::kPlane + (uint32_t)(c * 32 + lane) * 16u, ps);
+#pragma unroll
+          for (int e = 0; e < VEC; ++e) {
+            const int j = c * VEC + e;
+            const R o = zero_out ? R(0) : alpha * w[j];
+            const R xs = t.xkr[j] + ps.v[e];
+            po.v[e] = o - xs;
+            px.v[e] = xs + po.v[e];  // the generic ψ argument (xk + sj) + s
+            // ψ(s) in the association of group_value_kernel: w = sj + s against the ball, v = w + xk
+            const R wv = ps.v[e] + po.v[e];
+            infeasible = infeasible || (double)wv < -rad || (double)wv > rad;
+            const R v = wv + t.xkr[j];
+            vv += (double)v * (double)v;
+            ss2 = __fma_rn((double)po.v[e], (double)po.v[e], ss2);
+            dot = __fma_rn((double)pg[c].v[e], (double)po.v[e], dot);
+          }
+          st_stream(y + t.base + c * (L * VEC), po);
+          if (xsy != nullptr) st_stream(xsy + t.base + c * (L * VEC), px);
+        }
+      }
+      vv = usum<L>(vv);
+      if (t.valid && lane % L == 0) uni_acc[0][threadIdx.x] += (double)(lam * (R)sqrt_fast(vv));  // λ_g ‖v_g‖  groupNormL2.jl:36
+      uni_acc[1][threadIdx.x] += ss2;
+      uni_acc[2][threadIdx.x] += dot;
+    } else if (t.valid) {
 #pragma unroll
       for (int c = 0; c < NCH; ++c) {
         Pack<R, VEC> ps, po;
@@ -1332,6 +1415,16 @@ __global__ void __launch_bounds__(kGroupThreads, FAST ? SPX_GU_MINB : 2)
         }
         st_stream(y + t.base + c * (L * VEC), po);
       }
+    }
+  }
+  if constexpr (STEP) {
+    Partial p{uni_acc[0][threadIdx.x], uni_acc[1][threadIdx.x], infeasible ? 1 : -1};
+    p = block_fold<kGroupThreads>(p);
+    Partial p2{uni_acc[2][threadIdx.x], 0.0, -1};
+    p2 = block_fold<kGroupThreads>(p2);
+    if (threadIdx.x == 0) {
+      part0[blockIdx.x] = p;
+      part1[blockIdx.x] = p2;
     }
   }
 }
@@ -2189,37 +2282,71 @@ static int32_t launch_group_l2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const
   return join_side_streams(ctx);
 }
 
-template <class R, int L>
+// the operands of the step form of the uniform kernels (spx_step_groupl2binf); nblocks returns the CTAs of both
+// launches, whose two partial slots each lie at d_partials[k * nblocks ...]
+template <class R> struct UniformStep {
+  R* xsy;
+  R mnu;
+  double rad;
+  unsigned char* declined;
+  int nblocks;
+};
+
+template <class R, int L, bool STEP>
 static int32_t launch_uniform_binf_L(spx_ctx* ctx, R* y, const R* xk, const R* sj, const R* q, int64_t ngroups,
                                      const R* lambda_g, R sigma, R delta, UDiv<R> by_sigma, const unsigned* uniform_flag,
-                                     unsigned* wl_count, unsigned* wl_rounds) {
+                                     unsigned* wl_count, unsigned* wl_rounds, UniformStep<R>* step) {
   const long long nrounds = (ngroups + (32 / L) - 1) / (32 / L);
   const long long want = (nrounds + (kGroupThreads / 32) - 1) / (kGroupThreads / 32);
   const size_t smem = (size_t)(kGroupThreads / 32) * UTile<R, L>::kWarpBytes;
+  auto fast = group_l2binf_uniform_kernel<R, L, true, STEP>;
+  auto list = group_l2binf_uniform_kernel<R, L, false, STEP>;
   int grid_fast = 0, grid_list = 0;
-  int32_t st = grid_for(ctx, (const void*)group_l2binf_uniform_kernel<R, L, true>, kGroupThreads, smem, want, kGridMax,
-                        true, &grid_fast);
-  if (st == SPX_OK)
-    st = grid_for(ctx, (const void*)group_l2binf_uniform_kernel<R, L, false>, kGroupThreads, smem, want, kGridMax, true,
-                  &grid_list);
+  int32_t st = grid_for(ctx, (const void*)fast, kGroupThreads, smem, want, kGridMax, true, &grid_fast);
+  if (st == SPX_OK) st = grid_for(ctx, (const void*)list, kGroupThreads, smem, want, kGridMax, true, &grid_list);
   if (st != SPX_OK) return st;
-  group_l2binf_uniform_kernel<R, L, true><<<grid_fast, kGroupThreads, smem, ctx->stream>>>(
-      y, xk, sj, q, ngroups, lambda_g, sigma, delta, by_sigma, uniform_flag, wl_count, wl_rounds);
-  group_l2binf_uniform_kernel<R, L, false><<<grid_list, kGroupThreads, smem, ctx->stream>>>(
-      y, xk, sj, q, ngroups, lambda_g, sigma, delta, by_sigma, uniform_flag, wl_count, wl_rounds);
+  UniformStep<R> a{nullptr, R(0), 0.0, nullptr, 0};
+  Partial *p0 = nullptr, *p1 = nullptr;
+  if constexpr (STEP) {
+    step->nblocks = grid_fast + grid_list;
+    a = *step;
+    p0 = ctx->d_partials;
+    p1 = ctx->d_partials + step->nblocks;
+  }
+  fast<<<grid_fast, kGroupThreads, smem, ctx->stream>>>(y, xk, sj, q, ngroups, lambda_g, sigma, delta, by_sigma,
+                                                        uniform_flag, wl_count, wl_rounds, a.xsy, a.mnu, a.rad,
+                                                        a.declined, p0, p1);
+  list<<<grid_list, kGroupThreads, smem, ctx->stream>>>(y, xk, sj, q, ngroups, lambda_g, sigma, delta, by_sigma,
+                                                        uniform_flag, wl_count, wl_rounds, a.xsy, a.mnu, a.rad,
+                                                        a.declined, STEP ? p0 + grid_fast : nullptr,
+                                                        STEP ? p1 + grid_fast : nullptr);
   return SPX_OK;
 }
-template <class R>
+template <class R, bool STEP = false>
 static int32_t launch_uniform_binf(spx_ctx* ctx, int L, R* y, const R* xk, const R* sj, const R* q, int64_t ngroups,
                                    const R* lambda_g, R sigma, R delta, UDiv<R> by_sigma, const unsigned* uniform_flag,
-                                   unsigned* wl_count, unsigned* wl_rounds) {
+                                   unsigned* wl_count, unsigned* wl_rounds, UniformStep<R>* step = nullptr) {
   switch (L) {
-#define SPX_UL(LL) \
-  case LL: return launch_uniform_binf_L<R, LL>(ctx, y, xk, sj, q, ngroups, lambda_g, sigma, delta, by_sigma, uniform_flag, wl_count, wl_rounds);
+#define SPX_UL(LL)                                                                                                   \
+  case LL:                                                                                                           \
+    return launch_uniform_binf_L<R, LL, STEP>(ctx, y, xk, sj, q, ngroups, lambda_g, sigma, delta, by_sigma,         \
+                                              uniform_flag, wl_count, wl_rounds, step);
     SPX_UL(2) SPX_UL(4) SPX_UL(8) SPX_UL(16) SPX_UL(32)
 #undef SPX_UL
     default: return SPX_OK;
   }
+}
+
+// The uniform kernels' conditions that the host can check (whether offs is {0, m, 2m, ...} is checked on the device):
+// n == ngroups m with m = 8 L, 16-byte aligned vectors, and σ, Δ far enough inside the normal range for the fast
+// searches' branch-free quotients (sol/σ).
+static bool binf_sigma_ok(double sigma, double delta) {
+  return std::isfinite(sigma) && std::fabs(sigma) > 1e-30 && std::fabs(sigma) < 1e30 && std::isfinite(delta) &&
+         std::fabs(delta) < 1e30;
+}
+static bool uniform_binf_candidate(int64_t n, int64_t m, bool aligned, double sigma, double delta) {
+  return binf_sigma_ok(sigma, delta) && aligned && (m == 16 || m == 32 || m == 64 || m == 128 || m == 256) &&
+         n < (int64_t(1) << 39);
 }
 
 // ctx->d_scratch during a GroupNormL2Binf prox!: a head that every call clears, the work list of the uniform kernels at
@@ -2266,9 +2393,8 @@ static int32_t prox_group(spx_ctx* ctx, bool binf, int64_t n, R* y, const R* xk,
     const int64_t m = ngroups > 0 && n % ngroups == 0 ? n / ngroups : 0;
     const bool aligned = (((uintptr_t)y | (uintptr_t)xk | (uintptr_t)sj | (uintptr_t)q) & 15u) == 0;
     // the fast searches take sol/σ through the branch-free quotient: σ far inside the normal range only
-    const bool sigma_ok = std::isfinite(sigma) && std::fabs(sigma) > 1e-30 && std::fabs(sigma) < 1e30 &&
-                          std::isfinite(delta) && std::fabs(delta) < 1e30;
-    const bool uni = sigma_ok && aligned && (m == 16 || m == 32 || m == 64 || m == 128 || m == 256) && n < (int64_t(1) << 39);
+    const bool sigma_ok = binf_sigma_ok(sigma, delta);
+    const bool uni = uniform_binf_candidate(n, m, aligned, sigma, delta);
     const size_t done_off = BinfScratch::done_offset(uni ? (n + kRoundElems - 1) / kRoundElems : 0);
     st = ensure_scratch(ctx, done_off + (size_t)ngroups + 256);
     if (st != SPX_OK) return st;
@@ -2514,6 +2640,69 @@ static int32_t step_groupl2(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, 
   return SPX_OK;
 }
 
+// ---- the solver step of ShiftedGroupNormL2Binf ---------------------------------------------------------------------
+//     q = (-ν) ∇f;  prox!(s, ψ, q, ν);  xsy = (xk + sj) + s;  ψ(s) (Inf outside the ball of 1.1Δ);  Σ s²;  Σ ∇f·s
+// A uniform layout (the host conditions of prox_group's uniform kernels, and more than one group) runs it in the ONE
+// pass of the step form of group_l2binf_uniform_kernel: s is bit for bit what prox! writes.  When the device finds
+// offs is not {0, m, 2m, ...} after all, the kernels only raise the redo flag (it travels in the folded slots, so every
+// rank of a sharded vector sees it) and the call is redone in the composed form, which every other layout takes at
+// once: spx_step_pre, prox! in place with ψ(s) from its value pass, spx_step_post.
+template <class R>
+static int32_t step_groupl2binf(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad,
+                                int64_t ngroups, const int64_t* offs, const R* lambda_g, double nu, double delta,
+                                double* out3) {
+  SPX_REQUIRE(ctx != nullptr, "null context");
+  SPX_REQUIRE(n >= 0 && ngroups >= 0, "negative size");
+  SPX_REQUIRE(out3 != nullptr, "null result array");
+  SPX_REQUIRE(ngroups == 0 || n == 0 || (s && xk && sj && grad && offs && lambda_g), "null device vector");
+  SPX_REQUIRE(s != grad || n == 0, "s must not alias grad");
+  DeviceGuard g(ctx->device);
+  out3[0] = out3[1] = out3[2] = 0.0;
+  if (ngroups == 0 || n == 0) return SPX_OK;
+  const int64_t m = n % ngroups == 0 ? n / ngroups : 0;
+  const bool aligned = (((uintptr_t)s | (uintptr_t)xsy | (uintptr_t)xk | (uintptr_t)sj | (uintptr_t)grad) & 15u) == 0;
+  if (ngroups > 1 && uniform_binf_candidate(n, m, aligned, nu, delta)) {
+    const int64_t nrounds = (n + kRoundElems - 1) / kRoundElems;
+    const size_t declined_off = BinfScratch::done_offset(nrounds);
+    int32_t st = ensure_scratch(ctx, declined_off + (size_t)nrounds + 256);
+    if (st != SPX_OK) return st;
+    BinfScratch* const scratch = (BinfScratch*)ctx->d_scratch;
+    unsigned* const uniform_flag = &scratch->head.uniform_flag;
+    UniformStep<R> step{xsy, -(R)nu, 1.1 * (double)(R)delta, (unsigned char*)ctx->d_scratch + declined_off, 0};
+    SPX_CUDA(cudaMemsetAsync(&scratch->head, 0, sizeof(BinfScratch::Head), ctx->stream));
+    SPX_CUDA(cudaMemsetAsync(uniform_flag, 1, sizeof(unsigned), ctx->stream));
+    SPX_CUDA(cudaMemsetAsync(step.declined, 0, (size_t)nrounds, ctx->stream));
+    const int cgrid = (int)std::min<int64_t>((ngroups + 256) / 256, (int64_t)ctx->sm_count * 8);
+    group_uniform_check_kernel<<<cgrid, 256, 0, ctx->stream>>>((const long long*)offs, ngroups, m, uniform_flag);
+    UDiv<R> by_sigma;
+    by_sigma.set((R)nu);
+    st = launch_uniform_binf<R, true>(ctx, (int)(m / kEPL), s, xk, sj, grad, ngroups, lambda_g, (R)nu, (R)delta,
+                                      by_sigma, uniform_flag, &scratch->head.wl_count, scratch->wl_rounds, &step);
+    if (st != SPX_OK) return st;
+    ctx->launches += 3;
+    SPX_CUDA(cudaGetLastError());
+    st = finalize_partials(ctx, step.nblocks, 2, false);
+    if (st != SPX_OK) return st;
+    if (ctx->h_result[1].bad <= 0) {
+      // the reference accumulates ψ in R: one rounding to R here, as value_group_binf
+      out3[0] = ctx->h_result[0].bad > 0 ? std::numeric_limits<double>::infinity() : (double)(R)ctx->h_result[0].s;
+      out3[1] = ctx->h_result[0].s2;
+      out3[2] = ctx->h_result[1].s;
+      return SPX_OK;
+    }  // else: offs was rewritten after validation and is no longer uniform -- redo the call the long way
+  }
+  int32_t st = step_pre<R>(ctx, n, s, grad, nu);
+  if (st != SPX_OK) return st;
+  st = prox_group<R>(ctx, true, n, s, xk, sj, s, ngroups, offs, lambda_g, nu, delta, &out3[0]);
+  if (st != SPX_OK) return st;
+  double out2[2] = {0.0, 0.0};
+  st = step_post<R>(ctx, n, xsy, xk, sj, s, grad, out2);
+  if (st != SPX_OK) return st;
+  out3[1] = out2[0];
+  out3[2] = out2[1];
+  return SPX_OK;
+}
+
 }  // namespace spx
 
 using namespace spx;
@@ -2605,6 +2794,11 @@ extern "C" int32_t spx_group_validate_offsets(spx_ctx* ctx, int64_t n, int64_t n
                                             const R* grad, int64_t ngroups, const int64_t* offs,                 \
                                             const R* lambda_g, double nu, double* out3) {                        \
     return step_groupl2<R>(ctx, n, s, xsy, xk, sj, grad, ngroups, offs, lambda_g, nu, out3);                     \
+  }                                                                                                              \
+  extern "C" int32_t spx_step_groupl2binf_##SUF(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, \
+                                                const R* grad, int64_t ngroups, const int64_t* offs,             \
+                                                const R* lambda_g, double nu, double delta, double* out3) {      \
+    return step_groupl2binf<R>(ctx, n, s, xsy, xk, sj, grad, ngroups, offs, lambda_g, nu, delta, out3);          \
   }
 
 SPX_DEFINE_GROUP(f64, double)

@@ -699,6 +699,20 @@ class ShiftedGroupNormL2Binf(_GroupBase):
                    C.byref(out))
         return out.value
 
+    def step_(self, s, grad, nu, xsy=None):
+        """spx_step_groupl2binf_*: the whole step in one pass on a uniform layout (n == ngroups m, m = 16 ... 256, the
+        C4 shape), the two passes around prox! otherwise (decided in the library)."""
+        self._check(s, grad, ("s", "grad"))
+        if xsy is not None:
+            _vec(xsy, self.xk, "xsy")
+        if s.numel() > 0 and s.data_ptr() == grad.data_ptr():
+            raise ValueError("step_: s must not alias grad")
+        out = (C.c_double * 3)()
+        self._call("step_groupl2binf", C.c_int64(self.n), _p(s), _p(xsy), _p(self.xk), _p(self.sj), _p(grad),
+                   C.c_int64(self.ngroups), _p(self._offs), _p(self._lam_g), C.c_double(nu), C.c_double(self.Delta),
+                   out)
+        return s, StepResult(out[0], math.sqrt(out[1]), out[2])
+
 
 # ------------------------------------------------------------------- verbs ---
 _PLAIN = {NormL1: ShiftedNormL1, NormL0: ShiftedNormL0, RootNormLhalf: ShiftedRootNormLhalf}

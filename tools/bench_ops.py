@@ -176,7 +176,8 @@ def main():
     # groups of 64 (and ragged)
     for gname in ("g64", "ragged"):
         names = [f"prox_groupl2_{gname}", f"value_groupl2_{gname}", f"prox_groupl2binf_{gname}",
-                 "prox_groupl2binf_g64_biglambda", "step_groupl2_g64"]
+                 "prox_groupl2binf_g64_biglambda", "step_groupl2_g64", "step_groupl2binf_g64",
+                 "step_groupl2binf_g64_composed", "step_groupl2binf_g64_biglambda"]
         if not any(re.search(args.only, nm) for nm in names):
             continue
         if gname == "g64":
@@ -208,6 +209,26 @@ def main():
             psil = sp.shifted(sp.shifted(hb, xk, 0.5, sp.NormLinf(1.0)), sj)
             timeit("prox_groupl2binf_g64_biglambda", lambda psi=psil: sp.prox_(y, psi, q, 0.3), 4 * R,
                    note="lambda_g x 200")
+            # the one-pass step against the base-class composition of the same ψ (spx_step_pre, prox! in place with
+            # ψ(s) from its value pass, spx_step_post), alternated three times: the comparison is what these rows are for
+            if any(re.search(args.only, nm) for nm in ("step_groupl2binf_g64", "step_groupl2binf_g64_biglambda")):
+                xsy_b = torch.empty_like(y)
+                s2, xsy2 = torch.empty_like(y), torch.empty_like(y)
+                _, r = sp.step_(y, psib, q, 0.3, xsy=xsy_b)
+                _, r2 = sp.ShiftedProximableFunction.step_(psib, s2, q, 0.3, xsy=xsy2)
+                same = torch.equal(y, s2) and torch.equal(xsy_b, xsy2)
+                print(f"step_groupl2binf_g64 vs composed: s and xsy bit-identical: {same}; scalars {tuple(r)} vs "
+                      f"{tuple(r2)}", flush=True)
+                del s2, xsy2
+                for _ in range(3):
+                    timeit("step_groupl2binf_g64", lambda: sp.step_(y, psib, q, 0.3, xsy=xsy_b), 5 * R,
+                           note="spx_step_groupl2binf: one pass; alg. bytes = 3 reads + 2 writes")
+                    timeit("step_groupl2binf_g64_composed",
+                           lambda: sp.ShiftedProximableFunction.step_(psib, y, q, 0.3, xsy=xsy_b), 5 * R,
+                           note="step_pre, prox! in place + ψ pass, step_post; alg. bytes as above")
+                timeit("step_groupl2binf_g64_biglambda", lambda: sp.step_(y, psil, q, 0.3, xsy=xsy_b), 5 * R,
+                       note="lambda_g x 200")
+                del xsy_b
     # top-r batch: problems of 65536, r = 1024
     if any(re.search(args.only, nm) for nm in ("prox_indballl0_batch", "prox_indballl0binf_batch", "prox_indballl0_single")):
         pn = 65536
