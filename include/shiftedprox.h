@@ -402,6 +402,20 @@ typedef struct spx_box_job_f32 {
                                      const R* sj, const R* grad, int64_t ngroups,                    \
                                      const int64_t* offs, const R* lambda_g, double nu,              \
                                      double delta, double* out3_host);                               \
+  /* The whole step of ShiftedIndBallL0 (shiftedIndBallL0.jl:54-72) and ShiftedIndBallL0BInf       */ \
+  /* (binf != 0, shiftedIndBallL0BInf.jl:73-95) for nprob problems of length n back to back: ONE     */ \
+  /* pass of the stream top-r kernel when spx_prox_indballl0 would take its stream form (16-byte    */ \
+  /* aligned vectors, n % 8 == 0, 4096 <= n <= 131072, 0 < r < n, nprob >= 2 x the SM count) and    */ \
+  /* xsy is given and overlaps no input; the calls above otherwise.  s is bit for bit               */ \
+  /* spx_prox_indballl0(nprob, n, s, xk, sj, q = (-nu) .* grad rounded to R, r, binf, delta).       */ \
+  /* out3_host = {ψ(s) as the type's ψ(y) returns it (spx_value_sep / spx_value_binf over the whole */ \
+  /* batch: the count of xk + sj + s != 0 against r; BInf: Inf when sj + s leaves the ball of       */ \
+  /* 1.1 delta, shiftedIndBallL0BInf.jl:44-49), Σ s², Σ grad·s} (Float64 sums).  sj must be given   */ \
+  /* (zeros when ψ is shifted once); s must not alias grad (SPX_E_INVALID).  The call synchronises; */ \
+  /* the scalars are all-reduced when the context reduces scalars.                                  */ \
+  int32_t spx_step_indballl0_##SUF(spx_ctx* ctx, int64_t nprob, int64_t n, R* s, R* xsy,             \
+                                   const R* xk, const R* sj, const R* grad, int64_t r, int32_t binf, \
+                                   double delta, double nu, double* out3_host);                      \
   int32_t spx_step_post_##SUF(spx_ctx* ctx, int64_t n, R* xsy, const R* xk, const R* sj, const R* s, \
                               const R* grad, double* out2_host);                                     \
   /* ------------------------------ host-buffer entry points (end-to-end path) */              \

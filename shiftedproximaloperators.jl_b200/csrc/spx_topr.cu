@@ -24,6 +24,7 @@
 #include <vector>
 
 #include "spx_common.cuh"
+#include "spx_setup.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -679,12 +680,65 @@ template <int THREADS> struct TsShared {
   unsigned long long cand_key[kTsCand];
 };
 
+// The operands the STEP form (spx_step_indballl0) adds: y is s, q is ∇f, and q = mnu ∇f is formed in R on every load.
+// a or c, chosen at compile time
+template <bool B, class A, class C> __device__ __forceinline__ auto& pick(A& a, C& c) {
+  if constexpr (B) return a;
+  else return c;
+}
+template <class R> struct TsStep {
+  R* xsy;             // (xk + sj) + s, every element
+  R mnu;              // -ν
+  double rad;         // BINF: 1.1 Δ in Float64, the ball of ψ(s) (shiftedIndBallL0BInf.jl:44-49)
+  Partial* partials;  // slot 0 at [blockIdx.x], slot 1 at [stride + blockIdx.x]
+  int stride;
+};
+
+// ψ(s), Σ s² and Σ ∇f·s of one entry, added with sign `sg` (+1 for the form written, -1 for the form it replaces).
+// The ψ predicates are those of ψ(y): ValueSep (xsy != 0) for the plain type, ValueBinfCount ((sj + s) + xk != 0 and
+// |sj + s| > 1.1Δ) for BInf.  The two counts are integers; the violation count leaves in a double slot, exactly.
+// One thread's counts of one problem stay within ±2047 (at most 512 entries per thread per pass, plus its candidates),
+// so both share one register: cnt = nnz + 4096 viol (the Float64 BInf instances spill with two).
+template <class R, bool BINF> struct TsStepAcc {
+  double s2 = 0.0, dot = 0.0;
+  int cnt = 0;
+  __device__ __forceinline__ void add(int sg, R xk, R sj, R xsy, R s, R g, double rad) {
+    const double ds = sg > 0 ? (double)s : -(double)s;
+    s2 = __fma_rn(ds, (double)s, s2);
+    dot = __fma_rn((double)g, ds, dot);
+    if (BINF) {
+      const R w = sj + s;
+      cnt += (fabs((double)w) > rad) ? 4096 * sg : 0;  // w < -rad || w > rad, NaN neither
+      cnt += ((w + xk) != R(0)) ? sg : 0;
+    } else {
+      cnt += (xsy != R(0)) ? sg : 0;
+    }
+  }
+  __device__ __forceinline__ int viol() const { return BINF ? (cnt + 2048) >> 12 : 0; }
+  __device__ __forceinline__ int nnz() const { return cnt - 4096 * viol(); }
+};
+
 // THREADS x MINB resident threads per SM.  SMEMKEYS: the 16-bit keys of the problem live in (dynamic) shared memory
 // -- 2 n bytes, one 1024-thread CTA per SM for n = 65536 -- instead of the L2-resident global scratch (larger n).
-template <class R, bool BINF, int THREADS, int MINB, bool SMEMKEYS>
-__global__ void __launch_bounds__(THREADS, MINB)
+// STEP (spx_step_indballl0): y = s and q = ∇f; q = (-ν)∇f is formed in R wherever q was loaded, so keys, selection and
+// s are those of prox!(s, ψ, fl(-ν∇f), ν).  Every write of s also writes xsy = (xk + sj) + s.  Pass 1 sums ψ(s),
+// Σ s², Σ ∇f·s for the form it wrote; every rewrite of pass 2b adds (new - old).  The candidates of the threshold value
+// are rewritten in rank order on a static rank-to-thread map (not in the atomicAdd order of the list), so the sums are
+// the same on every call.  A problem's sums go into the CTA's partial slots (slot 0 {ψ count, Σs², flag}, slot 1
+// {Σ∇f·s, violations}) after a block fold, unless the problem is hard: then the CTA writes q into its s for the radix
+// kernel (run with y = q = s) and topr_step_fixup_kernel writes its xsy and sums.
+// Resident CTAs per SM of an instance.  At 64 registers three Float64 STEP forms spill (4 to 36 bytes): the L2-key form
+// (n > 102400: global key pointer and cache policies next to the step's sums) and the 256-thread BInf form (the ball
+// test next to the clamp).  Those alone run one CTA per SM lower; every other instance keeps its prox! twin's.
+template <class R, bool BINF, int THREADS, int MINB, bool SMEMKEYS, bool STEP>
+constexpr int ts_min_blocks() {
+  return (STEP && sizeof(R) == 8 && (!SMEMKEYS || (BINF && THREADS == 256))) ? MINB - 1 : MINB;
+}
+template <class R, bool BINF, int THREADS, int MINB, bool SMEMKEYS, bool STEP = false>
+__global__ void __launch_bounds__(THREADS, (ts_min_blocks<R, BINF, THREADS, MINB, SMEMKEYS, STEP>()))
     topr_stream_kernel(R* y, const R* xk, const R* sj, const R* q, long long n, long long r, R delta, long long nprob,
-                       unsigned short* __restrict__ key_scratch, unsigned char* __restrict__ fallback) {
+                       unsigned short* __restrict__ key_scratch, unsigned char* __restrict__ fallback,
+                       TsStep<R> step = TsStep<R>{}) {
   using KT = KeyTraits<R>;
   constexpr int VEC = 16 / (int)sizeof(R);
   constexpr int kTsThreads = THREADS;
@@ -706,22 +760,58 @@ __global__ void __launch_bounds__(THREADS, MINB)
     if (BINF) v = jl_min(jl_max(v, -delta), delta);
     return v;
   };
-  auto fix = [&](int i, const R* pxk, const R* psj, const R* pq, R* py) {  // rewrite entry i in its kept form
+  auto qof = [&](R qg) -> R {  // STEP: the q plane holds ∇f
+    if constexpr (STEP) return step.mnu * qg;
+    else return qg;
+  };
+  auto fix_y = [&](int i, const R* pxk, const R* psj, const R* pq, R* py) {  // rewrite entry i in its kept form
     const R xs = pxk[i] + psj[i];
     py[i] = keep(xs, xs + pq[i]);
   };
-  auto unfix = [&](int i, const R* pxk, const R* psj, R* py) { py[i] = drop(pxk[i] + psj[i]); };
+  auto unfix_y = [&](int i, const R* pxk, const R* psj, R* py) { py[i] = drop(pxk[i] + psj[i]); };
+  // STEP: rewrite entry i of s and xsy in the form `kept`, and add (new - old) to the sums.  The key scan below calls
+  // fix / unfix with its original text; in the STEP form they name the wrappers around refix.  Generic lambdas and a
+  // compile-time pick rather than `if constexpr` at the call: any branch there changes how the prox! instances compile.
+  const R* step_grad = nullptr;  // this problem's ∇f (unfix takes no q operand)
+  TsStepAcc<R, BINF> acc;
+  auto refix = [&](auto i, bool kept, const R* pxk, const R* psj, const R* pg, R* py, R* pxsy) {
+    const R a = pxk[i], b = psj[i], g = pg[i];
+    const R xs = a + b;
+    const R sk = keep(xs, xs + step.mnu * g), sd = drop(xs);
+    const R sn = kept ? sk : sd, so = kept ? sd : sk;
+    const R vn = xs + sn;
+    py[i] = sn;
+    pxsy[i] = vn;
+    acc.add(1, a, b, vn, sn, g, step.rad);
+    acc.add(-1, a, b, xs + so, so, g, step.rad);
+  };
+  R* pxsy = nullptr;  // STEP: this problem's xsy
+  auto fix_step = [&](auto i, const R* pxk, const R* psj, const R* pg, R* py) { refix(i, true, pxk, psj, pg, py, pxsy); };
+  auto unfix_step = [&](auto i, const R* pxk, const R* psj, R* py) { refix(i, false, pxk, psj, step_grad, py, pxsy); };
+  auto& fix = pick<STEP>(fix_step, fix_y);
+  auto& unfix = pick<STEP>(unfix_step, unfix_y);
   // Pass 1 already writes the KEPT form where the 16-bit key reaches `guess` -- the threshold key of the previous
   // problem of this CTA, which for a batch of like problems is the threshold of this one or its neighbour -- so pass
   // 2b only has to rewrite the entries the guess got wrong plus the unkept ones among the threshold-valued entries,
   // instead of re-reading three operands for every kept entry.  A guess that proves bad (more than r rewrites) is
   // dropped for the next problem.
   unsigned guess = 0x10000u;  // nothing pre-kept
+  if constexpr (STEP) {
+    if (t == 0) {
+      step.partials[blockIdx.x] = Partial{0.0, 0.0, -1};
+      step.partials[step.stride + blockIdx.x] = Partial{0.0, 0.0, -1};
+    }
+  }
   for (long long prob = blockIdx.x; prob < nprob; prob += gridDim.x) {
     const R* pxk = xk + prob * n;
     const R* psj = sj + prob * n;
     const R* pq = q + prob * n;
     R* py = y + prob * n;
+    if constexpr (STEP) {
+      step_grad = pq;
+      pxsy = step.xsy + prob * n;
+      acc = TsStepAcc<R, BINF>{};
+    }
     // ---- pass 1 -----------------------------------------------------------------------------------------
     unsigned kmax = 0;
     for (int v0 = t; v0 < nvec; v0 += kTsUnroll * kTsThreads) {
@@ -744,12 +834,21 @@ __global__ void __launch_bounds__(THREADS, MINB)
 #pragma unroll
           for (int e = 0; e < VEC; ++e) {
             const R xs = a[u].v[e] + b[u].v[e];
-            const R z = xs + c[u].v[e];  // (xk + sj) + q   shiftedIndBallL0.jl:66
+            const R z = xs + qof(c[u].v[e]);  // (xk + sj) + q   shiftedIndBallL0.jl:66
             k16[e] = key16_of(z);
             o.v[e] = (k16[e] >= guess) ? keep(xs, z) : drop(xs);
             kmax = k16[e] > kmax ? k16[e] : kmax;
           }
           st_stream(py + v * VEC, o);
+          if constexpr (STEP) {
+            Pack<R, VEC> w;
+#pragma unroll
+            for (int e = 0; e < VEC; ++e) {
+              w.v[e] = (a[u].v[e] + b[u].v[e]) + o.v[e];
+              acc.add(1, a[u].v[e], b[u].v[e], w.v[e], o.v[e], c[u].v[e], step.rad);
+            }
+            st_stream(pxsy + v * VEC, w);
+          }
           if (VEC == 2) {
             const unsigned w = k16[0] | (k16[1] << 16);
             if (SMEMKEYS) reinterpret_cast<unsigned*>(keys)[v] = w;
@@ -863,7 +962,7 @@ __global__ void __launch_bounds__(THREADS, MINB)
       const int C = sh.cand_count < kTsCand ? sh.cand_count : kTsCand;  // == sel_count <= kTsCand
       for (int ci = t; ci < C; ci += kTsThreads) {
         const int i = sh.cand_idx[ci];
-        const R z = (pxk[i] + psj[i]) + pq[i];
+        const R z = (pxk[i] + psj[i]) + qof(pq[i]);
         sh.cand_key[ci] = (unsigned long long)KT::key(z);
       }
       __syncthreads();
@@ -876,17 +975,96 @@ __global__ void __launch_bounds__(THREADS, MINB)
           const unsigned long long kj = sh.cand_key[j];
           rank += (kj > mk) || (kj == mk && sh.cand_idx[j] < mi);
         }
-        const bool kept = (long long)rank <= need;
-        if (kept != (t16 >= guess)) {
-          if (kept) fix(mi, pxk, psj, pq, py);
-          else unfix(mi, pxk, psj, py);
+        if constexpr (STEP) {
+          reinterpret_cast<int*>(sh.hist)[rank - 1] = mi;  // ranks are 1..C, each once; hist is free after the pick
+        } else {
+          const bool kept = (long long)rank <= need;
+          if (kept != (t16 >= guess)) {
+            if (kept) fix(mi, pxk, psj, pq, py);
+            else unfix(mi, pxk, psj, py);
+          }
+        }
+      }
+      if constexpr (STEP) {
+        __syncthreads();
+        for (int rk = t; rk < C; rk += kTsThreads) {  // the candidate of rank rk + 1, on a static map
+          const bool kept = (long long)rk < need;
+          if (kept != (t16 >= guess)) refix(reinterpret_cast<const int*>(sh.hist)[rk], kept, pxk, psj, pq, py, pxsy);
         }
       }
       if (nrewrite) atomicAdd(&sh.rewrites, nrewrite);
     }
+    if constexpr (STEP) {
+      if (hard) {  // q into s for the radix kernel, which runs on the flagged problems with y = q = s
+        for (int v = t; v < nvec; v += kTsThreads) {
+          Pack<R, VEC> g;
+          ld_stream(pq + v * VEC, g);
+#pragma unroll
+          for (int e = 0; e < VEC; ++e) g.v[e] = step.mnu * g.v[e];
+          st_stream(py + v * VEC, g);
+        }
+      } else {  // block-uniform
+        Partial p0, p1;
+        p0.s = (double)acc.nnz();
+        p0.s2 = acc.s2;
+        p0.bad = -1;
+        p1.s = acc.dot;
+        p1.s2 = (double)acc.viol();
+        p1.bad = -1;
+        p0 = block_fold<kTsThreads>(p0);
+        p1 = block_fold<kTsThreads>(p1);
+        if (t == 0) {  // the CTA owns its slots: plain read-modify-write, problems in a fixed order
+          Partial* s0 = step.partials + blockIdx.x;
+          Partial* s1 = step.partials + step.stride + blockIdx.x;
+          s0->s += p0.s;
+          s0->s2 += p0.s2;
+          s1->s += p1.s;
+          s1->s2 += p1.s2;
+          s0->bad = s1->s2 > 0.0 ? 1 : -1;  // BINF: an entry of sj + s outside the ball (the exact count)
+        }
+      }
+    }
     __syncthreads();  // shared state (and the key scratch) is reused by the next problem
     guess = (!hard && (long long)sh.rewrites <= r) ? t16 : 0x10000u;
     __syncthreads();
+  }
+}
+
+// The step's problems that the stream kernel flagged and the radix kernel then solved in place: xsy = (xk + sj) + s and
+// the sums of the STEP form, into partial slots of their own.  A fixed grid walks the problems on a static map and
+// skips the unflagged ones, so the sums come out the same on every call; with no flagged problem it only reads flags.
+constexpr int kFixThreads = 256;
+template <class R, bool BINF>
+__global__ void __launch_bounds__(kFixThreads)
+    topr_step_fixup_kernel(const R* s, R* xsy, const R* xk, const R* sj, const R* grad, long long n, long long nprob,
+                           double rad, const unsigned char* __restrict__ flagged, Partial* partials, int stride) {
+  TsStepAcc<R, BINF> acc;  // its packed count is emptied after every problem (at most n / 256 <= 512 entries)
+  double nnz = 0.0, viol = 0.0;
+  for (long long prob = blockIdx.x; prob < nprob; prob += gridDim.x) {
+    if (flagged[prob] == 0) continue;  // block-uniform
+    const long long b = prob * n;
+    for (long long i = b + threadIdx.x; i < b + n; i += kFixThreads) {
+      const R a = xk[i], c = sj[i], v = s[i];
+      const R w = (a + c) + v;
+      xsy[i] = w;
+      acc.add(1, a, c, w, v, grad[i], rad);
+    }
+    nnz += (double)acc.nnz();
+    viol += (double)acc.viol();
+    acc.cnt = 0;
+  }
+  Partial p0, p1;
+  p0.s = nnz;
+  p0.s2 = acc.s2;
+  p0.bad = viol > 0.0 ? 1 : -1;
+  p1.s = acc.dot;
+  p1.s2 = viol;
+  p1.bad = -1;
+  p0 = block_fold<kFixThreads>(p0);
+  p1 = block_fold<kFixThreads>(p1);
+  if (threadIdx.x == 0) {
+    partials[blockIdx.x] = p0;
+    partials[stride + blockIdx.x] = p1;
   }
 }
 
@@ -1240,9 +1418,11 @@ static int32_t topr_cluster_launch(spx_ctx* ctx, int64_t nprob, int64_t n, R* y,
   return SPX_OK;
 }
 
-template <class R, bool BINF>
+// STEP (spx_step_indballl0): y = s, q = ∇f, and `step` carries xsy, -ν, the ball and the partial slots; the radix kernel
+// then runs with q = s, and *step_grid returns the stream grid (the fixup kernel's slots follow it).
+template <class R, bool BINF, bool STEP = false>
 static int32_t topr_stream_launch(spx_ctx* ctx, int64_t nprob, int64_t n, R* y, const R* xk, const R* sj, const R* q,
-                                  int64_t r, R delta) {
+                                  int64_t r, R delta, TsStep<R> step = TsStep<R>{}, int* step_grid = nullptr) {
   const size_t flags_bytes = ((size_t)nprob + 255) & ~(size_t)255;
   const size_t key_bytes = (size_t)n * sizeof(unsigned short);
   // keys in shared memory while 2 n bytes fit next to the static state of a CTA: one 1024-thread CTA per SM above
@@ -1259,16 +1439,20 @@ static int32_t topr_stream_launch(spx_ctx* ctx, int64_t nprob, int64_t n, R* y, 
     if (s2 != SPX_OK) return s2;
     flags = (unsigned char*)ctx->d_scratch + 4096;  // the first 4 KiB belong to the reductions
     unsigned short* keys = (unsigned short*)((char*)ctx->d_scratch + 4096 + flags_bytes);
+    if constexpr (STEP) {
+      step.stride = (int)grid + ctx->sm_count;  // the fixup kernel's sm_count CTAs follow the stream grid
+      *step_grid = (int)grid;
+    }
     kern<<<(unsigned)grid, threads, dyn, ctx->stream>>>(y, xk, sj, q, (long long)n, (long long)r, delta, (long long)nprob,
-                                                        keys, flags);
+                                                        keys, flags, step);
     ctx->launches++;
     SPX_CUDA(cudaGetLastError());
     return SPX_OK;
   };
-  if (!smem_keys) st = go(topr_stream_kernel<R, BINF, 512, 2, false>, 512, 0, true);
-  else if (key_bytes > 72 * 1024) st = go(topr_stream_kernel<R, BINF, 1024, 1, true>, 1024, key_bytes, false);
-  else if (key_bytes > 36 * 1024) st = go(topr_stream_kernel<R, BINF, 512, 2, true>, 512, key_bytes, false);
-  else st = go(topr_stream_kernel<R, BINF, 256, 4, true>, 256, key_bytes, false);
+  if (!smem_keys) st = go(topr_stream_kernel<R, BINF, 512, 2, false, STEP>, 512, 0, true);
+  else if (key_bytes > 72 * 1024) st = go(topr_stream_kernel<R, BINF, 1024, 1, true, STEP>, 1024, key_bytes, false);
+  else if (key_bytes > 36 * 1024) st = go(topr_stream_kernel<R, BINF, 512, 2, true, STEP>, 512, key_bytes, false);
+  else st = go(topr_stream_kernel<R, BINF, 256, 4, true, STEP>, 256, key_bytes, false);
   if (st != SPX_OK) return st;
   // radix select on the problems it flagged (NaN / Inf / all-zero / crowded threshold value)
   int csize = 1;
@@ -1279,10 +1463,30 @@ static int32_t topr_stream_launch(spx_ctx* ctx, int64_t nprob, int64_t n, R* y, 
   auto rk = topr_cluster_kernel<R, BINF, true>;
   st = cluster_grid(ctx, rk, csize, smem, nprob, &cfg, attr);
   if (st != SPX_OK) return st;
-  SPX_CUDA(cudaLaunchKernelEx(&cfg, rk, y, xk, sj, q, (long long)n, (long long)r, delta, (long long)nprob,
-                              (const unsigned char*)flags));
+  SPX_CUDA(cudaLaunchKernelEx(&cfg, rk, y, xk, sj, STEP ? (const R*)y : q, (long long)n, (long long)r, delta,
+                              (long long)nprob, (const unsigned char*)flags));
   ctx->launches++;
+  if constexpr (STEP) {
+    topr_step_fixup_kernel<R, BINF><<<ctx->sm_count, kFixThreads, 0, ctx->stream>>>(
+        y, step.xsy, xk, sj, q, (long long)n, (long long)nprob, step.rad, flags, step.partials + *step_grid,
+        step.stride);
+    ctx->launches++;
+    SPX_CUDA(cudaGetLastError());
+  }
   return SPX_OK;
+}
+
+// The host conditions of the stream form (batches of problems: one CTA per problem), shared by prox! and the step:
+// 16-byte aligned vectors, n a multiple of 8 in [4096, the cluster capacity], 0 < r < n, at least two problems per SM,
+// and no output overlapping an input (pass 1 writes y before pass 2b re-reads the inputs at the kept positions).
+template <class R>
+static bool topr_stream_ok(const spx_ctx* ctx, int64_t nprob, int64_t n, int64_t r, bool aligned, bool overlap) {
+  return aligned && !overlap && n % 8 == 0 && n >= 4096 && n <= (int64_t)kTrMaxCluster * kTrChunk && r > 0 && r < n &&
+         nprob >= 2 * (int64_t)ctx->sm_count;
+}
+// does [p, p + bytes) overlap [o, o + bytes)
+static bool spans_overlap(const void* p, const void* o, size_t bytes) {
+  return p != nullptr && o != nullptr && (const char*)p < (const char*)o + bytes && (const char*)o < (const char*)p + bytes;
 }
 
 template <class R>
@@ -1304,10 +1508,9 @@ static int32_t prox_indballl0(spx_ctx* ctx, int64_t nprob, int64_t n, R* y, cons
   const bool vec = (bits & 15u) == 0 && (n * (int64_t)sizeof(R)) % 16 == 0;
   // batches: the stream form (one CTA per problem, several CTAs per SM)
   {
-    const char *y0 = (const char*)y, *y1 = y0 + (size_t)nprob * n * sizeof(R);
-    auto overlaps = [&](const R* p) { return (const char*)p < y1 && (const char*)p + (size_t)nprob * n * sizeof(R) > y0; };
-    const bool alias = overlaps(xk) || overlaps(sj) || overlaps(q);
-    if (vec && !alias && n % 8 == 0 && n >= 4096 && r > 0 && r < n && nprob >= 2 * (int64_t)ctx->sm_count) {
+    const size_t bytes = (size_t)nprob * n * sizeof(R);
+    const bool alias = spans_overlap(y, xk, bytes) || spans_overlap(y, sj, bytes) || spans_overlap(y, q, bytes);
+    if (topr_stream_ok<R>(ctx, nprob, n, r, vec, alias)) {
       return binf ? topr_stream_launch<R, true>(ctx, nprob, n, y, xk, sj, q, r, (R)delta)
                   : topr_stream_launch<R, false>(ctx, nprob, n, y, xk, sj, q, r, (R)delta);
     }
@@ -1318,6 +1521,69 @@ static int32_t prox_indballl0(spx_ctx* ctx, int64_t nprob, int64_t n, R* y, cons
   }
   return vec ? topr_cluster_launch<R, false, true>(ctx, nprob, n, y, xk, sj, q, r, (R)delta)
              : topr_cluster_launch<R, false, false>(ctx, nprob, n, y, xk, sj, q, r, (R)delta);
+}
+
+// ψ(y) of the two types over the whole batch, as their ψ(y) entries compute it (the composed step's value)
+static int32_t value_indballl0(spx_ctx* ctx, int64_t N, const double* xk, const double* sj, const double* y,
+                               int32_t binf, double delta, int64_t r, double* out) {
+  return binf ? spx_value_binf_f64(ctx, SPX_H_INDBALLL0, N, xk, sj, y, delta, r, 0, nullptr, nullptr, out)
+              : spx_value_sep_f64(ctx, SPX_H_INDBALLL0, N, xk, sj, y, 0.0, r, out);
+}
+static int32_t value_indballl0(spx_ctx* ctx, int64_t N, const float* xk, const float* sj, const float* y, int32_t binf,
+                               double delta, int64_t r, double* out) {
+  return binf ? spx_value_binf_f32(ctx, SPX_H_INDBALLL0, N, xk, sj, y, delta, r, 0, nullptr, nullptr, out)
+              : spx_value_sep_f32(ctx, SPX_H_INDBALLL0, N, xk, sj, y, 0.0, r, out);
+}
+
+// ---- the solver step of ShiftedIndBallL0 / ShiftedIndBallL0BInf (SURVEY.md 8f rank 1) -------------------------------
+//     q = (-ν) ∇f;  prox!(s, ψ, q, ν);  xsy = (xk + sj) + s;  ψ(s);  Σ s²;  Σ ∇f·s
+// A batch the stream form takes (topr_stream_ok, with xsy given and no output overlapping an input) runs it in ONE pass
+// of the STEP form of topr_stream_kernel, then the radix kernel on the problems it flagged (in place: y = q = s) and
+// topr_step_fixup_kernel for their xsy and sums: a fixed launch sequence, no host synchronisation until the fold.
+// Every other call takes the composed form: spx_step_pre, prox! in place, the type's ψ(y), spx_step_post.
+template <class R>
+static int32_t step_indballl0(spx_ctx* ctx, int64_t nprob, int64_t n, R* s, R* xsy, const R* xk, const R* sj,
+                              const R* grad, int64_t r, int32_t binf, double delta, double nu, double* out3) {
+  SPX_REQUIRE(ctx != nullptr, "null context");
+  SPX_REQUIRE(nprob >= 0 && n >= 0, "negative size");
+  SPX_REQUIRE(out3 != nullptr, "null result array");
+  const int64_t N = nprob * n;
+  SPX_REQUIRE(N == 0 || (s && xk && sj && grad), "null device vector");
+  const size_t bytes = (size_t)N * sizeof(R);
+  SPX_REQUIRE(!spans_overlap(s, grad, bytes), "s must not alias grad");
+  DeviceGuard g(ctx->device);
+  out3[0] = out3[1] = out3[2] = 0.0;
+  if (N == 0) return SPX_OK;
+  const bool aligned = (((uintptr_t)s | (uintptr_t)xsy | (uintptr_t)xk | (uintptr_t)sj | (uintptr_t)grad) & 15u) == 0;
+  const bool overlap = spans_overlap(s, xk, bytes) || spans_overlap(s, sj, bytes) || spans_overlap(xsy, xk, bytes) ||
+                       spans_overlap(xsy, sj, bytes) || spans_overlap(xsy, grad, bytes) || spans_overlap(xsy, s, bytes);
+  if (xsy != nullptr && topr_stream_ok<R>(ctx, nprob, n, r, aligned, overlap)) {
+    TsStep<R> step{xsy, -(R)nu, 1.1 * (double)(R)delta, ctx->d_partials, 0};
+    int grid = 0;
+    const int32_t st = binf ? topr_stream_launch<R, true, true>(ctx, nprob, n, s, xk, sj, grad, r, (R)delta, step, &grid)
+                            : topr_stream_launch<R, false, true>(ctx, nprob, n, s, xk, sj, grad, r, (R)delta, step, &grid);
+    if (st != SPX_OK) return st;
+    const int32_t st2 = finalize_partials(ctx, grid + ctx->sm_count, 2, false);
+    if (st2 != SPX_OK) return st2;
+    // the same predicates and scaling as ψ(y): ValueSep / scale_value, ValueBinfCount and its flag
+    const double count = ctx->h_result[0].s;
+    out3[0] = (binf && ctx->h_result[0].bad > 0) ? kInf : scale_value<R>(SPX_H_INDBALLL0, R(0), count, r);
+    out3[1] = ctx->h_result[0].s2;
+    out3[2] = ctx->h_result[1].s;
+    return SPX_OK;
+  }
+  int32_t st = step_pre<R>(ctx, N, s, grad, nu);
+  if (st != SPX_OK) return st;
+  st = prox_indballl0<R>(ctx, nprob, n, s, xk, sj, s, r, binf, delta);
+  if (st != SPX_OK) return st;
+  st = value_indballl0(ctx, N, xk, sj, s, binf, delta, r, &out3[0]);
+  if (st != SPX_OK) return st;
+  double out2[2] = {0.0, 0.0};
+  st = step_post<R>(ctx, N, xsy, xk, sj, s, grad, out2);
+  if (st != SPX_OK) return st;
+  out3[1] = out2[0];
+  out3[2] = out2[1];
+  return SPX_OK;
 }
 
 }  // namespace spx
@@ -1390,4 +1656,14 @@ extern "C" int32_t spx_prox_indballl0_sharded_f32(spx_ctx* ctx, int64_t n_local,
 extern "C" int32_t spx_prox_indballl0_f32(spx_ctx* ctx, int64_t nprob, int64_t n, float* y, const float* xk,
                                           const float* sj, const float* q, int64_t r, int32_t binf, double delta) {
   return prox_indballl0<float>(ctx, nprob, n, y, xk, sj, q, r, binf, delta);
+}
+extern "C" int32_t spx_step_indballl0_f64(spx_ctx* ctx, int64_t nprob, int64_t n, double* s, double* xsy,
+                                          const double* xk, const double* sj, const double* grad, int64_t r,
+                                          int32_t binf, double delta, double nu, double* out3) {
+  return step_indballl0<double>(ctx, nprob, n, s, xsy, xk, sj, grad, r, binf, delta, nu, out3);
+}
+extern "C" int32_t spx_step_indballl0_f32(spx_ctx* ctx, int64_t nprob, int64_t n, float* s, float* xsy,
+                                          const float* xk, const float* sj, const float* grad, int64_t r,
+                                          int32_t binf, double delta, double nu, double* out3) {
+  return step_indballl0<float>(ctx, nprob, n, s, xsy, xk, sj, grad, r, binf, delta, nu, out3);
 }

@@ -568,6 +568,20 @@ class ShiftedNormL1B2(ShiftedProximableFunction):
         return out.value
 
 
+def _step_indballl0(psi, s, grad, nu, xsy, binf, delta):
+    # spx_step_indballl0_*: the whole step in one pass of the stream top-r kernel on a batch it takes, the composed form
+    # (step_pre, prox! in place, ψ(s), step_post) otherwise -- decided in the library
+    psi._check(s, grad, ("s", "grad"))
+    if xsy is not None:
+        _vec(xsy, psi.xk, "xsy")
+    if s.numel() > 0 and s.data_ptr() == grad.data_ptr():
+        raise ValueError("step_: s must not alias grad")
+    out = (C.c_double * 3)()
+    psi._call("step_indballl0", C.c_int64(psi.nprob), C.c_int64(psi.n // psi.nprob), _p(s), _p(xsy), _p(psi.xk),
+              _p(psi.sj), _p(grad), C.c_int64(psi.h.r), C.c_int32(binf), C.c_double(delta), C.c_double(nu), out)
+    return s, StepResult(out[0], math.sqrt(out[1]), out[2])
+
+
 class ShiftedIndBallL0(ShiftedProximableFunction):
     """ShiftedIndBallL0  (src/shiftedIndBallL0.jl:3-49); the `p` permutation scratch does not exist here."""
     _H_KIND = L.H_INDBALLL0
@@ -583,6 +597,11 @@ class ShiftedIndBallL0(ShiftedProximableFunction):
         self._call("prox_indballl0", C.c_int64(self.nprob), C.c_int64(self.n // self.nprob), _p(y), _p(self.xk),
                    _p(self.sj), _p(q), C.c_int64(self.h.r), C.c_int32(0), C.c_double(0.0))
         return (y, self(y)) if want_value else y
+
+    def step_(self, s, grad, nu, xsy=None):
+        """spx_step_indballl0_*: the whole step in one pass of the stream top-r kernel for a batch of >= 2 problems per
+        SM (the C5 shape), the two passes around prox! otherwise."""
+        return _step_indballl0(self, s, grad, nu, xsy, 0, 0.0)
 
 
 class ShiftedIndBallL0BInf(ShiftedProximableFunction):
@@ -601,6 +620,10 @@ class ShiftedIndBallL0BInf(ShiftedProximableFunction):
         self._call("prox_indballl0", C.c_int64(self.nprob), C.c_int64(self.n // self.nprob), _p(y), _p(self.xk),
                    _p(self.sj), _p(q), C.c_int64(self.h.r), C.c_int32(1), C.c_double(self.Delta))
         return (y, self(y)) if want_value else y
+
+    def step_(self, s, grad, nu, xsy=None):
+        """spx_step_indballl0_*: as ShiftedIndBallL0.step_, with ψ(s) = Inf when sj + s leaves the ball of 1.1Δ."""
+        return _step_indballl0(self, s, grad, nu, xsy, 1, self.Delta)
 
     def __call__(self, y):  # shiftedIndBallL0BInf.jl:44-49
         _vec(y, self.xk, "y")

@@ -241,6 +241,46 @@ def main():
                    note=f"{nprob} problems x {pn}, r=1024")
         psi1 = sp.shifted(sp.shifted(sp.IndBallL0(1 << 20), xk), sj)
         timeit("prox_indballl0_single", lambda: sp.prox_(y, psi1, q, 1.0), 4 * R, note="one vector, r=2^20, global path")
+    # the top-r step at the C5 shape (problems of 65536, r = 1024; q plays ∇f): the one-pass step
+    # (spx_step_indballl0), the base-class composition (spx_step_pre, prox! in place, ψ(s), spx_step_post) and the
+    # caller's separate sweeps (q = -ν∇f into its own buffer, the stream prox!, ψ(s), xsy and the two sums as torch ops),
+    # alternated three times: the comparison is what these rows are for
+    if any(re.search(args.only, nm) for nm in ("step_indballl0_batch", "step_indballl0binf_batch")):
+        pn, nu = 65536, 0.3
+        nprob = n // pn
+        xsy_b = torch.empty_like(y)
+
+        def sweeps(psi, s, xsy, qbuf):
+            torch.mul(q, -nu, out=qbuf)
+            sp.prox_(s, psi, qbuf, nu)
+            val = psi(s)
+            torch.add(xk, sj, out=xsy).add_(s)
+            return val, torch.dot(s, s).item(), torch.dot(q, s).item()
+
+        for binf in (False, True):
+            h = sp.IndBallL0(1024)
+            psi = (sp.shifted(h, xk, 1.0, sp.NormLinf(1.0), nprob=nprob) if binf else sp.shifted(h, xk, nprob=nprob))
+            psi = sp.shifted(psi, sj)
+            tag = f"step_indballl0{'binf' if binf else ''}_batch"
+            if not any(re.search(args.only, nm) for nm in (tag, tag + "_composed", tag + "_sweeps")):
+                continue
+            s2, xsy2, qbuf = torch.empty_like(y), torch.empty_like(y), torch.empty_like(y)
+            _, r1 = sp.step_(y, psi, q, nu, xsy=xsy_b)
+            _, r2 = sp.ShiftedProximableFunction.step_(psi, s2, q, nu, xsy=xsy2)
+            same = torch.equal(y, s2) and torch.equal(xsy_b, xsy2)
+            r3 = sweeps(psi, s2, xsy2, qbuf)
+            same = same and torch.equal(y, s2) and torch.equal(xsy_b, xsy2)
+            print(f"{tag} vs composed vs sweeps: s and xsy bit-identical: {same}; scalars {tuple(r1)} / {tuple(r2)} / "
+                  f"(psi {r3[0]}, snorm {r3[1] ** 0.5}, gdots {r3[2]})", flush=True)
+            note = f"{nprob} problems x {pn}, r=1024; alg. bytes = 3 reads + 2 writes"
+            for _ in range(3):
+                timeit(tag, lambda psi=psi: sp.step_(y, psi, q, nu, xsy=xsy_b), 5 * R, note="one pass; " + note)
+                timeit(tag + "_composed", lambda psi=psi: sp.ShiftedProximableFunction.step_(psi, y, q, nu, xsy=xsy_b),
+                       5 * R, note="step_pre, prox! in place, ψ(s), step_post; " + note)
+                timeit(tag + "_sweeps", lambda psi=psi: sweeps(psi, y, xsy_b, qbuf), 5 * R,
+                       note="q buffer, stream prox!, ψ(s), torch xsy / dots; " + note)
+            del s2, xsy2, qbuf
+        del xsy_b
     if args.json:
         os.makedirs(os.path.dirname(os.path.abspath(args.json)), exist_ok=True)
         json.dump(results, open(args.json, "w"), indent=1)
