@@ -376,7 +376,7 @@ typedef struct spx_box_job_f32 {
                               const R* sj, const R* grad, const R* D, double dshift,             \
                               const spx_bound* l, const spx_bound* u, const spx_sel* sel,        \
                               double lambda, double* out4_host);                                 \
-  /* The step around a prox! that is not one streaming pass (groups, top-r, ShiftedNormL1B2): the    */ \
+  /* The step around a prox! that is not one streaming pass (groups, top-r): the                      */ \
   /* caller's sweeps as two passes around the operator's own entry point --                          */ \
   /*   spx_step_pre:   q = (-nu) .* grad (rounded to R), written where s will be;                    */ \
   /*   the type's spx_prox_* IN PLACE (y = q = s, sigma = nu, its psi_out / value entry gives ψ(s)); */ \
@@ -416,6 +416,28 @@ typedef struct spx_box_job_f32 {
   int32_t spx_step_indballl0_##SUF(spx_ctx* ctx, int64_t nprob, int64_t n, R* s, R* xsy,             \
                                    const R* xk, const R* sj, const R* grad, int64_t r, int32_t binf, \
                                    double delta, double nu, double* out3_host);                      \
+  /* The whole step of ShiftedNormL1B2 (shiftedNormL1B2.jl:47-64) inside the passes of its own root */ \
+  /* search: every pass forms q = (-nu) .* grad (rounded to R) on the load, the finish writes s and   */ \
+  /* xsy = (xk + sj) + s (xsy may be NULL).  s is bit for bit spx_prox_l1b2(y = s, q = (-nu) .* grad */ \
+  /* rounded to R, sigma = nu) into an s that overlaps no input.  out3_host = {ψ(s) as psi_out of     */ \
+  /* spx_prox_l1b2 (λ Σ|xk + sj + s| rounded to R, Inf when ‖sj + s‖ leaves the ball of delta,       */ \
+  /* shiftedNormL1B2.jl:32), Σ s², Σ grad·s} (Float64 sums); passes_out (may be NULL) as for          */ \
+  /* spx_prox_l1b2.  s uses itself as scratch, and the finish doubles as the check of an unverified   */ \
+  /* root, only when s and xsy overlap none of xk, sj, grad; otherwise (xsy = xk: x <- x + s) the     */ \
+  /* search converges by evaluation and each element's operands are read before its results are      */ \
+  /* written.  sj must be given (zeros when ψ is shifted once); s overlapping grad or xsy:          */ \
+  /* SPX_E_INVALID.                                                                                  */ \
+  /* The call synchronises; every decision of the search and out3_host are all-reduced when the       */ \
+  /* context reduces scalars.                                                                         */ \
+  int32_t spx_step_l1b2_##SUF(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj,       \
+                              const R* grad, double lambda, double nu, double delta,                 \
+                              double chi_lambda, int32_t* passes_out, double* out3_host);            \
+  /* the same step on this rank's shard of a sharded vector: `reduce` gets the 2K partial sums of     */ \
+  /* every norm pass and, once, the finish's four {Σ|xk + sj + s|, Σ (sj + s)², Σ s², Σ grad·s}       */ \
+  int32_t spx_step_l1b2_sharded_##SUF(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk,            \
+                                      const R* sj, const R* grad, double lambda, double nu,          \
+                                      double delta, double chi_lambda, spx_allreduce_sum_fn reduce,  \
+                                      void* user, int32_t* passes_out, double* out3_host);           \
   int32_t spx_step_post_##SUF(spx_ctx* ctx, int64_t n, R* xsy, const R* xk, const R* sj, const R* s, \
                               const R* grad, double* out2_host);                                     \
   /* ------------------------------ host-buffer entry points (end-to-end path) */              \

@@ -328,6 +328,10 @@ int32_t finalize_partials(spx_ctx* ctx, int nblocks, int nslot, bool bad_is_min)
 template <class R> int32_t step_pre(spx_ctx* ctx, int64_t n, R* q, const R* grad, double nu);
 template <class R>
 int32_t step_post(spx_ctx* ctx, int64_t n, R* xsy, const R* xk, const R* sj, const R* s, const R* grad, double* out2);
+// the finish pass of the ShiftedNormL1B2 step (spx_step.cu, called by the root search of spx_l1b2.cu)
+template <class R>
+int32_t step_l1b2_finish(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad, const R* mid,
+                         R nu, R ls, bool use_scale, R scale, R post, double* v);
 // spx_comm.cu: is the context in "scalars are global" mode; all-reduce ctx->d_result[0..nslot) on ctx->stream
 bool comm_active(const spx_ctx* ctx);
 int32_t comm_neutral_result(spx_ctx* ctx, int nslot);

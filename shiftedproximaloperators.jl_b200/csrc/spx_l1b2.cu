@@ -44,10 +44,14 @@ template <class R, int K> struct L1b2Unroll {
 // MODE 0: mid = sj + q from the two vectors.  MODE 1: same, and mid is stored to `midbuf` (the first pass, when
 // the output vector aliases no input and can serve as scratch).  MODE 2: `sj` IS the stored mid, q is not read:
 // every later pass of the search moves 2R instead of 3R.
-template <class R, int K, int VEC, int MODE>
+// GRAD (the solver step, MODE 0 and 1): the q plane holds ∇f, and q = mnu ∇f (mnu = -ν) is rounded to R before the
+// sum, as the caller's broadcast rounds it (-fmad=false keeps the product out of an FMA): mid, and so every sum of
+// the pass, is bit for bit the prox!'s of that q.
+template <class R, int K, int VEC, int MODE, bool GRAD>
 __global__ void __launch_bounds__(kEwThreads, L1b2Unroll<R, K>::minb)
     l1b2_norm_kernel(const R* xk, const R* sj, const R* q, R* midbuf, long long n, R ls, bool use_scale,
-                     ScaleSet<K> sc, int nblocks_stride, Partial* __restrict__ partials) {
+                     ScaleSet<K> sc, int nblocks_stride, Partial* __restrict__ partials, R mnu) {
+  static_assert(!(GRAD && MODE == 2), "MODE 2 does not read q");
   double acc[K], dot[K];
 #pragma unroll
   for (int k = 0; k < K; ++k) { acc[k] = 0.0; dot[k] = 0.0; }
@@ -63,7 +67,7 @@ __global__ void __launch_bounds__(kEwThreads, L1b2Unroll<R, K>::minb)
 #pragma unroll
     for (int e = 0; e < VEC; ++e) {
       const bool on = e < m;
-      const R mid = on ? (MODE == 2 ? s[e] : s[e] + qq[e]) : R(0);
+      const R mid = on ? (MODE == 2 ? s[e] : s[e] + (GRAD ? mnu * qq[e] : qq[e])) : R(0);
       if (MODE == 1) mid_out[e] = mid;
       lo[e] = mid - ls;
       hi[e] = mid + ls;
@@ -148,7 +152,7 @@ __global__ void __launch_bounds__(kEwThreads, L1b2Unroll<R, K>::minb)
 
 template <class R, int K>
 static int32_t norm_pass_k(spx_ctx* ctx, int64_t n, const R* xk, const R* sj, const R* q, R ls, const double* scale,
-                           int nscale, double* out, double* dot_out, int mode, R* midbuf) {
+                           int nscale, double* out, double* dot_out, int mode, R* midbuf, bool grad, R mnu) {
   ScaleSet<K> sc;
   for (int k = 0; k < K; ++k) sc.s[k] = scale ? scale[k < nscale ? k : nscale - 1] : 1.0;
   const uintptr_t bits = (uintptr_t)xk | (uintptr_t)sj | (uintptr_t)q | (uintptr_t)midbuf;
@@ -159,18 +163,21 @@ static int32_t norm_pass_k(spx_ctx* ctx, int64_t n, const R* xk, const R* sj, co
   if (want < 1) want = 1;
   long long cap = (long long)ctx->sm_count * 8;
   const int grid = (int)(want < cap ? want : cap);
-#define SPX_L1B2_LAUNCH(V, M)                                                                                  \
-  l1b2_norm_kernel<R, K, V, M><<<grid, kEwThreads, 0, ctx->stream>>>(xk, sj, q, midbuf, n, ls, scale != nullptr, sc, \
-                                                                     grid, ctx->d_partials)
+#define SPX_L1B2_LAUNCH(V, M, G)                                                                                \
+  l1b2_norm_kernel<R, K, V, M, G><<<grid, kEwThreads, 0, ctx->stream>>>(xk, sj, q, midbuf, n, ls, scale != nullptr, \
+                                                                        sc, grid, ctx->d_partials, mnu)
+#define SPX_L1B2_MODES(V)                                                  \
+  if (mode == 2) SPX_L1B2_LAUNCH(V, 2, false);                             \
+  else if (mode == 1 && grad) SPX_L1B2_LAUNCH(V, 1, true);                 \
+  else if (mode == 1) SPX_L1B2_LAUNCH(V, 1, false);                        \
+  else if (grad) SPX_L1B2_LAUNCH(V, 0, true);                              \
+  else SPX_L1B2_LAUNCH(V, 0, false)
   if (vec) {
-    if (mode == 0) SPX_L1B2_LAUNCH(VECW, 0);
-    else if (mode == 1) SPX_L1B2_LAUNCH(VECW, 1);
-    else SPX_L1B2_LAUNCH(VECW, 2);
+    SPX_L1B2_MODES(VECW);
   } else {
-    if (mode == 0) SPX_L1B2_LAUNCH(1, 0);
-    else if (mode == 1) SPX_L1B2_LAUNCH(1, 1);
-    else SPX_L1B2_LAUNCH(1, 2);
+    SPX_L1B2_MODES(1);
   }
+#undef SPX_L1B2_MODES
 #undef SPX_L1B2_LAUNCH
   ctx->launches++;
   SPX_CUDA(cudaGetLastError());
@@ -184,47 +191,21 @@ static int32_t norm_pass_k(spx_ctx* ctx, int64_t n, const R* xk, const R* sj, co
 
 template <class R>
 static int32_t norm_pass(spx_ctx* ctx, int64_t n, const R* xk, const R* sj, const R* q, R ls, const double* scale,
-                         int nscale, double* out, double* dot_out = nullptr, int mode = 0, R* midbuf = nullptr) {
+                         int nscale, double* out, double* dot_out = nullptr, int mode = 0, R* midbuf = nullptr,
+                         bool grad = false, R mnu = R(0)) {
   if (n == 0) {
     for (int k = 0; k < nscale; ++k) out[k] = 0.0;
     if (dot_out)
       for (int k = 0; k < nscale; ++k) dot_out[k] = 0.0;
     return SPX_OK;
   }
-  if (nscale <= 1) return norm_pass_k<R, 1>(ctx, n, xk, sj, q, ls, scale, nscale, out, dot_out, mode, midbuf);
-  if (nscale <= 4) return norm_pass_k<R, 4>(ctx, n, xk, sj, q, ls, scale, nscale, out, dot_out, mode, midbuf);
-  if (nscale <= 8) return norm_pass_k<R, 8>(ctx, n, xk, sj, q, ls, scale, nscale, out, dot_out, mode, midbuf);
-  return norm_pass_k<R, 16>(ctx, n, xk, sj, q, ls, scale, nscale, out, dot_out, mode, midbuf);
+  if (nscale <= 1) return norm_pass_k<R, 1>(ctx, n, xk, sj, q, ls, scale, nscale, out, dot_out, mode, midbuf, grad, mnu);
+  if (nscale <= 4) return norm_pass_k<R, 4>(ctx, n, xk, sj, q, ls, scale, nscale, out, dot_out, mode, midbuf, grad, mnu);
+  if (nscale <= 8) return norm_pass_k<R, 8>(ctx, n, xk, sj, q, ls, scale, nscale, out, dot_out, mode, midbuf, grad, mnu);
+  return norm_pass_k<R, 16>(ctx, n, xk, sj, q, ls, scale, nscale, out, dot_out, mode, midbuf, grad, mnu);
 }
 
-// y = ProjB(-xk scale) post - sj, with Σ|xk+sj+y| and Σ(sj+y)² for ψ(y)
-template <class R, bool PSI> struct L1B2Finish {
-  using Real = R;
-  static constexpr int NIN = 3, UNROLL = 2;
-  static constexpr bool OUT = true, ACC = PSI;
-  const R* in[NIN];  // xk, sj, q
-  R fill[NIN];
-  R* y;
-  R ls, scale, post;
-  bool use_scale;
-  bool have_mid;  // in[2] is the stashed sj + q (the output vector itself) instead of q
-  __device__ __forceinline__ R apply(const R (&x)[NIN], long long, Partial& acc) const {
-    const R mid = have_mid ? x[2] : x[1] + x[2];
-    const R lo = mid - ls, hi = mid + ls;
-    const R nx = -x[0];
-    const R z = use_scale ? nx * scale : nx;
-    R w = jl_min(jl_max(z, lo), hi);
-    if (use_scale) w = w * post;
-    const R o = w - x[1];
-    if (PSI) {
-      acc.s += (double)jl_abs((x[0] + x[1]) + o);
-      const double t = (double)(x[1] + o);
-      acc.s2 += t * t;
-    }
-    return o;
-  }
-};
-
+// y = ProjB(-xk scale) post - sj (L1B2Finish, spx_ops.cuh), with Σ|xk+sj+y| and Σ(sj+y)² for ψ(y)
 template <class R>
 static int32_t finish_pass(spx_ctx* ctx, int64_t n, R* y, const R* xk, const R* sj, const R* q, R ls, bool use_scale,
                            R scale, R post, double* psi_sum, double* w_sumsq, bool have_mid = false) {
@@ -263,22 +244,42 @@ template <class R> static bool in_ball_l2(R nw, R delta) {
   return std::fabs(nw - delta) <= tol;
 }
 
+template <class R> static bool overlap(const R* a, const R* b, int64_t n) {
+  return a && b && (const char*)a < (const char*)(b + n) && (const char*)b < (const char*)(a + n);
+}
+
+// What the search reads and writes.  prox!: q is the q vector; the finish writes y and sums ψ's two sums.  The solver
+// step (spx_step_l1b2): the q plane holds ∇f and every pass forms q = fl(mnu ∇f), mnu = -ν, on the load, so every sum of
+// the search is the prox!'s of that q bit for bit; the finish also writes xsy (may be NULL) and sums Σs², Σ∇f·s.
+template <class R> struct L1B2Io {
+  R* y;
+  const R *xk, *sj, *q;
+  bool grad = false;
+  R mnu = R(0);
+  R* xsy = nullptr;
+  double* sums = nullptr;  // step: {Σs², Σ∇f·s}
+};
+
 template <class R>
-static int32_t prox_l1b2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const R* sj, const R* q, double lambda_,
-                         double sigma_, double delta_, double chi_lambda_, spx_allreduce_sum_fn reduce, void* user,
-                         int32_t* passes_out, double* psi_out) {
+static int32_t l1b2_search(spx_ctx* ctx, int64_t n, const L1B2Io<R>& io, double lambda_, double sigma_, double delta_,
+                           double chi_lambda_, spx_allreduce_sum_fn reduce, void* user, int32_t* passes_out,
+                           double* psi_out) {
   SPX_REQUIRE(ctx != nullptr, "null context");
   SPX_REQUIRE(n >= 0, "n < 0");
+  R* const y = io.y;
+  const R *const xk = io.xk, *const sj = io.sj, *const q = io.q;
   SPX_REQUIRE(n == 0 || (y && xk && sj && q), "null device vector");
   DeviceGuard guard(ctx->device);
   const R lam = (R)lambda_, sig = (R)sigma_, delta = (R)delta_, chil = (R)chi_lambda_;
   const R ls = lam * sig;
+  const char* const who = io.grad ? "spx_step_l1b2" : "spx_prox_l1b2";  // the entry point, for error messages
   int passes = 0;
-  // y as scratch for mid = sj + q while the search runs (2R per pass instead of 3R): only when it overlaps no input
-  auto disjoint = [&](const R* p) {
-    return (const char*)p + (size_t)n * sizeof(R) <= (const char*)y || (const char*)y + (size_t)n * sizeof(R) <= (const char*)p;
-  };
-  const bool can_stash = n > 0 && disjoint(xk) && disjoint(sj) && disjoint(q);
+  // y as scratch for mid = sj + q while the search runs (2R per pass instead of 3R), and the finish as the check of an
+  // unverified root (after a failed check the search re-reads its inputs): only when no output overlaps an input.
+  // Otherwise (prox!(y, ψ, y, σ), or the step's x <- x + s) every pass reads xk, sj, q and the search converges by
+  // evaluation; the finish reads each element's operands before it writes its outputs.
+  auto clear_of_inputs = [&](const R* p) { return !overlap<R>(p, xk, n) && !overlap<R>(p, sj, n) && !overlap<R>(p, q, n); };
+  const bool can_stash = n > 0 && clear_of_inputs(y) && clear_of_inputs(io.xsy);
   bool stashed = false;
   // K residuals per pass: f_k = η_k - χ(ProjB(-xk η_k/Δ)) and their derivatives
   // f'_k = 1 - χ (Σ w dw/dscale) / (‖w‖ Δ)
@@ -290,14 +291,14 @@ static int32_t prox_l1b2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const R* sj
     // the search proper) also stores mid into y; later passes read it back instead of sj and q
     const int mode = (!can_stash || passes == 0) ? 0 : (stashed ? 2 : 1);
     int32_t st = norm_pass<R>(ctx, n, xk, mode == 2 ? (const R*)y : sj, q, ls, use_scale ? scale : nullptr, m, ss,
-                              ss + m, mode, y);
+                              ss + m, mode, y, io.grad && mode != 2, io.mnu);
     if (mode == 1) stashed = true;
     if (st != SPX_OK) return st;
     ++passes;
     if (reduce) {
       st = reduce(user, ss, 2 * m);
       if (st != SPX_OK) {
-        set_error("spx_prox_l1b2: all-reduce callback failed (%d)", (int)st);
+        set_error("%s: all-reduce callback failed (%d)", who, (int)st);
         return st;
       }
     }
@@ -310,22 +311,33 @@ static int32_t prox_l1b2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const R* sj
     }
     return SPX_OK;
   };
-  auto finish = [&](bool use_scale, R scale, R post) -> int32_t {
-    double s = 0.0, s2 = 0.0;
-    int32_t st = finish_pass<R>(ctx, n, y, xk, sj, q, ls, use_scale, scale, post, psi_out ? &s : nullptr,
-                                psi_out ? &s2 : nullptr, stashed);
+  // the finish pass: y = ProjB(-xk scale) post - sj and, when v is given, v = {Σ|xk+sj+y|, Σ(sj+y)²} -- for the step
+  // always, with xsy written and v[2..3] = {Σs², Σ∇f·s} -- all-reduced in one call when the vector is sharded
+  auto finish_pass_io = [&](bool use_scale, R scale, R post, double* v) -> int32_t {
+    int32_t st = io.grad ? step_l1b2_finish<R>(ctx, n, y, io.xsy, xk, sj, q, stashed ? y : nullptr, sig, ls, use_scale,
+                                               scale, post, v)
+                         : finish_pass<R>(ctx, n, y, xk, sj, q, ls, use_scale, scale, post, v ? &v[0] : nullptr,
+                                          v ? &v[1] : nullptr, stashed);
     ++passes;
-    if (passes_out) *passes_out = passes;
-    if (st != SPX_OK || psi_out == nullptr) return st;
-    if (reduce) {
-      double v[2] = {s, s2};
-      st = reduce(user, v, 2);
-      if (st != SPX_OK) return st;
-      s = v[0];
-      s2 = v[1];
+    if (st != SPX_OK || v == nullptr || reduce == nullptr) return st;
+    return reduce(user, v, io.grad ? 4 : 2);
+  };
+  // ψ(y) = h(xk+sj+y) + IndBallL2(Δ)(sj+y)   shiftedNormL1B2.jl:32;  the step's sums beside it
+  auto results = [&](const double* v) {
+    if (psi_out)
+      *psi_out = in_ball_l2<R>((R)std::sqrt(v[1]), delta) ? (double)(lam * (R)v[0]) : std::numeric_limits<double>::infinity();
+    if (io.sums) {
+      io.sums[0] = v[2];
+      io.sums[1] = v[3];
     }
-    // ψ(y) = h(xk+sj+y) + IndBallL2(Δ)(sj+y)   shiftedNormL1B2.jl:32
-    *psi_out = in_ball_l2<R>((R)std::sqrt(s2), delta) ? (double)(lam * (R)s) : std::numeric_limits<double>::infinity();
+  };
+  auto finish = [&](bool use_scale, R scale, R post) -> int32_t {
+    double v[4] = {0.0, 0.0, 0.0, 0.0};
+    const bool sums = psi_out != nullptr || io.grad;
+    int32_t st = finish_pass_io(use_scale, scale, post, sums ? v : nullptr);
+    if (passes_out) *passes_out = passes;
+    if (st != SPX_OK || !sums) return st;
+    results(v);
     return SPX_OK;
   };
 
@@ -371,7 +383,7 @@ static int32_t prox_l1b2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const R* sj
   };
   R eta = delta;
   int clusters = 0;
-  bool unverified_ok = can_stash;  // a failed check re-reads q, which must not have been overwritten by y
+  bool unverified_ok = can_stash;  // a failed check re-reads the inputs, which y (and xsy) must not have overwritten
   R b0 = std::max(R(2) * pts.back(), pts.back() + R(1));
   for (;;) {
     // bracket = the largest evaluated point with f < 0 and the smallest with f > 0 (f is increasing)
@@ -384,7 +396,7 @@ static int32_t prox_l1b2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const R* sj
     }
     if (pz) { eta = pz->x; break; }
     if (!pa || passes > 200) {
-      set_error("spx_prox_l1b2: no sign change of the trust-region residual");
+      set_error("%s: no sign change of the trust-region residual", who);
       return SPX_E_NOROOT;
     }
     if (!pb) {  // the ladder did not reach the root: the reference's own guesses max(2a, a+1) 4^k, and a Newton point
@@ -403,7 +415,7 @@ static int32_t prox_l1b2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const R* sj
       for (R x : pts)
         if (x > pa->x) in.push_back(x);
       if (in.empty()) {
-        set_error("spx_prox_l1b2: no sign change of the trust-region residual");
+        set_error("%s: no sign change of the trust-region residual", who);
         return SPX_E_NOROOT;
       }
       st = eval(in, true, f, df);
@@ -424,26 +436,17 @@ static int32_t prox_l1b2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const R* sj
     // bracket narrow enough for the interpolant to be good to an ulp: x̂ goes to the finish pass, which checks it
     const R narrow = (sizeof(R) == 8 ? R(1e-6) : R(2e-4)) * a;
     if (unverified_ok && clusters >= 1 && width <= narrow) {
-      double s = 0.0, s2 = 0.0;
+      double v[4] = {0.0, 0.0, 0.0, 0.0};
       const R scale = xh / delta, post = delta / xh;
-      st = finish_pass<R>(ctx, n, y, xk, sj, q, ls, true, scale, post, &s, &s2, stashed);
+      st = finish_pass_io(true, scale, post, v);
       if (st != SPX_OK) return st;
-      ++passes;
       stashed = false;  // y now holds the result, not sj + q
-      if (reduce) {
-        double v[2] = {s, s2};
-        st = reduce(user, v, 2);
-        if (st != SPX_OK) return st;
-        s = v[0];
-        s2 = v[1];
-      }
       // ||w|| = ||sj + y|| η/Δ;  f(x̂) = x̂ - χ ||w||
-      const R nw = (R)(std::sqrt(s2) * ((double)xh / (double)delta));
+      const R nw = (R)(std::sqrt(v[1]) * ((double)xh / (double)delta));
       const R fx = xh - chil * nw;
       if (std::fabs(fx) <= R(8) * ulp_of(xh)) {
         if (passes_out) *passes_out = passes;
-        if (psi_out)
-          *psi_out = in_ball_l2<R>((R)std::sqrt(s2), delta) ? (double)(lam * (R)s) : std::numeric_limits<double>::infinity();
+        results(v);
         return SPX_OK;
       }
       unverified_ok = false;  // re-enter the search with what the check measured (slope unknown: reuse the nearer end's)
@@ -468,6 +471,32 @@ static int32_t prox_l1b2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const R* sj
   return finish(true, eta / delta, delta / eta);
 }
 
+template <class R>
+static int32_t prox_l1b2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const R* sj, const R* q, double lambda,
+                         double sigma, double delta, double chi_lambda, spx_allreduce_sum_fn reduce, void* user,
+                         int32_t* passes_out, double* psi_out) {
+  L1B2Io<R> io;
+  io.y = y; io.xk = xk; io.sj = sj; io.q = q;
+  return l1b2_search<R>(ctx, n, io, lambda, sigma, delta, chi_lambda, reduce, user, passes_out, psi_out);
+}
+
+// the solver step: the search with σ = ν on q = fl(-ν∇f), formed from ∇f inside its passes
+template <class R>
+static int32_t step_l1b2(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad, double lambda,
+                         double nu, double delta, double chi_lambda, spx_allreduce_sum_fn reduce, void* user,
+                         int32_t* passes_out, double* out3) {
+  SPX_REQUIRE(out3 != nullptr, "null result array");
+  SPX_REQUIRE(n <= 0 || !overlap<R>(s, grad, n), "s overlaps grad");
+  SPX_REQUIRE(n <= 0 || !overlap<R>(s, xsy, n), "xsy overlaps s");  // the finish reads the stash in s while it writes xsy
+  L1B2Io<R> io;
+  io.y = s; io.xk = xk; io.sj = sj; io.q = grad;
+  io.grad = true;
+  io.mnu = -(R)nu;
+  io.xsy = xsy;
+  io.sums = out3 + 1;
+  return l1b2_search<R>(ctx, n, io, lambda, nu, delta, chi_lambda, reduce, user, passes_out, out3);
+}
+
 }  // namespace spx
 
 using namespace spx;
@@ -484,6 +513,19 @@ using namespace spx;
                                                  double chi_lambda, spx_allreduce_sum_fn reduce, void* user,        \
                                                  int32_t* passes_out, double* psi_out) {                            \
     return prox_l1b2<R>(ctx, n, y, xk, sj, q, lambda, sigma, delta, chi_lambda, reduce, user, passes_out, psi_out); \
+  }                                                                                                                 \
+  extern "C" int32_t spx_step_l1b2_##SUF(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj,           \
+                                         const R* grad, double lambda, double nu, double delta, double chi_lambda,  \
+                                         int32_t* passes_out, double* out3) {                                       \
+    return step_l1b2<R>(ctx, n, s, xsy, xk, sj, grad, lambda, nu, delta, chi_lambda, nullptr, nullptr, passes_out,  \
+                        out3);                                                                                      \
+  }                                                                                                                 \
+  extern "C" int32_t spx_step_l1b2_sharded_##SUF(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj,   \
+                                                 const R* grad, double lambda, double nu, double delta,             \
+                                                 double chi_lambda, spx_allreduce_sum_fn reduce, void* user,        \
+                                                 int32_t* passes_out, double* out3) {                               \
+    return step_l1b2<R>(ctx, n, s, xsy, xk, sj, grad, lambda, nu, delta, chi_lambda, reduce, user, passes_out,      \
+                        out3);                                                                                      \
   }                                                                                                                 \
   extern "C" int32_t spx_l1b2_projnorm2_##SUF(spx_ctx* ctx, int64_t n, const R* xk, const R* sj, const R* q,        \
                                               double lambda, double sigma, int32_t nscale,                          \

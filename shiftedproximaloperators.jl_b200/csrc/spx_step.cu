@@ -39,6 +39,13 @@ template <class Op, bool IPROX = false> struct StepBlocks {
   static constexpr int value = MinBlocks<Op>::value > cap ? cap : MinBlocks<Op>::value;
 };
 
+// An operator whose ψ fills both accumulators of the first slot (L1B2StepFinish: Σ|xk+sj+s| and Σ(sj+s)²) declares
+// SUMSQ_SLOT1: Σs² then goes to the second slot's s2, beside Σ∇f·s.
+template <class Op, class = void> struct SumsqSlot1 { static constexpr bool value = false; };
+template <class Op> struct SumsqSlot1<Op, std::void_t<decltype(Op::SUMSQ_SLOT1)>> {
+  static constexpr bool value = Op::SUMSQ_SLOT1;
+};
+
 // IPROX = false: the step around prox!, c = -ν scales ∇f into q.
 // IPROX = true:  the step around iprox!, ∇f goes to the functor as loaded, c = σ shifts the diagonal (x[3]) into
 //                d = D + σ, and Σ d s² is summed as well.
@@ -61,7 +68,10 @@ __global__ void __launch_bounds__(kEwThreads, StepBlocks<Op, IPROX>::value)
       x[2] = c * g;  // q = -ν ∇f
     s = op.apply(x, i, acc);
     v = (x[0] + x[1]) + s;
-    acc.s2 = __fma_rn((double)s, (double)s, acc.s2);
+    if constexpr (SumsqSlot1<Op>::value)
+      sds = __fma_rn((double)s, (double)s, sds);
+    else
+      acc.s2 = __fma_rn((double)s, (double)s, acc.s2);
     dot = __fma_rn((double)g, (double)s, dot);
     if constexpr (IPROX) sds = __fma_rn((double)x[3] * (double)s, (double)s, sds);
   };
@@ -136,7 +146,8 @@ template <int VEC, int UNROLL, class Op, bool IPROX> static int step_blocks_per_
   return cached;
 }
 
-// launch and fold the two slots into ctx->h_result: [0] = (ψ sum, Σs², flag), [1] = (Σ∇f·s, Σ d s² or 0)
+// launch and fold the two slots into ctx->h_result: [0] = (ψ sum, Σs², flag), [1] = (Σ∇f·s, Σ d s² or 0);
+// SUMSQ_SLOT1 operators: [0] = (their two ψ sums), [1] = (Σ∇f·s, Σs²)
 template <bool IPROX, class Op, class R>
 static int32_t step_launch(spx_ctx* ctx, const Op& op, R c, R* xsy, int64_t n) {
   constexpr int VECW = 16 / (int)sizeof(R);
@@ -354,6 +365,33 @@ int32_t step_post(spx_ctx* ctx, int64_t n, R* xsy, const R* xk, const R* sj, con
   return SPX_OK;
 }
 
+// The finish pass of the ShiftedNormL1B2 step's root search (spx_l1b2.cu): s = ProjB(-xk scale) post - sj with
+// q = (-ν)∇f, xsy = (xk + sj) + s (xsy may be NULL), and v = {Σ|xk+sj+s|, Σ(sj+s)², Σs², Σ∇f·s}.  mid: the search's
+// stash of sj + q (it is s itself), NULL when there is none.  Its grid is step_kernel's, not the prox! finish's
+// (ew_kernel): where the two differ, Σ(sj+s)² -- and with it the check of an unverified root -- is summed in another order.
+template <class R>
+int32_t step_l1b2_finish(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad, const R* mid,
+                         R nu, R ls, bool use_scale, R scale, R post, double* v) {
+  L1B2StepFinish<R> op;
+  op.in[0] = xk; op.in[1] = sj; op.in[2] = grad; op.in[3] = mid;
+  op.fill[0] = op.fill[1] = op.fill[2] = op.fill[3] = R(0);
+  op.y = s;
+  op.f = L1B2Finish<R, true>{};
+  op.f.ls = ls; op.f.scale = scale; op.f.post = post; op.f.use_scale = use_scale;
+  op.f.have_mid = mid != nullptr;
+  int32_t st = step_launch<false>(ctx, op, -nu, xsy, n);
+  if (st != SPX_OK) return st;
+  v[0] = ctx->h_result[0].s;
+  v[1] = ctx->h_result[0].s2;
+  v[2] = ctx->h_result[1].s2;
+  v[3] = ctx->h_result[1].s;
+  return SPX_OK;
+}
+
+template int32_t step_l1b2_finish<double>(spx_ctx*, int64_t, double*, double*, const double*, const double*,
+                                          const double*, const double*, double, double, bool, double, double, double*);
+template int32_t step_l1b2_finish<float>(spx_ctx*, int64_t, float*, float*, const float*, const float*, const float*,
+                                         const float*, float, float, bool, float, float, double*);
 template int32_t step_pre<double>(spx_ctx*, int64_t, double*, const double*, double);
 template int32_t step_pre<float>(spx_ctx*, int64_t, float*, const float*, double);
 template int32_t step_post<double>(spx_ctx*, int64_t, double*, const double*, const double*, const double*, const double*,

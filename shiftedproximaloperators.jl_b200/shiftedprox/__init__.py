@@ -560,6 +560,27 @@ class ShiftedNormL1B2(ShiftedProximableFunction):
         self.last_passes = passes.value
         return (y, out.value) if want_value else y
 
+    def _step_args(self, s, grad, nu, xsy):
+        self._check(s, grad, ("s", "grad"))
+        if xsy is not None:
+            _vec(xsy, self.xk, "xsy")
+        span = s.numel() * s.element_size()
+        if s.numel() > 0 and abs(s.data_ptr() - grad.data_ptr()) < span:
+            raise ValueError("step_: s must not overlap grad")
+        if s.numel() > 0 and xsy is not None and abs(s.data_ptr() - xsy.data_ptr()) < span:
+            raise ValueError("step_: xsy must not overlap s")
+        return (C.c_int64(self.n), _p(s), _p(xsy), _p(self.xk), _p(self.sj), _p(grad), C.c_double(self.h.lam),
+                C.c_double(nu), C.c_double(self.Delta), C.c_double(self.chi.lam))
+
+    def step_(self, s, grad, nu, xsy=None):
+        """spx_step_l1b2_*: the whole step inside the passes of prox!'s own root search -- q = -ν∇f is formed from ∇f
+        in every pass, the finish writes s and xsy and sums ψ(s), Σs², Σ∇f·s.  s is bit-identical to
+        prox_(y, ψ, -ν∇f, ν) into a y that overlaps no input; `last_passes` is set as by prox_."""
+        out, passes = (C.c_double * 3)(), C.c_int32()
+        self._call("step_l1b2", *self._step_args(s, grad, nu, xsy), C.byref(passes), out)
+        self.last_passes = passes.value
+        return s, StepResult(out[0], math.sqrt(out[1]), out[2])
+
     def __call__(self, y):  # shiftedNormL1B2.jl:32
         _vec(y, self.xk, "y")
         out = C.c_double()

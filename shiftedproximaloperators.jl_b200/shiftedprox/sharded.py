@@ -285,6 +285,19 @@ def prox_l1b2_sharded_(y_local, psi, q_local, sigma, group=None, want_value=Fals
     return (y_local, out.value) if want_value else y_local
 
 
+def step_l1b2_sharded_(s_local, psi, grad_local, nu, xsy_local=None, group=None):
+    """ShiftedNormL1B2 solver step (ShiftedNormL1B2.step_) on a sharded vector: the search's partial sums go through
+    one all-reduce per pass, the finish's four sums (ψ's two, Σs², Σ∇f·s) through one more.  Returns
+    (s_local, StepResult) with the whole-vector scalars, identical on every rank."""
+    from . import _lib as L, StepResult
+
+    cb = L.ALLREDUCE_FN(_make_reduce(psi.xk.device, group))
+    out, passes = (C.c_double * 3)(), C.c_int32()
+    psi._call("step_l1b2_sharded", *psi._step_args(s_local, grad_local, nu, xsy_local), cb, None, C.byref(passes), out)
+    psi.last_passes = passes.value
+    return s_local, StepResult(out[0], math.sqrt(out[1]), out[2])
+
+
 # ----------------------------------------------------- single-vector top-r sharded ---
 def prox_indballl0_sharded_(y_local, psi, q_local, n_global: int, group=None):
     """ShiftedIndBallL0(BInf) prox! of ONE vector spread over the ranks in rank order (this rank holds

@@ -173,6 +173,49 @@ def main():
         timeit("prox_l1b2", lambda: sp.prox_(y, psi, q, sigma), 3 * R + (4 * R if nsearch else 0) + 2 * R * max(nsearch - 1, 0) + 4 * R,
                note=f"{passes - 1} norm passes (3R, 3R+1W, then 2R each) + 1 finish (4R)")
         timeit("prox_l1b2_inactive", lambda: sp.prox_(y, psi0, q, sigma), 7 * R, note="1 norm pass + finish")
+    # the ShiftedNormL1B2 step (q plays ∇f, ν = sigma): the one call spx_step_l1b2 against the base-class composition
+    # (spx_step_pre, prox! in place with ψ, spx_step_post), ball active, alternated three times: the comparison is what
+    # these rows are for.  The composed form takes the in-place prox! route (no stash, no unverified finish), so its s is
+    # held to the L1B2 bar of the fused s, which must equal the stand-alone out-of-place prox!'s bit for bit.
+    if any(re.search(args.only, nm) for nm in ("step_l1b2", "step_l1b2_composed", "step_l1b2_inactive")):
+        nu = sigma
+        xsy_l, s2, y2 = torch.empty_like(y), torch.empty_like(y), torch.empty_like(y)
+        qn = q * torch.tensor(-nu, dtype=tdt, device=dev)  # fl(-ν∇f)
+        psi0 = two(sp.NormL1(lam), 1e30, sp.NormL2(1.0))
+        sp.prox_(y, psi0, qn, nu)
+        full = float(torch.linalg.vector_norm((y + sj).double()))
+        psi = two(sp.NormL1(lam), 0.5 * full, sp.NormL2(1.0))
+        sp.prox_(y2, psi, qn, nu)  # the stand-alone out-of-place prox!
+        _, r1 = sp.step_(y, psi, q, nu, xsy=xsy_l)
+        fused = psi.last_passes
+        same = torch.equal(y, y2)
+        _, r2 = sp.ShiftedProximableFunction.step_(psi, s2, q, nu, xsy=xsy_l)
+        composed = psi.last_passes
+        ulps = 64 if R == 8 else 16
+        tol = ulps * torch.finfo(tdt).eps * (y.double().abs() + sj.double().abs() + 1)
+        within = bool(((s2.double() - y.double()).abs() <= tol).all())
+        del tol
+        sp.step_(s2, psi0, q, nu, xsy=xsy_l)
+        inactive = psi0.last_passes
+        print(f"step_l1b2: fused s bit-identical to the out-of-place prox!: {same}; composed s within "
+              f"{ulps} ulp of |s| + |sj| + 1: {within}; passes fused {fused}, composed prox! {composed}, inactive "
+              f"{inactive}; scalars {tuple(r1)} vs {tuple(r2)}", flush=True)
+        del s2, y2, qn
+        # bytes per pass: fused -- decision pass 3R (xk, sj, ∇f), first search pass 3R + 1W (stashes mid in s), later
+        # passes 2R (xk, mid), finish 4R + 2W (xk, sj, mid, ∇f -> s, xsy; 3R + 2W without a stash);
+        # composed -- step_pre 1R + 1W, every norm pass 3R (in place: no stash), finish 3R + 1W, step_post 4R + 1W
+        nsearch = fused - 2
+        fused_b = 3 * R + (4 * R + 2 * R * (nsearch - 1) + 6 * R if nsearch > 0 else 5 * R)
+        composed_b = 2 * R + 3 * R * (composed - 1) + 4 * R + 5 * R
+        for _ in range(3):
+            timeit("step_l1b2", lambda: sp.step_(y, psi, q, nu, xsy=xsy_l), fused_b,
+                   note=f"{fused} passes: {fused - 1} norm passes (3R, 3R+1W, then 2R each) + finish (4R+2W)")
+            timeit("step_l1b2_composed", lambda: sp.ShiftedProximableFunction.step_(psi, y, q, nu, xsy=xsy_l),
+                   composed_b, note=f"{composed + 2} passes: step_pre (1R+1W), {composed - 1} norm passes (3R) + "
+                                    f"finish (3R+1W) in place, step_post (4R+1W)")
+        timeit("step_l1b2_inactive", lambda: sp.step_(y, psi0, q, nu, xsy=xsy_l), 8 * R,
+               note=f"{inactive} passes: decision pass (3R) + finish (3R+2W)")
+        del xsy_l
     # groups of 64 (and ragged)
     for gname in ("g64", "ragged"):
         names = [f"prox_groupl2_{gname}", f"value_groupl2_{gname}", f"prox_groupl2binf_{gname}",
