@@ -335,105 +335,92 @@ typedef struct spx_box_job_f32 {
                                   const spx_bound* u, const spx_sel* sel, int32_t boxed,         \
                                   double* out_host);                                             \
   /* ------------------------------ fused solver step (SURVEY.md §8f rank 1) */                 \
-  /* The sweeps a solver iteration wraps around every prox! (R2 / TR of RegularizedOptimization.jl, */ \
-  /* reference README.md:17), in the one pass of the prox! itself:                                */ \
-  /*   q = (-nu) .* grad;  prox!(s, ψ, q, nu)   [the method bodies cited at spx_prox_* above]      */ \
-  /*   xsy = (xk + sj) + s                      [ψ's argument, ShiftedProximalOperators.jl:52;     */ \
-  /*                                             xsy == NULL: not written]                         */ \
-  /*   out3_host[0] = ψ(s)                      [ShiftedProximalOperators.jl:51-54; Box forms      */ \
-  /*                                             shiftedNormL1Box.jl:70-82: Inf outside the box]   */ \
-  /*   out3_host[1] = Σ s_i²,  out3_host[2] = Σ grad_i s_i   (Float64 sums)                        */ \
-  /* s is bit-identical to spx_prox_*(q = (-nu) .* grad rounded to R, sigma = nu).  sj == NULL: ψ   */ \
-  /* shifted once (sj = 0).  kind = SPX_H_L1, _L0, _LHALF.  The call synchronises.                 */ \
+  /* The sweeps a solver iteration wraps around every prox! (R2 / TR of RegularizedOptimization.jl,          */ \
+  /* reference README.md:17) or iprox! (R2DH / TRDH), in one call:                                           */ \
+  /*   q = (-nu) .* grad   (spx_step_*)    rounded to R like the caller's broadcast                          */ \
+  /*   d = D .+ dshift     (spx_istep_*)   rounded to R likewise                                             */ \
+  /*   s = prox!(ψ, q, nu) or iprox!(ψ, grad, d)   [the method bodies cited at spx_prox_* / spx_iprox_*]     */ \
+  /*   xsy = (xk + sj) + s                         [ψ's argument, ShiftedProximalOperators.jl:52;            */ \
+  /*                                                xsy == NULL: not written]                                */ \
+  /*   out3_host = {ψ(s), Σ s_i², Σ grad_i s_i}    [ψ(s): ShiftedProximalOperators.jl:51-54, Inf outside     */ \
+  /*                                                the type's box or ball]                                  */ \
+  /*   out4_host = out3_host and Σ d_i s_i²        (spx_istep_*)                                             */ \
+  /* The sums are in Float64.  s is bit for bit the type's spx_prox_* of that q with sigma = nu (spx_iprox_* */ \
+  /* of grad and that d).  sj == NULL reads as zeros (ψ shifted once) for spx_step_sep / _box and            */ \
+  /* spx_istep_*; the other steps need sj (zeros when ψ is shifted once).  Every step synchronises, and      */ \
+  /* its scalars are all-reduced when the context reduces scalars.                                           */ \
+  /* Aliasing, for n > 0: no output (s, xsy) overlaps an input (xk, sj, grad, D, l->vec, u->vec) or the      */ \
+  /* other output partially, and beyond that (anything else: SPX_E_INVALID)                                  */ \
+  /*                                   s == grad   s == xk or sj   xsy == an input or s                      */ \
+  /*   spx_step_sep / _box, istep_*    yes         yes             yes                                       */ \
+  /*   groupl2, groupl2binf, indballl0 no          no              yes                                       */ \
+  /*   l1b2, l1b2_sharded              no          yes             yes, but xsy must not overlap s           */ \
+  /* The one-pass forms read every element's (group's) operands before they write its results.  The          */ \
+  /* composed forms below write q into s before prox! reads xk and sj, and spx_step_post reads grad;         */ \
+  /* the search of spx_step_l1b2 keeps its stash in s while the finish writes xsy.                           */ \
+  /* kind = SPX_H_L1, _L0, _LHALF: one pass                                                                  */ \
   int32_t spx_step_sep_##SUF(spx_ctx* ctx, int32_t kind, int64_t n, R* s, R* xsy, const R* xk,   \
                              const R* sj, const R* grad, double lambda, double nu,               \
                              double* out3_host);                                                 \
-  /* the same step for the Box / BInf forms; op: 0 L1Box, 1 L0Box, 2 LhalfBox */                 \
+  /* the Box / BInf forms; op: 0 L1Box, 1 L0Box, 2 LhalfBox: one pass                                        */ \
   int32_t spx_step_box_##SUF(spx_ctx* ctx, int32_t op, int64_t n, R* s, R* xsy, const R* xk,     \
                              const R* sj, const R* grad, const spx_bound* l, const spx_bound* u, \
                              const spx_sel* sel, double lambda, double nu, double* out3_host);   \
-  /* The fused step around iprox! (diagonal model: the R2DH / TRDH iterations of               */ \
-  /* RegularizedOptimization.jl), in the one pass of the iprox! itself:                          */ \
-  /*   d = D .+ dshift                          [rounded to R like the caller's broadcast]       */ \
-  /*   iprox!(s, ψ, grad, d)                    [shiftedNormL1.jl:60-75, shiftedNormL0.jl:61-80, */ \
-  /*                                             shiftedNormL1Box.jl:131-225,                    */ \
-  /*                                             shiftedNormL0Box.jl:137-231]                    */ \
-  /*   xsy = (xk + sj) + s                      [xsy == NULL: not written]                       */ \
-  /*   out4_host[0] = ψ(s)                      [ShiftedProximalOperators.jl:51-54; Box forms    */ \
-  /*                                             shiftedNormL1Box.jl:70-82: Inf outside the box] */ \
-  /*   out4_host[1] = Σ s_i², out4_host[2] = Σ grad_i s_i, out4_host[3] = Σ d_i s_i² (Float64)   */ \
-  /* s is bit-identical to spx_iprox_*(g = grad, d = D .+ dshift rounded to R).  sj == NULL: ψ    */ \
-  /* shifted once (sj = 0).  kind = SPX_H_L1, _L0 (no iprox! for _LHALF: SPX_E_INVALID).  The     */ \
-  /* `@assert d[i] > 0` of the unboxed forms applies to d: SPX_E_ASSERT_D and *first_bad_d (may   */ \
-  /* be NULL) as for spx_iprox_l1; s is written in full either way.  s may be grad and xsy may be */ \
-  /* xk (each element's operands are read before its results are written).  The call            */ \
-  /* synchronises; the four sums are all-reduced when the context reduces scalars.               */ \
+  /* kind = SPX_H_L1, _L0 (no iprox! for _LHALF: SPX_E_INVALID): one pass.  The `@assert d[i] > 0` of the    */ \
+  /* unboxed forms applies to d: SPX_E_ASSERT_D and *first_bad_d (may be NULL) as for spx_iprox_l1; s is     */ \
+  /* written in full either way.                                                                             */ \
   int32_t spx_istep_sep_##SUF(spx_ctx* ctx, int32_t kind, int64_t n, R* s, R* xsy, const R* xk,  \
                               const R* sj, const R* grad, const R* D, double dshift,             \
                               double lambda, int64_t* first_bad_d, double* out4_host);           \
-  /* the same step for the Box forms; op: 0 L1Box, 1 L0Box (2 LhalfBox: SPX_E_INVALID) */        \
+  /* the Box forms; op: 0 L1Box, 1 L0Box (2 LhalfBox: SPX_E_INVALID): one pass                               */ \
   int32_t spx_istep_box_##SUF(spx_ctx* ctx, int32_t op, int64_t n, R* s, R* xsy, const R* xk,    \
                               const R* sj, const R* grad, const R* D, double dshift,             \
                               const spx_bound* l, const spx_bound* u, const spx_sel* sel,        \
                               double lambda, double* out4_host);                                 \
-  /* The step around a prox! that is not one streaming pass (groups, top-r): the                      */ \
-  /* caller's sweeps as two passes around the operator's own entry point --                          */ \
-  /*   spx_step_pre:   q = (-nu) .* grad (rounded to R), written where s will be;                    */ \
-  /*   the type's spx_prox_* IN PLACE (y = q = s, sigma = nu, its psi_out / value entry gives ψ(s)); */ \
-  /*   spx_step_post:  xsy = (xk + sj) + s (xsy may be NULL), out2_host = {Σ s², Σ grad·s} (Float64; */ \
-  /*   all-reduced like every folded reduction when the context reduces scalars).  sj == NULL: zeros. */ \
-  /* s must not alias grad.  spx_step_post synchronises.                                             */ \
+  /* The composed form of the step around a prox! that is not one streaming pass (groups, top-r): the        */ \
+  /* caller's sweeps as two passes around the type's own entry point --                                      */ \
+  /*   spx_step_pre:   q = (-nu) .* grad (rounded to R), written where s will be;                            */ \
+  /*   the type's spx_prox_* IN PLACE (y = q = s, sigma = nu, its psi_out / value entry gives ψ(s));         */ \
+  /*   spx_step_post:  xsy = (xk + sj) + s (xsy may be NULL), out2_host = {Σ s², Σ grad·s}.                  */ \
+  /* sj == NULL: zeros.  spx_step_post synchronises.                                                         */ \
   int32_t spx_step_pre_##SUF(spx_ctx* ctx, int64_t n, R* q, const R* grad, double nu);               \
-  /* The whole step of ShiftedGroupNormL2 (shiftedGroupNormL2.jl:52-79) in one call: ONE pass when   */ \
-  /* every group of a validated layout holds <= 256 elements (spx_group_validate_offsets), the three */ \
-  /* calls above otherwise.  out3_host as for spx_step_sep.  sj must be given (zeros when ψ is       */ \
-  /* shifted once); s must not alias grad, xsy must not alias an input of the call.                   */ \
+  /* ShiftedGroupNormL2 (shiftedGroupNormL2.jl:52-79): ONE pass when every group of a validated layout       */ \
+  /* holds <= 256 elements (spx_group_validate_offsets), the composed form otherwise.  A layout rewritten    */ \
+  /* after validation so that it holds a longer group is redone in the composed form, which re-reads the     */ \
+  /* inputs: with xsy aliasing one of them, validate the layout again after rewriting it.                    */ \
   int32_t spx_step_groupl2_##SUF(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj,    \
                                  const R* grad, int64_t ngroups, const int64_t* offs,                \
                                  const R* lambda_g, double nu, double* out3_host);                   \
-  /* The whole step of ShiftedGroupNormL2Binf (shiftedGroupNormL2Binf.jl:67-119) in one call: ONE   */ \
-  /* pass when the layout is uniform (n == ngroups m, m in {16, 32, 64, 128, 256}, offs == {0, m,    */ \
-  /* 2m, ...}, ngroups > 1, 16-byte aligned vectors), the three calls above otherwise.  s is bit for */ \
-  /* bit prox!(s, ψ, (-nu) .* grad, nu).  out3_host = {ψ(s) of shiftedGroupNormL2Binf.jl:34-39 (Inf  */ \
-  /* when sj + s leaves the ball of 1.1 delta), Σ s², Σ grad·s}, the sums in Float64.  Contract as   */ \
-  /* for spx_step_groupl2; the call synchronises, the scalars are all-reduced when the context       */ \
-  /* reduces scalars.                                                                                */ \
+  /* ShiftedGroupNormL2Binf (shiftedGroupNormL2Binf.jl:67-119): ONE pass when the layout is uniform          */ \
+  /* (n == ngroups m, m in {16, 32, 64, 128, 256}, offs == {0, m, 2m, ...}, ngroups > 1, 16-byte aligned     */ \
+  /* vectors), the composed form otherwise.  ψ(s) of shiftedGroupNormL2Binf.jl:34-39: Inf when sj + s        */ \
+  /* leaves the ball of 1.1 delta.                                                                           */ \
   int32_t spx_step_groupl2binf_##SUF(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk,             \
                                      const R* sj, const R* grad, int64_t ngroups,                    \
                                      const int64_t* offs, const R* lambda_g, double nu,              \
                                      double delta, double* out3_host);                               \
-  /* The whole step of ShiftedIndBallL0 (shiftedIndBallL0.jl:54-72) and ShiftedIndBallL0BInf       */ \
-  /* (binf != 0, shiftedIndBallL0BInf.jl:73-95) for nprob problems of length n back to back: ONE     */ \
-  /* pass of the stream top-r kernel when spx_prox_indballl0 would take its stream form (16-byte    */ \
-  /* aligned vectors, n % 8 == 0, 4096 <= n <= 131072, 0 < r < n, nprob >= 2 x the SM count) and    */ \
-  /* xsy is given and overlaps no input; the calls above otherwise.  s is bit for bit               */ \
-  /* spx_prox_indballl0(nprob, n, s, xk, sj, q = (-nu) .* grad rounded to R, r, binf, delta).       */ \
-  /* out3_host = {ψ(s) as the type's ψ(y) returns it (spx_value_sep / spx_value_binf over the whole */ \
-  /* batch: the count of xk + sj + s != 0 against r; BInf: Inf when sj + s leaves the ball of       */ \
-  /* 1.1 delta, shiftedIndBallL0BInf.jl:44-49), Σ s², Σ grad·s} (Float64 sums).  sj must be given   */ \
-  /* (zeros when ψ is shifted once); s must not alias grad (SPX_E_INVALID).  The call synchronises; */ \
-  /* the scalars are all-reduced when the context reduces scalars.                                  */ \
+  /* ShiftedIndBallL0 (shiftedIndBallL0.jl:54-72) and ShiftedIndBallL0BInf (binf != 0,                       */ \
+  /* shiftedIndBallL0BInf.jl:73-95) for nprob problems of length n back to back: ONE pass of the stream      */ \
+  /* top-r kernel when spx_prox_indballl0 would take its stream form (16-byte aligned vectors, n % 8 == 0,   */ \
+  /* 4096 <= n <= 131072, 0 < r < n, nprob >= 2 x the SM count) and xsy is given and overlaps no input,      */ \
+  /* the composed form otherwise.  ψ(s) as the type's ψ(y) returns it over the whole batch (the count of     */ \
+  /* xk + sj + s != 0 against r; BInf: Inf when sj + s leaves the ball of 1.1 delta,                         */ \
+  /* shiftedIndBallL0BInf.jl:44-49).                                                                         */ \
   int32_t spx_step_indballl0_##SUF(spx_ctx* ctx, int64_t nprob, int64_t n, R* s, R* xsy,             \
                                    const R* xk, const R* sj, const R* grad, int64_t r, int32_t binf, \
                                    double delta, double nu, double* out3_host);                      \
-  /* The whole step of ShiftedNormL1B2 (shiftedNormL1B2.jl:47-64) inside the passes of its own root */ \
-  /* search: every pass forms q = (-nu) .* grad (rounded to R) on the load, the finish writes s and   */ \
-  /* xsy = (xk + sj) + s (xsy may be NULL).  s is bit for bit spx_prox_l1b2(y = s, q = (-nu) .* grad */ \
-  /* rounded to R, sigma = nu) into an s that overlaps no input.  out3_host = {ψ(s) as psi_out of     */ \
-  /* spx_prox_l1b2 (λ Σ|xk + sj + s| rounded to R, Inf when ‖sj + s‖ leaves the ball of delta,       */ \
-  /* shiftedNormL1B2.jl:32), Σ s², Σ grad·s} (Float64 sums); passes_out (may be NULL) as for          */ \
-  /* spx_prox_l1b2.  s uses itself as scratch, and the finish doubles as the check of an unverified   */ \
-  /* root, only when s and xsy overlap none of xk, sj, grad; otherwise (xsy = xk: x <- x + s) the     */ \
-  /* search converges by evaluation and each element's operands are read before its results are      */ \
-  /* written.  sj must be given (zeros when ψ is shifted once); s overlapping grad or xsy:          */ \
-  /* SPX_E_INVALID.                                                                                  */ \
-  /* The call synchronises; every decision of the search and out3_host are all-reduced when the       */ \
-  /* context reduces scalars.                                                                         */ \
+  /* ShiftedNormL1B2 (shiftedNormL1B2.jl:47-64) inside the passes of its own root search: every pass         */ \
+  /* forms q on the load, the finish writes s and xsy.  ψ(s) as psi_out of spx_prox_l1b2 (λ Σ|xk + sj + s|   */ \
+  /* rounded to R, Inf when ‖sj + s‖ leaves the ball of delta, shiftedNormL1B2.jl:32); passes_out (may be    */ \
+  /* NULL) as for spx_prox_l1b2.  s uses itself as scratch, and the finish doubles as the check of an        */ \
+  /* unverified root, only when s and xsy overlap none of xk, sj, grad; otherwise (xsy = xk: x <- x + s)     */ \
+  /* the search converges by evaluation and each element's operands are read before its results are          */ \
+  /* written.  Every decision of the search is all-reduced when the context reduces scalars.                 */ \
   int32_t spx_step_l1b2_##SUF(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj,       \
                               const R* grad, double lambda, double nu, double delta,                 \
                               double chi_lambda, int32_t* passes_out, double* out3_host);            \
-  /* the same step on this rank's shard of a sharded vector: `reduce` gets the 2K partial sums of     */ \
-  /* every norm pass and, once, the finish's four {Σ|xk + sj + s|, Σ (sj + s)², Σ s², Σ grad·s}       */ \
+  /* the same step on this rank's shard of a sharded vector: `reduce` gets the 2K partial sums of            */ \
+  /* every norm pass and, once, the finish's four {Σ|xk + sj + s|, Σ (sj + s)², Σ s², Σ grad·s}              */ \
   int32_t spx_step_l1b2_sharded_##SUF(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk,            \
                                       const R* sj, const R* grad, double lambda, double nu,          \
                                       double delta, double chi_lambda, spx_allreduce_sum_fn reduce,  \

@@ -9,6 +9,7 @@
 
 #include <cmath>
 #include <cstdio>
+#include <initializer_list>
 #include <limits>
 
 #include "../../include/shiftedprox.h"
@@ -324,10 +325,48 @@ int32_t make_sel(const spx_sel* s, int64_t n, DevSel* out);
 // fold `nblocks` partials (slot stride `stride`, `nslot` independent slots) into
 // ctx->d_result[slot], copy to the pinned mirror, synchronise
 int32_t finalize_partials(spx_ctx* ctx, int nblocks, int nslot, bool bad_is_min);
+// does [a, a + bytes) overlap [b, b + bytes); false when either is NULL
+inline bool spans_overlap(const void* a, const void* b, size_t bytes) {
+  return a != nullptr && b != nullptr && (const char*)a < (const char*)b + bytes && (const char*)b < (const char*)a + bytes;
+}
+
+// ---- the solver step entries (spx_step_*, spx_istep_*) ------------------------------------------------------------
+// The alias rule of shiftedprox.h ("The solver steps"), for steps over `bytes` of each vector.  Every entry: no
+// output (s, xsy) overlaps an input or the other output partially.  STEP_ONE_PASS (the element-wise entries: every
+// element's operands are read before its results are written) allows every exact alias.  STEP_COMPOSED (groups,
+// top-r: the composed form writes q into s before prox! reads xk and sj, and step_post reads grad) refuses any
+// overlap of s with xk, sj or grad.  STEP_L1B2 refuses any overlap of s with grad or xsy (the finish reads the
+// search's stash in s while it writes xsy).  `more`: the entry's input vectors beyond xk, sj and grad.  `fn`, the C
+// entry point, is named in the message.
+enum StepAlias { STEP_ONE_PASS, STEP_COMPOSED, STEP_L1B2 };
+int32_t step_check_alias(const char* fn, StepAlias rule, size_t bytes, const void* s, const void* xsy, const void* xk,
+                         const void* sj, const void* grad, std::initializer_list<const void*> more);
+// the checks every step entry starts with: FN its C entry point, m the elements it steps over, OUT its result array,
+// the variadic rest its input vectors beyond xk, sj and grad
+#define SPX_STEP_COMMON_CHECKS(FN, RULE, m, OUT, ...)                                                             \
+  SPX_REQUIRE(ctx != nullptr, "null context");                                                                  \
+  SPX_REQUIRE((m) >= 0, "negative size");                                                                       \
+  SPX_REQUIRE((OUT) != nullptr, "null result array");                                                           \
+  SPX_REQUIRE((m) == 0 || (s && xk && grad), "null device vector");                                             \
+  if (const int32_t st__ = spx::step_check_alias(FN, RULE, (size_t)(m) * sizeof(*s), s, xsy, xk, sj, grad, {__VA_ARGS__})) \
+    return st__;                                                                                                \
+  DeviceGuard guard__(ctx->device)
+
 // the two passes of the solver step around a prox! that is not one streaming pass (spx_step.cu)
 template <class R> int32_t step_pre(spx_ctx* ctx, int64_t n, R* q, const R* grad, double nu);
 template <class R>
 int32_t step_post(spx_ctx* ctx, int64_t n, R* xsy, const R* xk, const R* sj, const R* s, const R* grad, double* out2);
+// the composed form of such a step: q = (-ν)∇f into s, prox_in_place(&out3[0]) -- the type's prox! on s in place,
+// ψ(s) into out3[0] -- then xsy = (xk + sj) + s, out3[1] = Σs², out3[2] = Σ∇f·s
+template <class R, class Prox>
+int32_t step_composed(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad, double nu,
+                      Prox&& prox_in_place, double* out3) {
+  int32_t st = step_pre<R>(ctx, n, s, grad, nu);
+  if (st != SPX_OK) return st;
+  st = prox_in_place(&out3[0]);
+  if (st != SPX_OK) return st;
+  return step_post<R>(ctx, n, xsy, xk, sj, s, grad, out3 + 1);
+}
 // the finish pass of the ShiftedNormL1B2 step (spx_step.cu, called by the root search of spx_l1b2.cu)
 template <class R>
 int32_t step_l1b2_finish(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad, const R* mid,

@@ -12,7 +12,6 @@
 // results are deterministic.
 #include <algorithm>
 #include <cstddef>
-#include <cstdlib>
 
 #include "spx_elementwise.cuh"
 #include "spx_ops.cuh"
@@ -2418,10 +2417,7 @@ static int32_t prox_group(spx_ctx* ctx, bool binf, int64_t n, R* y, const R* xk,
     // overlaps an input partially (a group's y would land on another group's inputs) or σ, Δ are outside the range of
     // the branch-free quotient.
     unsigned char* done = nullptr;
-    const char *y0 = (const char*)y, *y1 = y0 + (size_t)n * sizeof(R);
-    auto overlaps = [&](const R* p) {
-      return p != y && (const char*)p < y1 && (const char*)p + (size_t)n * sizeof(R) > y0;
-    };
+    auto overlaps = [&](const R* p) { return p != y && spans_overlap(y, p, (size_t)n * sizeof(R)); };
     if (sigma_ok && !(overlaps(xk) || overlaps(sj) || overlaps(q))) {
       done = (unsigned char*)ctx->d_scratch + done_off;
       SPX_CUDA(cudaMemsetAsync(done, 0, (size_t)ngroups, ctx->stream));
@@ -2600,17 +2596,14 @@ __global__ void __launch_bounds__(kGroupThreads, SPX_GSTEP_MINB)
 template <class R>
 static int32_t step_groupl2(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad,
                             int64_t ngroups, const int64_t* offs, const R* lambda_g, double nu, double* out3) {
-  SPX_REQUIRE(ctx != nullptr, "null context");
   SPX_REQUIRE(n >= 0 && ngroups >= 0, "negative size");
-  SPX_REQUIRE(out3 != nullptr, "null result array");
-  SPX_REQUIRE(ngroups == 0 || (s && xk && sj && grad && offs && lambda_g), "null device vector");
-  SPX_REQUIRE(s != grad || n == 0, "s must not alias grad");
-  DeviceGuard g(ctx->device);
+  SPX_STEP_COMMON_CHECKS("spx_step_groupl2", STEP_COMPOSED, ngroups == 0 ? 0 : n, out3);
+  SPX_REQUIRE(ngroups == 0 || n == 0 || (sj && offs && lambda_g), "null device vector");
   out3[0] = out3[1] = out3[2] = 0.0;
   if (ngroups == 0 || n == 0) return SPX_OK;
   const spx_ctx::GroupCensus* census = find_census(ctx, offs, ngroups, n);
   // a validated layout whose groups all have <= 256 elements (the packed warp rounds hold every group)
-  if (ngroups > 1 && census && census->classes == 0u && std::getenv("SPX_STEP_COMPOSED") == nullptr) {
+  if (ngroups > 1 && census && census->classes == 0u) {
     int grid = 0;
     int32_t st = grid_for(ctx, (const void*)group_l2_step_kernel<R>, kGroupThreads, 0, warp_kernel_ctas(ngroups),
                           kMaxPartials / 2, true, &grid);
@@ -2628,16 +2621,9 @@ static int32_t step_groupl2(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, 
       return SPX_OK;
     }  // else: the layout is not what the census recorded -- redo the call the long way
   }
-  int32_t st = step_pre<R>(ctx, n, s, grad, nu);
-  if (st != SPX_OK) return st;
-  st = prox_group<R>(ctx, false, n, s, xk, sj, s, ngroups, offs, lambda_g, nu, 0.0, &out3[0]);
-  if (st != SPX_OK) return st;
-  double out2[2] = {0.0, 0.0};
-  st = step_post<R>(ctx, n, xsy, xk, sj, s, grad, out2);
-  if (st != SPX_OK) return st;
-  out3[1] = out2[0];
-  out3[2] = out2[1];
-  return SPX_OK;
+  return step_composed<R>(ctx, n, s, xsy, xk, sj, grad, nu, [&](double* psi) {
+    return prox_group<R>(ctx, false, n, s, xk, sj, s, ngroups, offs, lambda_g, nu, 0.0, psi);
+  }, out3);
 }
 
 // ---- the solver step of ShiftedGroupNormL2Binf ---------------------------------------------------------------------
@@ -2651,12 +2637,9 @@ template <class R>
 static int32_t step_groupl2binf(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad,
                                 int64_t ngroups, const int64_t* offs, const R* lambda_g, double nu, double delta,
                                 double* out3) {
-  SPX_REQUIRE(ctx != nullptr, "null context");
   SPX_REQUIRE(n >= 0 && ngroups >= 0, "negative size");
-  SPX_REQUIRE(out3 != nullptr, "null result array");
-  SPX_REQUIRE(ngroups == 0 || n == 0 || (s && xk && sj && grad && offs && lambda_g), "null device vector");
-  SPX_REQUIRE(s != grad || n == 0, "s must not alias grad");
-  DeviceGuard g(ctx->device);
+  SPX_STEP_COMMON_CHECKS("spx_step_groupl2binf", STEP_COMPOSED, ngroups == 0 ? 0 : n, out3);
+  SPX_REQUIRE(ngroups == 0 || n == 0 || (sj && offs && lambda_g), "null device vector");
   out3[0] = out3[1] = out3[2] = 0.0;
   if (ngroups == 0 || n == 0) return SPX_OK;
   const int64_t m = n % ngroups == 0 ? n / ngroups : 0;
@@ -2691,16 +2674,9 @@ static int32_t step_groupl2binf(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* 
       return SPX_OK;
     }  // else: offs was rewritten after validation and is no longer uniform -- redo the call the long way
   }
-  int32_t st = step_pre<R>(ctx, n, s, grad, nu);
-  if (st != SPX_OK) return st;
-  st = prox_group<R>(ctx, true, n, s, xk, sj, s, ngroups, offs, lambda_g, nu, delta, &out3[0]);
-  if (st != SPX_OK) return st;
-  double out2[2] = {0.0, 0.0};
-  st = step_post<R>(ctx, n, xsy, xk, sj, s, grad, out2);
-  if (st != SPX_OK) return st;
-  out3[1] = out2[0];
-  out3[2] = out2[1];
-  return SPX_OK;
+  return step_composed<R>(ctx, n, s, xsy, xk, sj, grad, nu, [&](double* psi) {
+    return prox_group<R>(ctx, true, n, s, xk, sj, s, ngroups, offs, lambda_g, nu, delta, psi);
+  }, out3);
 }
 
 }  // namespace spx

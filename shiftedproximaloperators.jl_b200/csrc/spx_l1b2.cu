@@ -244,10 +244,6 @@ template <class R> static bool in_ball_l2(R nw, R delta) {
   return std::fabs(nw - delta) <= tol;
 }
 
-template <class R> static bool overlap(const R* a, const R* b, int64_t n) {
-  return a && b && (const char*)a < (const char*)(b + n) && (const char*)b < (const char*)(a + n);
-}
-
 // What the search reads and writes.  prox!: q is the q vector; the finish writes y and sums ψ's two sums.  The solver
 // step (spx_step_l1b2): the q plane holds ∇f and every pass forms q = fl(mnu ∇f), mnu = -ν, on the load, so every sum of
 // the search is the prox!'s of that q bit for bit; the finish also writes xsy (may be NULL) and sums Σs², Σ∇f·s.
@@ -278,7 +274,10 @@ static int32_t l1b2_search(spx_ctx* ctx, int64_t n, const L1B2Io<R>& io, double 
   // unverified root (after a failed check the search re-reads its inputs): only when no output overlaps an input.
   // Otherwise (prox!(y, ψ, y, σ), or the step's x <- x + s) every pass reads xk, sj, q and the search converges by
   // evaluation; the finish reads each element's operands before it writes its outputs.
-  auto clear_of_inputs = [&](const R* p) { return !overlap<R>(p, xk, n) && !overlap<R>(p, sj, n) && !overlap<R>(p, q, n); };
+  auto clear_of_inputs = [&](const R* p) {
+    const size_t bytes = (size_t)n * sizeof(R);
+    return !spans_overlap(p, xk, bytes) && !spans_overlap(p, sj, bytes) && !spans_overlap(p, q, bytes);
+  };
   const bool can_stash = n > 0 && clear_of_inputs(y) && clear_of_inputs(io.xsy);
   bool stashed = false;
   // K residuals per pass: f_k = η_k - χ(ProjB(-xk η_k/Δ)) and their derivatives
@@ -485,9 +484,7 @@ template <class R>
 static int32_t step_l1b2(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad, double lambda,
                          double nu, double delta, double chi_lambda, spx_allreduce_sum_fn reduce, void* user,
                          int32_t* passes_out, double* out3) {
-  SPX_REQUIRE(out3 != nullptr, "null result array");
-  SPX_REQUIRE(n <= 0 || !overlap<R>(s, grad, n), "s overlaps grad");
-  SPX_REQUIRE(n <= 0 || !overlap<R>(s, xsy, n), "xsy overlaps s");  // the finish reads the stash in s while it writes xsy
+  SPX_STEP_COMMON_CHECKS("spx_step_l1b2", STEP_L1B2, n, out3);
   L1B2Io<R> io;
   io.y = s; io.xk = xk; io.sj = sj; io.q = grad;
   io.grad = true;

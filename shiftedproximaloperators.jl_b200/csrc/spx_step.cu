@@ -185,17 +185,28 @@ static int32_t step_run(spx_ctx* ctx, const Op& op, R nu, R* xsy, int64_t n, int
   return SPX_OK;
 }
 
-#define SPX_STEP_COMMON_CHECKS()                                                   \
-  SPX_REQUIRE(ctx != nullptr, "null context");                                     \
-  SPX_REQUIRE(n >= 0, "n < 0");                                                    \
-  SPX_REQUIRE(out3 != nullptr, "null result array");                               \
-  SPX_REQUIRE(n == 0 || (s && xk && grad), "null device vector");                  \
-  DeviceGuard guard__(ctx->device)
+int32_t step_check_alias(const char* fn, StepAlias rule, size_t bytes, const void* s, const void* xsy, const void* xk,
+                         const void* sj, const void* grad, std::initializer_list<const void*> more) {
+  auto refuse = [&](const char* what) {
+    set_error("%s: %s", fn, what);
+    return SPX_E_INVALID;
+  };
+  auto partial = [&](const void* a, const void* b) { return a != b && spans_overlap(a, b, bytes); };
+  if (rule == STEP_ONE_PASS ? partial(s, grad) : spans_overlap(s, grad, bytes)) return refuse("s overlaps grad");
+  if (rule == STEP_COMPOSED && (spans_overlap(s, xk, bytes) || spans_overlap(s, sj, bytes)))
+    return refuse("s overlaps xk or sj");
+  if (rule == STEP_L1B2 ? spans_overlap(s, xsy, bytes) : partial(s, xsy)) return refuse("xsy overlaps s");
+  for (const void* in : {xk, sj, grad})
+    if (partial(s, in) || partial(xsy, in)) return refuse("an output overlaps an input partially");
+  for (const void* in : more)
+    if (partial(s, in) || partial(xsy, in)) return refuse("an output overlaps an input partially");
+  return SPX_OK;
+}
 
 template <class R>
 static int32_t step_sep(spx_ctx* ctx, int32_t kind, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad,
                         double lambda, double nu, double* out3) {
-  SPX_STEP_COMMON_CHECKS();
+  SPX_STEP_COMMON_CHECKS("spx_step_sep", STEP_ONE_PASS, n, out3);
   const R lam = (R)lambda, sig = (R)nu;
   auto go = [&](auto op) {
     set3(op, xk, sj, grad);
@@ -214,8 +225,8 @@ template <class R>
 static int32_t step_box(spx_ctx* ctx, int32_t opc, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad,
                         const spx_bound* l, const spx_bound* u, const spx_sel* sel, double lambda, double nu,
                         double* out3) {
-  SPX_STEP_COMMON_CHECKS();
   SPX_REQUIRE(l && u, "null bounds");
+  SPX_STEP_COMMON_CHECKS("spx_step_box", STEP_ONE_PASS, n, out3, l->vec, u->vec);
   DevSel ds;
   int32_t st = make_sel(sel, n, &ds);
   if (st != SPX_OK) return st;
@@ -236,13 +247,6 @@ static int32_t step_box(spx_ctx* ctx, int32_t opc, int64_t n, R* s, R* xsy, cons
 
 // ---- the step around iprox! (diagonal model: R2DH, TRDH) --------------------------------------------------------
 // The same pass with the iprox! functors: d = D + σ in R, s = iprox!(ψ, ∇f, d), and out4 = (ψ(s), Σs², Σ∇f·s, Σ d s²).
-#define SPX_ISTEP_COMMON_CHECKS()                                                  \
-  SPX_REQUIRE(ctx != nullptr, "null context");                                     \
-  SPX_REQUIRE(n >= 0, "n < 0");                                                    \
-  SPX_REQUIRE(out4 != nullptr, "null result array");                               \
-  SPX_REQUIRE(n == 0 || (s && xk && grad && D), "null device vector");             \
-  DeviceGuard guard__(ctx->device)
-
 static void istep_sums(const spx_ctx* ctx, double* out4) {
   out4[1] = ctx->h_result[0].s2;
   out4[2] = ctx->h_result[1].s;
@@ -252,7 +256,8 @@ static void istep_sums(const spx_ctx* ctx, double* out4) {
 template <class R>
 static int32_t istep_sep(spx_ctx* ctx, int32_t kind, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad,
                          const R* D, double dshift, double lambda, int64_t* first_bad_d, double* out4) {
-  SPX_ISTEP_COMMON_CHECKS();
+  SPX_STEP_COMMON_CHECKS("spx_istep_sep", STEP_ONE_PASS, n, out4, D);
+  SPX_REQUIRE(n == 0 || D, "null device vector");
   const R lam = (R)lambda;
   auto go = [&](auto op) {
     set_iprox(op, s, xk, sj, grad, D, lam);
@@ -279,8 +284,9 @@ template <class R>
 static int32_t istep_box(spx_ctx* ctx, int32_t opc, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad,
                          const R* D, double dshift, const spx_bound* l, const spx_bound* u, const spx_sel* sel,
                          double lambda, double* out4) {
-  SPX_ISTEP_COMMON_CHECKS();
   SPX_REQUIRE(l && u, "null bounds");
+  SPX_STEP_COMMON_CHECKS("spx_istep_box", STEP_ONE_PASS, n, out4, D, l->vec, u->vec);
+  SPX_REQUIRE(n == 0 || D, "null device vector");
   if (opc != BOX_L1 && opc != BOX_L0) {
     set_error("spx_istep_box: Box operator %d has no iprox!", (int)opc);
     return SPX_E_INVALID;

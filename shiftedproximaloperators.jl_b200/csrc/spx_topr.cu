@@ -1484,10 +1484,6 @@ static bool topr_stream_ok(const spx_ctx* ctx, int64_t nprob, int64_t n, int64_t
   return aligned && !overlap && n % 8 == 0 && n >= 4096 && n <= (int64_t)kTrMaxCluster * kTrChunk && r > 0 && r < n &&
          nprob >= 2 * (int64_t)ctx->sm_count;
 }
-// does [p, p + bytes) overlap [o, o + bytes)
-static bool spans_overlap(const void* p, const void* o, size_t bytes) {
-  return p != nullptr && o != nullptr && (const char*)p < (const char*)o + bytes && (const char*)o < (const char*)p + bytes;
-}
 
 template <class R>
 static int32_t prox_indballl0(spx_ctx* ctx, int64_t nprob, int64_t n, R* y, const R* xk, const R* sj, const R* q,
@@ -1544,19 +1540,17 @@ static int32_t value_indballl0(spx_ctx* ctx, int64_t N, const float* xk, const f
 template <class R>
 static int32_t step_indballl0(spx_ctx* ctx, int64_t nprob, int64_t n, R* s, R* xsy, const R* xk, const R* sj,
                               const R* grad, int64_t r, int32_t binf, double delta, double nu, double* out3) {
-  SPX_REQUIRE(ctx != nullptr, "null context");
   SPX_REQUIRE(nprob >= 0 && n >= 0, "negative size");
-  SPX_REQUIRE(out3 != nullptr, "null result array");
   const int64_t N = nprob * n;
-  SPX_REQUIRE(N == 0 || (s && xk && sj && grad), "null device vector");
+  SPX_STEP_COMMON_CHECKS("spx_step_indballl0", STEP_COMPOSED, N, out3);
+  SPX_REQUIRE(N == 0 || sj, "null device vector");
   const size_t bytes = (size_t)N * sizeof(R);
-  SPX_REQUIRE(!spans_overlap(s, grad, bytes), "s must not alias grad");
-  DeviceGuard g(ctx->device);
   out3[0] = out3[1] = out3[2] = 0.0;
   if (N == 0) return SPX_OK;
   const bool aligned = (((uintptr_t)s | (uintptr_t)xsy | (uintptr_t)xk | (uintptr_t)sj | (uintptr_t)grad) & 15u) == 0;
-  const bool overlap = spans_overlap(s, xk, bytes) || spans_overlap(s, sj, bytes) || spans_overlap(xsy, xk, bytes) ||
-                       spans_overlap(xsy, sj, bytes) || spans_overlap(xsy, grad, bytes) || spans_overlap(xsy, s, bytes);
+  // (s overlaps no input: step_check_alias)
+  const bool overlap = spans_overlap(xsy, xk, bytes) || spans_overlap(xsy, sj, bytes) || spans_overlap(xsy, grad, bytes) ||
+                       spans_overlap(xsy, s, bytes);
   if (xsy != nullptr && topr_stream_ok<R>(ctx, nprob, n, r, aligned, overlap)) {
     TsStep<R> step{xsy, -(R)nu, 1.1 * (double)(R)delta, ctx->d_partials, 0};
     int grid = 0;
@@ -1572,18 +1566,10 @@ static int32_t step_indballl0(spx_ctx* ctx, int64_t nprob, int64_t n, R* s, R* x
     out3[2] = ctx->h_result[1].s;
     return SPX_OK;
   }
-  int32_t st = step_pre<R>(ctx, N, s, grad, nu);
-  if (st != SPX_OK) return st;
-  st = prox_indballl0<R>(ctx, nprob, n, s, xk, sj, s, r, binf, delta);
-  if (st != SPX_OK) return st;
-  st = value_indballl0(ctx, N, xk, sj, s, binf, delta, r, &out3[0]);
-  if (st != SPX_OK) return st;
-  double out2[2] = {0.0, 0.0};
-  st = step_post<R>(ctx, N, xsy, xk, sj, s, grad, out2);
-  if (st != SPX_OK) return st;
-  out3[1] = out2[0];
-  out3[2] = out2[1];
-  return SPX_OK;
+  return step_composed<R>(ctx, N, s, xsy, xk, sj, grad, nu, [&](double* psi) {
+    const int32_t st = prox_indballl0<R>(ctx, nprob, n, s, xk, sj, s, r, binf, delta);
+    return st != SPX_OK ? st : value_indballl0(ctx, N, xk, sj, s, binf, delta, r, psi);
+  }, out3);
 }
 
 }  // namespace spx

@@ -131,6 +131,12 @@ def _p(t: Optional[torch.Tensor]) -> C.c_void_p:
     return C.c_void_p(0 if t is None else t.data_ptr())
 
 
+def _overlap(a: torch.Tensor, b: torch.Tensor) -> bool:
+    """spans_overlap of the library (csrc/spx_common.cuh) on two vectors of the same length and type"""
+    nbytes = a.numel() * a.element_size()
+    return a.data_ptr() < b.data_ptr() + nbytes and b.data_ptr() < a.data_ptr() + nbytes
+
+
 def _bound(b, like: torch.Tensor, name: str) -> L.Bound:
     if isinstance(b, torch.Tensor) and b.dim() > 0:
         _vec(b, like, name)
@@ -274,8 +280,8 @@ class ShiftedProximableFunction:
         self._check(s, grad, ("s", "grad"))
         if xsy is not None:
             _vec(xsy, self.xk, "xsy")
-        if s.data_ptr() == grad.data_ptr():
-            raise ValueError("step_: s must not alias grad")
+        if _overlap(s, grad):  # spx_step_pre would overwrite ∇f before spx_step_post reads it
+            raise ValueError("step_: s overlaps grad")
         self._call("step_pre", C.c_int64(self.n), _p(s), _p(grad), C.c_double(nu))
         _, val = self.prox_(s, s, nu, want_value=True)
         out = (C.c_double * 2)()
@@ -283,37 +289,42 @@ class ShiftedProximableFunction:
         self._call("step_post", C.c_int64(self.n), _p(xsy), _p(self.xk), _p(sj), _p(s), _p(grad), out)
         return s, StepResult(val, math.sqrt(out[0]), out[1])
 
-    def _step_sep(self, s, grad, nu, xsy):
-        # spx_step_sep_*: q = -ν∇f, prox!, ψ(s), xk+sj+s, Σs², Σ∇f·s in the one pass of the prox!
+    def _lib_step(self, name, head, s, grad, xsy, tail, d=None, sj_null=False):
+        """One fused step entry of the library: spx_<name>_*(ctx, *head, s, xsy, xk, sj, grad[, d], *tail, out) with
+        out = (ψ(s), Σs², Σ∇f·s[, Σ d s²]).  The vectors are checked against ψ's here; which may share memory is the
+        library's rule (include/shiftedprox.h), its SPX_E_INVALID raised as ValueError.  sj_null: ψ shifted once passes
+        NULL for sj, which reads as the zero vector the constructor made (shift! then writes xk,
+        ShiftedProximalOperators.jl:72-79) without its traffic."""
         self._check(s, grad, ("s", "grad"))
         if xsy is not None:
             _vec(xsy, self.xk, "xsy")
-        out = (C.c_double * 3)()
-        # ψ shifted once: sj is the zero vector the constructor made (shift! then writes xk,
-        # ShiftedProximalOperators.jl:72-79) -- NULL reads it as zeros without the traffic
-        sj = self.sj if self.shifted_twice else None
-        self._call("step_sep", C.c_int32(self._H_KIND), C.c_int64(self.n), _p(s), _p(xsy), _p(self.xk), _p(sj),
-                   _p(grad), C.c_double(self.h.lam), C.c_double(nu), out)
-        return s, StepResult(out[0], math.sqrt(out[1]), out[2])
+        if d is not None:
+            _vec(d, self.xk, "d")
+        out = (C.c_double * (3 if d is None else 4))()
+        sj = None if sj_null and not self.shifted_twice else self.sj
+        vecs = (_p(s), _p(xsy), _p(self.xk), _p(sj), _p(grad)) + ((_p(d),) if d is not None else ())
+        try:
+            self._call(name, *head, *vecs, *tail, out)
+        except SpxError as e:
+            if e.status == L.SPX_E_INVALID:
+                raise ValueError(str(e)) from None
+            raise
+        if d is None:
+            return s, StepResult(out[0], math.sqrt(out[1]), out[2])
+        return s, IStepResult(out[0], math.sqrt(out[1]), out[2], out[3])
+
+    def _step_sep(self, s, grad, nu, xsy):
+        # spx_step_sep_*: q = -ν∇f, prox!, ψ(s), xk+sj+s, Σs², Σ∇f·s in the one pass of the prox!
+        return self._lib_step("step_sep", (C.c_int32(self._H_KIND), C.c_int64(self.n)), s, grad, xsy,
+                              (C.c_double(self.h.lam), C.c_double(nu)), sj_null=True)
 
     def istep_(self, s, grad, d, dshift=0.0, xsy=None):
         raise NotImplementedError(f"iprox! is not defined for {type(self).__name__}")
 
-    def _istep_check(self, s, grad, d, xsy):
-        self._check(s, grad, ("s", "grad"))
-        _vec(d, self.xk, "d")
-        if xsy is not None:
-            _vec(xsy, self.xk, "xsy")
-
     def _istep_sep(self, s, grad, d, dshift, xsy):
         # spx_istep_sep_*: D + σ, iprox!, ψ(s), xk+sj+s, Σs², Σ∇f·s, Σ d s² in the one pass of the iprox!
-        self._istep_check(s, grad, d, xsy)
-        out = (C.c_double * 4)()
-        bad = C.c_int64()
-        sj = self.sj if self.shifted_twice else None  # ψ shifted once: NULL reads zeros (see _step_sep)
-        self._call("istep_sep", C.c_int32(self._H_KIND), C.c_int64(self.n), _p(s), _p(xsy), _p(self.xk), _p(sj),
-                   _p(grad), _p(d), C.c_double(dshift), C.c_double(self.h.lam), C.byref(bad), out)
-        return s, IStepResult(out[0], math.sqrt(out[1]), out[2], out[3])
+        return self._lib_step("istep_sep", (C.c_int32(self._H_KIND), C.c_int64(self.n)), s, grad, xsy,
+                              (C.c_double(dshift), C.c_double(self.h.lam), C.byref(C.c_int64())), d=d, sj_null=True)
 
     def __repr__(self):  # Base.show  (ShiftedProximalOperators.jl:123-133)
         return f"{type(self).__name__}(n={self.n}, dtype={self.xk.dtype}, shifted_twice={self.shifted_twice})"
@@ -497,26 +508,17 @@ class _BoxBase(ShiftedProximableFunction):
         return (y, out.value) if want_value else y
 
     def step_(self, s, grad, nu, xsy=None):
-        self._check(s, grad, ("s", "grad"))
-        if xsy is not None:
-            _vec(xsy, self.xk, "xsy")
         lb, ub = self._bounds()
-        out = (C.c_double * 3)()
-        self._call("step_box", C.c_int32(_BOX_OP[self._BOX_NAME]), C.c_int64(self.n), _p(s), _p(xsy), _p(self.xk),
-                   _p(self.sj), _p(grad), C.byref(lb), C.byref(ub), self._sel.ref(), C.c_double(self.h.lam),
-                   C.c_double(nu), out)
-        return s, StepResult(out[0], math.sqrt(out[1]), out[2])
+        return self._lib_step("step_box", (C.c_int32(_BOX_OP[self._BOX_NAME]), C.c_int64(self.n)), s, grad, xsy,
+                              (C.byref(lb), C.byref(ub), self._sel.ref(), C.c_double(self.h.lam), C.c_double(nu)))
 
     def istep_(self, s, grad, d, dshift=0.0, xsy=None):
         if self._BOX_NAME == "lhalfbox":
             raise NotImplementedError("iprox! is not defined for ShiftedRootNormLhalfBox")
-        self._istep_check(s, grad, d, xsy)
         lb, ub = self._bounds()
-        out = (C.c_double * 4)()
-        self._call("istep_box", C.c_int32(_BOX_OP[self._BOX_NAME]), C.c_int64(self.n), _p(s), _p(xsy), _p(self.xk),
-                   _p(self.sj), _p(grad), _p(d), C.c_double(dshift), C.byref(lb), C.byref(ub), self._sel.ref(),
-                   C.c_double(self.h.lam), out)
-        return s, IStepResult(out[0], math.sqrt(out[1]), out[2], out[3])
+        return self._lib_step("istep_box", (C.c_int32(_BOX_OP[self._BOX_NAME]), C.c_int64(self.n)), s, grad, xsy,
+                              (C.c_double(dshift), C.byref(lb), C.byref(ub), self._sel.ref(), C.c_double(self.h.lam)),
+                              d=d)
 
     def __call__(self, y):  # shiftedNormL1Box.jl:70-82
         _vec(y, self.xk, "y")
@@ -560,26 +562,20 @@ class ShiftedNormL1B2(ShiftedProximableFunction):
         self.last_passes = passes.value
         return (y, out.value) if want_value else y
 
-    def _step_args(self, s, grad, nu, xsy):
-        self._check(s, grad, ("s", "grad"))
-        if xsy is not None:
-            _vec(xsy, self.xk, "xsy")
-        span = s.numel() * s.element_size()
-        if s.numel() > 0 and abs(s.data_ptr() - grad.data_ptr()) < span:
-            raise ValueError("step_: s must not overlap grad")
-        if s.numel() > 0 and xsy is not None and abs(s.data_ptr() - xsy.data_ptr()) < span:
-            raise ValueError("step_: xsy must not overlap s")
-        return (C.c_int64(self.n), _p(s), _p(xsy), _p(self.xk), _p(self.sj), _p(grad), C.c_double(self.h.lam),
-                C.c_double(nu), C.c_double(self.Delta), C.c_double(self.chi.lam))
+    def _step_l1b2(self, name, s, grad, nu, xsy, reduce=()):
+        # spx_step_l1b2_* and spx_step_l1b2_sharded_* (reduce: the all-reduce callback and its user pointer)
+        passes = C.c_int32()
+        res = self._lib_step(name, (C.c_int64(self.n),), s, grad, xsy,
+                             (C.c_double(self.h.lam), C.c_double(nu), C.c_double(self.Delta), C.c_double(self.chi.lam),
+                              *reduce, C.byref(passes)))
+        self.last_passes = passes.value
+        return res
 
     def step_(self, s, grad, nu, xsy=None):
         """spx_step_l1b2_*: the whole step inside the passes of prox!'s own root search -- q = -ν∇f is formed from ∇f
         in every pass, the finish writes s and xsy and sums ψ(s), Σs², Σ∇f·s.  s is bit-identical to
         prox_(y, ψ, -ν∇f, ν) into a y that overlaps no input; `last_passes` is set as by prox_."""
-        out, passes = (C.c_double * 3)(), C.c_int32()
-        self._call("step_l1b2", *self._step_args(s, grad, nu, xsy), C.byref(passes), out)
-        self.last_passes = passes.value
-        return s, StepResult(out[0], math.sqrt(out[1]), out[2])
+        return self._step_l1b2("step_l1b2", s, grad, nu, xsy)
 
     def __call__(self, y):  # shiftedNormL1B2.jl:32
         _vec(y, self.xk, "y")
@@ -592,15 +588,8 @@ class ShiftedNormL1B2(ShiftedProximableFunction):
 def _step_indballl0(psi, s, grad, nu, xsy, binf, delta):
     # spx_step_indballl0_*: the whole step in one pass of the stream top-r kernel on a batch it takes, the composed form
     # (step_pre, prox! in place, ψ(s), step_post) otherwise -- decided in the library
-    psi._check(s, grad, ("s", "grad"))
-    if xsy is not None:
-        _vec(xsy, psi.xk, "xsy")
-    if s.numel() > 0 and s.data_ptr() == grad.data_ptr():
-        raise ValueError("step_: s must not alias grad")
-    out = (C.c_double * 3)()
-    psi._call("step_indballl0", C.c_int64(psi.nprob), C.c_int64(psi.n // psi.nprob), _p(s), _p(xsy), _p(psi.xk),
-              _p(psi.sj), _p(grad), C.c_int64(psi.h.r), C.c_int32(binf), C.c_double(delta), C.c_double(nu), out)
-    return s, StepResult(out[0], math.sqrt(out[1]), out[2])
+    return psi._lib_step("step_indballl0", (C.c_int64(psi.nprob), C.c_int64(psi.n // psi.nprob)), s, grad, xsy,
+                         (C.c_int64(psi.h.r), C.c_int32(binf), C.c_double(delta), C.c_double(nu)))
 
 
 class ShiftedIndBallL0(ShiftedProximableFunction):
@@ -708,15 +697,8 @@ class ShiftedGroupNormL2(_GroupBase):
     def step_(self, s, grad, nu, xsy=None):
         """spx_step_groupl2_*: the whole step in one pass when every group holds <= 256 elements (the C4 shape), the
         two passes around prox! otherwise (decided in the library from the census of the validated layout)."""
-        self._check(s, grad, ("s", "grad"))
-        if xsy is not None:
-            _vec(xsy, self.xk, "xsy")
-        if s.data_ptr() == grad.data_ptr():
-            raise ValueError("step_: s must not alias grad")
-        out = (C.c_double * 3)()
-        self._call("step_groupl2", C.c_int64(self.n), _p(s), _p(xsy), _p(self.xk), _p(self.sj), _p(grad),
-                   C.c_int64(self.ngroups), _p(self._offs), _p(self._lam_g), C.c_double(nu), out)
-        return s, StepResult(out[0], math.sqrt(out[1]), out[2])
+        return self._lib_step("step_groupl2", (C.c_int64(self.n),), s, grad, xsy,
+                              (C.c_int64(self.ngroups), _p(self._offs), _p(self._lam_g), C.c_double(nu)))
 
 
 class ShiftedGroupNormL2Binf(_GroupBase):
@@ -746,16 +728,9 @@ class ShiftedGroupNormL2Binf(_GroupBase):
     def step_(self, s, grad, nu, xsy=None):
         """spx_step_groupl2binf_*: the whole step in one pass on a uniform layout (n == ngroups m, m = 16 ... 256, the
         C4 shape), the two passes around prox! otherwise (decided in the library)."""
-        self._check(s, grad, ("s", "grad"))
-        if xsy is not None:
-            _vec(xsy, self.xk, "xsy")
-        if s.numel() > 0 and s.data_ptr() == grad.data_ptr():
-            raise ValueError("step_: s must not alias grad")
-        out = (C.c_double * 3)()
-        self._call("step_groupl2binf", C.c_int64(self.n), _p(s), _p(xsy), _p(self.xk), _p(self.sj), _p(grad),
-                   C.c_int64(self.ngroups), _p(self._offs), _p(self._lam_g), C.c_double(nu), C.c_double(self.Delta),
-                   out)
-        return s, StepResult(out[0], math.sqrt(out[1]), out[2])
+        return self._lib_step("step_groupl2binf", (C.c_int64(self.n),), s, grad, xsy,
+                              (C.c_int64(self.ngroups), _p(self._offs), _p(self._lam_g), C.c_double(nu),
+                               C.c_double(self.Delta)))
 
 
 # ------------------------------------------------------------------- verbs ---

@@ -289,13 +289,10 @@ def step_l1b2_sharded_(s_local, psi, grad_local, nu, xsy_local=None, group=None)
     """ShiftedNormL1B2 solver step (ShiftedNormL1B2.step_) on a sharded vector: the search's partial sums go through
     one all-reduce per pass, the finish's four sums (ψ's two, Σs², Σ∇f·s) through one more.  Returns
     (s_local, StepResult) with the whole-vector scalars, identical on every rank."""
-    from . import _lib as L, StepResult
+    from . import _lib as L
 
     cb = L.ALLREDUCE_FN(_make_reduce(psi.xk.device, group))
-    out, passes = (C.c_double * 3)(), C.c_int32()
-    psi._call("step_l1b2_sharded", *psi._step_args(s_local, grad_local, nu, xsy_local), cb, None, C.byref(passes), out)
-    psi.last_passes = passes.value
-    return s_local, StepResult(out[0], math.sqrt(out[1]), out[2])
+    return psi._step_l1b2("step_l1b2_sharded", s_local, grad_local, nu, xsy_local, (cb, None))
 
 
 # ----------------------------------------------------- single-vector top-r sharded ---

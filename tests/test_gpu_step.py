@@ -5,11 +5,14 @@ Bars: `s` bit-identical to the stand-alone prox! of the same library AND (for th
 `xsy` bit-identical to (xk + sj) + s; the three scalars against the oracle's composition -- ψ(s) to 1e-12 / 1e-5
 relative (Float64 / Float32: λ·Σ is rounded to R), the Float64 sums to 1e-12 relative to Σ|terms|.
 """
+import ctypes as C
+
 import numpy as np
 import pytest
 import torch
 
 from gpu_util import DEV, N, T, bounds, inputs, orc, sp
+from shiftedprox import _lib as L
 
 pytestmark = pytest.mark.gpu
 
@@ -140,6 +143,19 @@ def test_step_in_place(dt):
     _, res = sp.step_(tg, psi, tg, 0.25, xsy=txk)
     assert np.array_equal(N(tg), rs) and np.array_equal(N(txk), rxsy)
     assert res.psi == pytest.approx(rpsi, rel=1e-5) and res.snorm == pytest.approx(rsn) and res.gdots == pytest.approx(rgd)
+    # an output overlapping an input partially would land on other elements' operands, which another CTA reads
+    # before or after the store: refused, through the Python API and the raw ABI alike
+    buf = T(np.concatenate([grad, grad]))
+    with pytest.raises(ValueError):
+        sp.step_(buf[1:n + 1], psi, buf[:n], 0.25)
+    with pytest.raises(ValueError):
+        sp.step_(torch.empty_like(tg), psi, buf[:n], 0.25, xsy=buf[1:n + 1])
+    f = getattr(L.lib(), f"spx_step_sep_{'f64' if dt == np.float64 else 'f32'}")
+    f.restype = C.c_int32
+    st = f(sp.context(DEV), C.c_int32(L.H_L0), C.c_int64(n), C.c_void_p(buf[1:].data_ptr()), None,
+           C.c_void_p(buf[n:].data_ptr()), None, C.c_void_p(buf.data_ptr()), C.c_double(0.9), C.c_double(0.25),
+           (C.c_double * 3)())
+    assert st == L.SPX_E_INVALID
 
 
 # ---- the step around a prox! that is not one streaming pass (spx_step_pre_*, the type's prox! in place, spx_step_post_*)
@@ -192,24 +208,34 @@ def test_step_composed_types(dt, kind):
     ref_psi = oracle_value(gs)
     scalars_close(res, ref_psi, float(np.sqrt(np.sum(s64 * s64))), float(np.sum(g64 * s64)), grad, gs, dt)
     assert res.psi == pytest.approx(psi(s), rel=1e-12 if dt == np.float64 else 1e-6, abs=1e-300)
-    # xsy is optional; s must not be the gradient itself
+    # xsy is optional; s must not overlap the gradient, and no output may overlap an input partially
     s2 = torch.empty_like(s)
     _, res2 = sp.step_(s2, psi, T(grad), nu)
     assert torch.equal(s2, s) and tuple(res2) == tuple(res)
     tg = T(grad)
     with pytest.raises(ValueError):
         sp.step_(tg, psi, tg, nu)
+    buf = T(np.concatenate([grad, grad]))
+    with pytest.raises(ValueError):
+        sp.step_(buf[1:n + 1], psi, buf[:n], nu)
+    with pytest.raises(ValueError):
+        sp.step_(s2, psi, buf[:n], nu, xsy=buf[1:n + 1])
+    if kind != "l1b2":  # the composed form writes q into s before prox! reads xk
+        with pytest.raises(ValueError):
+            sp.step_(psi.xk, psi, tg, nu)
+    # x <- x + s: xsy may be ψ's own xk
+    sp.step_(s2, psi, tg, nu, xsy=psi.xk)
+    assert np.array_equal(N(psi.xk), ((xk + sj) + N(s2)).astype(dt))
 
 
 @pytest.mark.parametrize("dt", DT)
 @pytest.mark.parametrize("layout", ["g64", "short_ragged"])
 def test_step_groupl2_single_pass_on_short_group_layouts(dt, layout):
     """ShiftedGroupNormL2 with every group <= 256 elements (the C4 shape): spx_step_groupl2_* runs the whole step in the
-    one pass of the packed warp rounds.  Same bars as above, the composed form of the same call (SPX_STEP_COMPOSED)
-    gives the same s bit for bit, and a layout rewritten after validation so that it holds a long group (stale census)
-    is still computed correctly (the kernel flags it and the call is redone the long way)."""
-    import os
-
+    one pass of the packed warp rounds.  Same bars as above, the composed form of the same call
+    (ShiftedProximableFunction.step_) gives the same s bit for bit, and a layout rewritten after validation so that it
+    holds a long group (stale census) is still computed correctly (the kernel flags it and the call is redone the long
+    way)."""
     rng = np.random.default_rng(7)
     sizes = np.full(1500, 64) if layout == "g64" else rng.integers(1, 257, 1500)
     offs = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
@@ -220,9 +246,9 @@ def test_step_groupl2_single_pass_on_short_group_layouts(dt, layout):
     s = torch.empty(n, dtype=T(grad).dtype, device=DEV)
     xsy = torch.empty_like(s)
 
-    def check(offsets):
+    def check(offsets, step=type(psi).step_):
         launches0 = sp.launch_count(DEV) if hasattr(sp, "launch_count") else None
-        _, res = sp.step_(s, psi, T(grad), nu, xsy=xsy)
+        _, res = step(psi, s, T(grad), nu, xsy=xsy)
         q = (dt(-dt(nu)) * grad).astype(dt)
         y = torch.empty_like(s)
         sp.prox_(y, psi, T(q), nu)
@@ -236,11 +262,7 @@ def test_step_groupl2_single_pass_on_short_group_layouts(dt, layout):
 
     res, _ = check(offs)
     s_fused = s.clone()
-    os.environ["SPX_STEP_COMPOSED"] = "1"
-    try:
-        res_c, _ = check(offs)
-    finally:
-        del os.environ["SPX_STEP_COMPOSED"]
+    res_c, _ = check(offs, sp.ShiftedProximableFunction.step_)
     assert torch.equal(s, s_fused)
     assert res_c.psi == pytest.approx(res.psi, rel=1e-12 if dt == np.float64 else 1e-6)
     assert res_c.snorm == pytest.approx(res.snorm, rel=1e-12) and res_c.gdots == pytest.approx(res.gdots, rel=1e-9, abs=1e-9)

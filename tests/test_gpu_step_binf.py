@@ -183,3 +183,10 @@ def test_step_binf_s_must_not_alias_grad():
     tg = T(grad)
     with pytest.raises(ValueError):
         sp.step_(tg, psi, tg, NU)
+    # nor overlap it partially: the composed form would overwrite part of ∇f before spx_step_post reads it, the one
+    # pass another group's ∇f before or after its CTA reads it
+    n = grad.size
+    buf = T(np.concatenate([grad, grad]))
+    for a, b in ((1, 0), (0, 1)):
+        with pytest.raises(ValueError):
+            sp.step_(buf[a:a + n], psi, buf[b:b + n], NU)

@@ -650,10 +650,10 @@ def test_step_groupl2binf_uniform_many_rounds(dt, m):
 @gpu
 @pytest.mark.parametrize("dt", DT)
 @pytest.mark.parametrize("layout", ["g64", "short_ragged"])
-def test_step_groupl2_single_pass_at_scale(dt, layout):
+def test_step_groupl2_single_pass_at_scale_against_base_composed(dt, layout):
     """The one-pass GroupNormL2 step (group_l2_step_kernel) at 2^23 elements: the bars of
-    test_step_groupl2_single_pass_on_short_group_layouts, its composed form (SPX_STEP_COMPOSED) giving the same s, and
-    windows of whole groups against the oracle at 8 ulp of the value scale."""
+    test_step_groupl2_single_pass_on_short_group_layouts, its composed form (ShiftedProximableFunction.step_) giving the
+    same s, and windows of whole groups against the oracle at 8 ulp of the value scale."""
     rng = np.random.default_rng(7)
     sizes = np.full((1 << 23) // 64 + 3, 64) if layout == "g64" else rng.integers(1, 257, (1 << 23) // 128 + 3)
     offs = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
@@ -677,11 +677,7 @@ def test_step_groupl2_single_pass_at_scale(dt, layout):
         _, again = call()
         assert same_scalars(again, res)
     s_fused = s.clone()
-    os.environ["SPX_STEP_COMPOSED"] = "1"
-    try:
-        (_, res_c), nl = launches(call)
-    finally:
-        del os.environ["SPX_STEP_COMPOSED"]
+    (_, res_c), nl = launches(lambda: sp.ShiftedProximableFunction.step_(psi, s, tg, NU_G, xsy=xsy))
     assert nl > 2 and torch.equal(s, s_fused)
     q = (dt(-dt(NU_G)) * grad).astype(dt)
     eps = np.finfo(dt).eps
