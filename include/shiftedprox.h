@@ -384,10 +384,10 @@ typedef struct spx_box_job_f32 {
   /*   spx_step_post:  xsy = (xk + sj) + s (xsy may be NULL), out2_host = {Σ s², Σ grad·s}.                  */ \
   /* sj == NULL: zeros.  spx_step_post synchronises.                                                         */ \
   int32_t spx_step_pre_##SUF(spx_ctx* ctx, int64_t n, R* q, const R* grad, double nu);               \
-  /* ShiftedGroupNormL2 (shiftedGroupNormL2.jl:52-79): ONE pass when every group of a validated layout       */ \
-  /* holds <= 256 elements (spx_group_validate_offsets), the composed form otherwise.  A layout rewritten    */ \
-  /* after validation so that it holds a longer group is redone in the composed form, which re-reads the     */ \
-  /* inputs: with xsy aliasing one of them, validate the layout again after rewriting it.                    */ \
+  /* ShiftedGroupNormL2 (shiftedGroupNormL2.jl:52-79): on every layout, inside the passes of the prox!      */ \
+  /* kernels of its group sizes -- ONE pass per group (two grid-wide passes for a single group spanning the  */ \
+  /* vector), no spx_step_pre / spx_step_post.  A layout rewritten after validation is still computed right: */ \
+  /* only the groups the first kernel left are read again, so xsy may alias xk or sj in that case as well.  */ \
   int32_t spx_step_groupl2_##SUF(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj,    \
                                  const R* grad, int64_t ngroups, const int64_t* offs,                \
                                  const R* lambda_g, double nu, double* out3_host);                   \

@@ -371,6 +371,10 @@ int32_t step_composed(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const 
 template <class R>
 int32_t step_l1b2_finish(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad, const R* mid,
                          R nu, R ls, bool use_scale, R scale, R post, double* v);
+// the scaling pass of the ShiftedGroupNormL2 step on one group spanning the vector (spx_step.cu, called by spx_group.cu)
+template <class R>
+int32_t step_group_scale(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad, R nu, R alpha,
+                         bool zero, double* v);
 // spx_comm.cu: is the context in "scalars are global" mode; all-reduce ctx->d_result[0..nslot) on ctx->stream
 bool comm_active(const spx_ctx* ctx);
 int32_t comm_neutral_result(spx_ctx* ctx, int nslot);

@@ -192,9 +192,14 @@ template <class R, bool KEEP_XS> struct Tile {
 // shiftedGroupNormL2.jl:52-79
 // Loads are batched four iterations deep before anything is stored: y may alias q, so the compiler
 // cannot hoist them itself, and a warp that owns a long group is alone in hiding its latency.
-template <class R, bool PSI, bool SHIFTED>
+// STEP (the solver step, spx_step_groupl2): y = s, q = ∇f read as q = (-ν)∇f rounded to R (mnu = -ν); the second loop
+// re-reads ∇f beside the stash, also writes xsy = (xk + sj) + s (when given) and adds Σ s² and Σ ∇f·s of the lane's
+// elements to ss2 and dot.  s overlaps none of xk, sj, ∇f (the alias rule of the group steps), so stashing sol in s is
+// safe; xsy may be xk or sj: every element is read before the same lane writes it.
+template <class R, bool PSI, bool SHIFTED, bool STEP = false>
 __device__ __forceinline__ double l2_long_group(R* y, const R* xk, const R* sj, const R* q, long long b, long long e,
-                                                R lam, R sigma, int lane) {
+                                                R lam, R sigma, int lane, R* xsy = nullptr, R mnu = R(0),
+                                                double* ss2 = nullptr, double* dot = nullptr) {
   double ss = 0.0;
   for (long long i0 = b + lane; i0 < e; i0 += 128) {
     R xv[4], sv[4], qv[4];
@@ -211,6 +216,7 @@ __device__ __forceinline__ double l2_long_group(R* y, const R* xk, const R* sj, 
     for (int u = 0; u < 4; ++u) {
       const long long i = i0 + 32 * u;
       if (i < e) {
+        if constexpr (STEP) qv[u] = mnu * qv[u];  // q = -ν ∇f
         const R s = (qv[u] + xv[u]) + sv[u];
         y[i] = s;  // stash sol (each lane re-reads only what it wrote)
         ss += (double)s * (double)s;
@@ -222,7 +228,7 @@ __device__ __forceinline__ double l2_long_group(R* y, const R* xk, const R* sj, 
   const R alpha = jl_max(R(1) - sigma * lam / snorm, R(0));
   double vv = 0.0;
   for (long long i0 = b + lane; i0 < e; i0 += 128) {
-    R xv[4], sv[4], yv[4];
+    R xv[4], sv[4], yv[4], gv[STEP ? 4 : 1];
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
       const long long i = i0 + 32 * u;
@@ -230,6 +236,7 @@ __device__ __forceinline__ double l2_long_group(R* y, const R* xk, const R* sj, 
         xv[u] = SHIFTED ? xk[i] : R(0);
         sv[u] = SHIFTED ? sj[i] : R(0);
         yv[u] = y[i];
+        if constexpr (STEP) gv[u] = q[i];
       }
     }
 #pragma unroll
@@ -239,7 +246,13 @@ __device__ __forceinline__ double l2_long_group(R* y, const R* xk, const R* sj, 
         const R xsi = xv[u] + sv[u];
         const R o = (snorm == R(0) ? R(0) : alpha * yv[u]) - xsi;
         stv(y + i, o);
-        if (PSI) {
+        if constexpr (STEP) {
+          const R v = xsi + o;  // ψ's own argument (ShiftedProximalOperators.jl:52)
+          if (xsy != nullptr) stv(xsy + i, v);
+          vv += (double)v * (double)v;
+          *ss2 = __fma_rn((double)o, (double)o, *ss2);
+          *dot = __fma_rn((double)gv[u], (double)o, *dot);
+        } else if (PSI) {
           const double v = (double)(xsi + o);
           vv += v * v;
         }
@@ -252,16 +265,19 @@ __device__ __forceinline__ double l2_long_group(R* y, const R* xk, const R* sj, 
 }
 
 // PART 0: groups of <= 256 elements, 1: the longer ones; SHIFTED = false: xk == sj == NULL
-template <class R, bool PSI, int PART, bool SHIFTED>
+// STEP (PART 1 only, PSI and SHIFTED): the long groups of the solver step (l2_long_group), q = ∇f; slot 0 is
+// partials[blockIdx.x] = {ψ, Σ s², -1}, slot 1 part1[blockIdx.x] = {Σ ∇f·s, 0, -1}
+template <class R, bool PSI, int PART, bool SHIFTED, bool STEP = false>
 __global__ void __launch_bounds__(kGroupThreads)
     group_l2_kernel(R* y, const R* xk, const R* sj, const R* q, long long ngroups,
                     const long long* __restrict__ offs, const R* __restrict__ lambda_g, R sigma, unsigned classes,
-                    Partial* __restrict__ partials) {
+                    Partial* __restrict__ partials, R* xsy, R mnu, Partial* __restrict__ part1) {
+  static_assert(!STEP || (PSI && PART == 1 && SHIFTED), "the step form takes the shifted long groups");
   const int lane = threadIdx.x & 31;
   const long long warp = ((long long)blockIdx.x * kGroupThreads + threadIdx.x) >> 5;
   const long long nwarps = ((long long)gridDim.x * kGroupThreads) >> 5;
   const long long ntasks = (ngroups + kTask - 1) / kTask;
-  double psi = 0.0;
+  double psi = 0.0, ss2 = 0.0, dot = 0.0;
   for (long long task = warp; task < ntasks; task += nwarps) {
     const long long g0 = task * kTask;
     const TaskHead th = load_task(offs, g0, ngroups, lane);
@@ -276,7 +292,8 @@ __global__ void __launch_bounds__(kGroupThreads)
           const long long b = __shfl_sync(0xffffffffu, th.lo, pos), e = __shfl_sync(0xffffffffu, th.hi, pos);
           if (!in_launched_class(e - b, classes)) {
             const R lam = __shfl_sync(0xffffffffu, lam_lane, pos);
-            const double vv = l2_long_group<R, PSI, SHIFTED>(y, xk, sj, q, b, e, lam, sigma, lane);
+            const double vv =
+                l2_long_group<R, PSI, SHIFTED, STEP>(y, xk, sj, q, b, e, lam, sigma, lane, xsy, mnu, &ss2, &dot);
             if (PSI && lane == 0) psi += (double)(lam * (R)sqrt(vv));  // λ_g ‖v_g‖  groupNormL2.jl:36
           }
         }
@@ -317,7 +334,15 @@ __global__ void __launch_bounds__(kGroupThreads)
       pos += 32 >> k;
     }
   }
-  if (PSI) {
+  if constexpr (STEP) {
+    Partial p{psi, ss2, -1}, p2{dot, 0.0, -1};
+    p = block_fold<kGroupThreads>(p);
+    p2 = block_fold<kGroupThreads>(p2);
+    if (threadIdx.x == 0) {
+      partials[blockIdx.x] = p;
+      part1[blockIdx.x] = p2;
+    }
+  } else if (PSI) {
     Partial p;
     p.s = psi;
     p.s2 = 0.0;
@@ -461,10 +486,15 @@ template <class R, int NP, int PLS, int ST> struct StageRing {
 // barrier of the first block sum) thread 0 refills the buffer with [nb, ne), the group ST places further down the list,
 // so that group's HBM latency is spent under the work on the ST - 1 groups in between (ST = 1: under this group's
 // scaling and stores).
-template <class R, bool PSI, bool SHIFTED, int E, int T, int PLS, class Ring>
+// STEP (the solver step): the q plane holds ∇f and q = (-ν)∇f is rounded to R as it is read (mnu = -ν); the store loop
+// also writes xsy = (xk + sj) + s (when given) and adds Σ s² and Σ ∇f·s of the thread's elements to ss2 and dot.  The
+// store loop reads ∇f from the stage again, so the buffer is refilled only after the block sum of ψ (∇f held in
+// registers, or re-read from global memory, needs more registers still).
+template <class R, bool PSI, bool SHIFTED, int E, int T, int PLS, bool STEP = false, class Ring>
 __device__ __forceinline__ double l2_big_group(R* y, const R* xk, const R* sj, const R* q, long long b, long long e, R lam,
                                                R sigma, double* red, const R* stage, Ring& ring, long long nb,
-                                               long long ne) {
+                                               long long ne, R* xsy = nullptr, R mnu = R(0), double* ss2 = nullptr,
+                                               double* dot = nullptr) {
   const int t = threadIdx.x;
   R sol[E], xs[E];
   double ss = 0.0;
@@ -477,41 +507,64 @@ __device__ __forceinline__ double l2_big_group(R* y, const R* xk, const R* sj, c
     sol[k] = R(0);
     xs[k] = R(0);
     if (i < e) {
-      const R xi = SHIFTED ? px[k * T] : R(0), si = SHIFTED ? pj[k * T] : R(0), qi = pq[k * T];
+      const R xi = SHIFTED ? px[k * T] : R(0), si = SHIFTED ? pj[k * T] : R(0);
+      const R qi = STEP ? mnu * pq[k * T] : pq[k * T];  // STEP: q = -ν ∇f
       sol[k] = (qi + xi) + si;  // shiftedGroupNormL2.jl:65
       xs[k] = xi + si;
       ss += (double)sol[k] * (double)sol[k];
     }
   }
   ss = block_sum<T>(ss, red);
-  if (t == 0 && ne > nb) ring.refill(q, xk, sj, nb, ne);
+  if (!STEP && t == 0 && ne > nb) ring.refill(q, xk, sj, nb, ne);
   const R snorm = (R)sqrt(ss);
   const R alpha = jl_max(R(1) - sigma * lam / snorm, R(0));
   double vv = 0.0;
+  if constexpr (STEP) {
 #pragma unroll
-  for (int k = 0; k < E; ++k) {
-    const long long i = b + (long long)k * T + t;
-    if (i < e) {
-      const R o = (snorm == R(0) ? R(0) : alpha * sol[k]) - xs[k];  // :70-77
-      stv(y + i, o);
-      if (PSI) {
-        const double v = (double)(xs[k] + o);
-        vv += v * v;
+    for (int k = 0; k < E; ++k) {
+      const long long i = b + (long long)k * T + t;
+      if (i < e) {
+        const R gk = pq[k * T];
+        const R o = (snorm == R(0) ? R(0) : alpha * sol[k]) - xs[k];  // :70-77
+        stv(y + i, o);
+        const R v = xs[k] + o;  // ψ's own argument (ShiftedProximalOperators.jl:52)
+        if (xsy != nullptr) stv(xsy + i, v);
+        vv += (double)v * (double)v;
+        *ss2 = __fma_rn((double)o, (double)o, *ss2);
+        *dot = __fma_rn((double)gk, (double)o, *dot);
+      }
+    }
+  } else {
+#pragma unroll
+    for (int k = 0; k < E; ++k) {
+      const long long i = b + (long long)k * T + t;
+      if (i < e) {
+        const R o = (snorm == R(0) ? R(0) : alpha * sol[k]) - xs[k];  // :70-77
+        stv(y + i, o);
+        if (PSI) {
+          const double v = (double)(xs[k] + o);
+          vv += v * v;
+        }
       }
     }
   }
   if (!PSI) return 0.0;
   vv = block_sum<T>(vv, red);
+  if (STEP && t == 0 && ne > nb) ring.refill(q, xk, sj, nb, ne);  // every thread has read its ∇f from the stage
   // shifted: λ_g ‖(xk + sj + y)_g‖; unshifted: λ_g ‖x_g‖ of the input (groupNormL2.jl:49-54)
   return (double)(lam * (SHIFTED ? (R)sqrt(vv) : snorm));
 }
 
 // T threads per group of LO < m <= EB T elements (EA per thread up to EA T elements, EB above); ST staging buffers
-template <class R, bool PSI, bool SHIFTED, int T, int LO, int EA, int EB, int ST>
-__global__ void __launch_bounds__(T, (sizeof(R) == 4 ? 3 : 2) * 256 / T)
+// STEP (PSI and SHIFTED): the solver step, q = ∇f (see l2_big_group); slot 0 is partials[blockIdx.x] = {ψ, Σ s², -1},
+// slot 1 part1[blockIdx.x] = {Σ ∇f·s, 0, -1}.  With 256 threads the STEP form runs one CTA per SM fewer than the prox!
+// form (Float32 3 -> 2, Float64 2 -> 1), the occupancy at which it does not spill.
+template <class R, bool PSI, bool SHIFTED, int T, int LO, int EA, int EB, int ST, bool STEP = false>
+__global__ void __launch_bounds__(T, (sizeof(R) == 4 ? 3 : 2) * 256 / T - (STEP && T == 256 ? 1 : 0))
     group_l2_big_kernel(R* y, const R* xk, const R* sj, const R* q, long long ngroups,
                         const long long* __restrict__ offs, const R* __restrict__ lambda_g, R sigma,
-                        Partial* __restrict__ partials) {
+                        Partial* __restrict__ partials, R* xsy, R mnu, Partial* __restrict__ part1) {
+  static_assert(!STEP || (PSI && SHIFTED), "the step form is the shifted one with ψ");
   constexpr int PLS = bulk_plane<R>(EB * T), NP = SHIFTED ? 3 : 1;
   __shared__ int list[T];
   __shared__ int wcount[T / 32];
@@ -520,7 +573,7 @@ __global__ void __launch_bounds__(T, (sizeof(R) == 4 ? 3 : 2) * 256 / T)
   extern __shared__ __align__(128) unsigned char l2_stage_raw[];
   const int t = threadIdx.x;
   StageRing<R, NP, PLS, ST> ring(bar, reinterpret_cast<R*>(l2_stage_raw));  // q | xk | sj
-  double psi = 0.0;
+  double psi = 0.0, ss2 = 0.0, dot = 0.0;
   for (long long g0 = (long long)blockIdx.x * T; g0 < ngroups; g0 += (long long)gridDim.x * T) {
     const int nbig = list_class_groups<T, LO, EB * T>(offs, g0, ngroups, list, wcount);
     ring.prime(list, nbig, g0, offs, q, xk, sj);
@@ -533,13 +586,23 @@ __global__ void __launch_bounds__(T, (sizeof(R) == 4 ? 3 : 2) * 256 / T)
       const R* const stage = ring.wait(j);
       double term;
       if (e - b <= EA * T)
-        term = l2_big_group<R, PSI, SHIFTED, EA, T, PLS>(y, xk, sj, q, b, e, lam, sigma, red, stage, ring, nb, ne);
+        term = l2_big_group<R, PSI, SHIFTED, EA, T, PLS, STEP>(y, xk, sj, q, b, e, lam, sigma, red, stage, ring, nb, ne,
+                                                               xsy, mnu, &ss2, &dot);
       else
-        term = l2_big_group<R, PSI, SHIFTED, EB, T, PLS>(y, xk, sj, q, b, e, lam, sigma, red, stage, ring, nb, ne);
+        term = l2_big_group<R, PSI, SHIFTED, EB, T, PLS, STEP>(y, xk, sj, q, b, e, lam, sigma, red, stage, ring, nb, ne,
+                                                               xsy, mnu, &ss2, &dot);
       if (PSI && t == 0) psi += term;
     }
   }
-  if (PSI && t == 0) {
+  if constexpr (STEP) {
+    Partial p{t == 0 ? psi : 0.0, ss2, -1}, p2{dot, 0.0, -1};
+    p = block_fold<T>(p);
+    p2 = block_fold<T>(p2);
+    if (t == 0) {
+      partials[blockIdx.x] = p;
+      part1[blockIdx.x] = p2;
+    }
+  } else if (PSI && t == 0) {
     Partial p;
     p.s = psi;
     p.s2 = 0.0;
@@ -1995,24 +2058,13 @@ template <class R> struct SolSumSq {
     return R(0);
   }
 };
-template <class R, bool PSI> struct SolScale {
-  using Real = R;
-  static constexpr int NIN = 3, UNROLL = 2;
-  static constexpr bool OUT = true, ACC = PSI;
-  const R* in[NIN];  // xk, sj, q
-  R fill[NIN];
-  R* y;
-  R alpha;
-  bool zero;
-  __device__ __forceinline__ R apply(const R (&x)[NIN], long long, Partial& acc) const {
-    const R sol = (x[2] + x[0]) + x[1];
-    const R xs = x[0] + x[1];
-    const R o = (zero ? R(0) : alpha * sol) - xs;
-    if (PSI) {
-      const double v = (double)(xs + o);
-      acc.s2 += v * v;
-    }
-    return o;
+// the same pass in the solver step: in[2] is ∇f and q = (-ν)∇f is rounded to R as it is read (same grid, same order)
+template <class R> struct SolSumSqGrad : SolSumSq<R> {
+  R mnu;
+  __device__ __forceinline__ R apply(const R (&x)[3], long long, Partial& acc) const {
+    const double s = (double)((mnu * x[2] + x[0]) + x[1]);
+    acc.s2 += s * s;
+    return R(0);
   }
 };
 template <class R> struct VSumSq {
@@ -2228,15 +2280,16 @@ static int32_t launch_group_l2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const
     if (st == SPX_OK && (classes & 1u)) st = big_grid(ctx, ngroups, (const void*)mid_psi, kMidT, mid_bytes, &grid3);
     if (st != SPX_OK) return st;
     group_l2_kernel<R, true, 0, SHIFTED><<<grid0, kGroupThreads, 0, ctx->stream>>>(
-        y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma, classes, ctx->d_partials);
+        y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma, classes, ctx->d_partials, nullptr, R(0), nullptr);
     group_l2_kernel<R, true, 1, SHIFTED><<<grid1, kGroupThreads, 0, ctx->stream>>>(
-        y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma, classes, ctx->d_partials + grid0);
+        y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma, classes, ctx->d_partials + grid0, nullptr, R(0),
+        nullptr);
     if (grid2 > 0)
       big_psi<<<grid2, kGroupThreads, big_bytes, ctx->stream>>>(y, xk, sj, q, ngroups, (const long long*)offs, lambda_g,
-                                                               sigma, ctx->d_partials + grid0 + grid1);
+                                                               sigma, ctx->d_partials + grid0 + grid1, nullptr, R(0), nullptr);
     if (grid3 > 0)
       mid_psi<<<grid3, kMidT, mid_bytes, ctx->stream>>>(y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma,
-                                                       ctx->d_partials + grid0 + grid1 + grid2);
+                                                       ctx->d_partials + grid0 + grid1 + grid2, nullptr, R(0), nullptr);
     ctx->launches += 2 + (grid2 > 0) + (grid3 > 0);
     SPX_CUDA(cudaGetLastError());
     st = finalize_partials(ctx, grid0 + grid1 + grid2 + grid3, 1, false);
@@ -2262,20 +2315,20 @@ static int32_t launch_group_l2(spx_ctx* ctx, int64_t n, R* y, const R* xk, const
   if (st != SPX_OK) return st;
   if (grid2 > 0) {
     big_run<<<grid2, kGroupThreads, big_bytes, ctx->stream>>>(y, xk, sj, q, ngroups, (const long long*)offs, lambda_g,
-                                                             sigma, ctx->d_partials);
+                                                             sigma, ctx->d_partials, nullptr, R(0), nullptr);
     ctx->launches++;
   }
   if (grid3 > 0) {
     mid_run<<<grid3, kMidT, mid_bytes, ctx->pipe_streams[0]>>>(y, xk, sj, q, ngroups, (const long long*)offs, lambda_g,
-                                                              sigma, ctx->d_partials);
+                                                              sigma, ctx->d_partials, nullptr, R(0), nullptr);
     ctx->launches++;
   }
   // groups above 4096 elements (and those of a class not launched): the warp path, whose CTAs exit at once when there
   // are none -- on the side stream, under the short-group kernel
   group_l2_kernel<R, false, 1, SHIFTED><<<grid0, kGroupThreads, 0, ctx->pipe_streams[1]>>>(
-      y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma, classes, ctx->d_partials);
+      y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma, classes, ctx->d_partials, nullptr, R(0), nullptr);
   group_l2_kernel<R, false, 0, SHIFTED><<<grid0, kGroupThreads, 0, classes == 0u ? ctx->stream : ctx->pipe_streams[1]>>>(
-      y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma, classes, ctx->d_partials);
+      y, xk, sj, q, ngroups, (const long long*)offs, lambda_g, sigma, classes, ctx->d_partials, nullptr, R(0), nullptr);
   ctx->launches += 2;
   SPX_CUDA(cudaGetLastError());
   return join_side_streams(ctx);
@@ -2499,13 +2552,15 @@ static int32_t prox_group(spx_ctx* ctx, bool binf, int64_t n, R* y, const R* xk,
 
 // ---- the solver step of ShiftedGroupNormL2 (SURVEY.md 8f rank 1; spx_step.cu for the separable types) ---------------
 //     q = (-ν) ∇f;  prox!(s, ψ, q, ν);  xsy = (xk + sj) + s;  ψ(s);  Σ s²;  Σ ∇f·s
-// Layouts whose groups all hold <= 256 elements (the C4 shape: the census of spx_group_validate_offsets says so) run it
-// in the ONE pass of the packed warp rounds: ∇f takes the place of q on the load (q = (-ν)∇f rounded to R, as the
-// caller's broadcast would), the store loop also writes xsy and folds the two sums next to the ψ term.  s is bit for
-// bit what prox! writes.  A group longer than that (a stale census) raises the flag and the call is redone in the
-// composed form; every other layout takes the composed form at once: spx_step_pre, prox! in place, spx_step_post.
-// two CTAs per SM (125 registers in Float64: sol, ∇f and xk + sj of 8 elements per lane); three spill and measure the
-// same (2.60 vs 2.54 ms at 2^28 Float64)
+// Every layout runs it in the passes of the prox! kernels of its group sizes, with ∇f in place of q on the load (q =
+// (-ν)∇f rounded to R, as the caller's broadcast would) and a store loop that also writes xsy and folds the two sums next
+// to the ψ term: s is bit for bit what prox! writes.  Groups of <= 256 elements take the packed warp rounds of
+// group_l2_step_kernel (on a validated layout without longer groups, the C4 shape, alone: one launch and the fold), the
+// CTA-per-group classes the step forms of group_l2_big_kernel, longer groups the step form of the warp path
+// (group_l2_kernel<…, PART 1>), and a single group spanning the vector the two grid-wide passes of prox_single_group.
+// group_l2_step_kernel: two CTAs per SM (125 registers in Float64: sol, ∇f and xk + sj of 8 elements per lane); three
+// spill and measure the same (2.60 vs 2.54 ms at 2^28 Float64).  long_runs: the long-group kernels run in the same call,
+// so a group of more than 256 elements is theirs; without them such a group (a stale census) raises the flag.
 #ifndef SPX_GSTEP_MINB
 #define SPX_GSTEP_MINB 2
 #endif
@@ -2513,7 +2568,7 @@ template <class R>
 __global__ void __launch_bounds__(kGroupThreads, SPX_GSTEP_MINB)
     group_l2_step_kernel(R* s, R* xsy, const R* xk, const R* sj, const R* grad, long long ngroups,
                          const long long* __restrict__ offs, const R* __restrict__ lambda_g, R sigma, R mnu,
-                         Partial* __restrict__ partials) {
+                         Partial* __restrict__ partials, Partial* __restrict__ part1, bool long_runs) {
   const int lane = threadIdx.x & 31;
   const long long warp = ((long long)blockIdx.x * kGroupThreads + threadIdx.x) >> 5;
   const long long nwarps = ((long long)gridDim.x * kGroupThreads) >> 5;
@@ -2527,8 +2582,8 @@ __global__ void __launch_bounds__(kGroupThreads, SPX_GSTEP_MINB)
     int pos = 0;
     while (pos < th.cnt) {
       const int k = plan_round(th.le, pos);
-      if (k < 0) {  // a group of more than 256 elements: not this kernel's (the host redoes the call)
-        bad = 1;
+      if (k < 0) {  // a group of more than 256 elements: the long-group kernels' (flagged when they do not run)
+        if (!long_runs) bad = 1;
         pos += 1;
         continue;
       }
@@ -2589,8 +2644,107 @@ __global__ void __launch_bounds__(kGroupThreads, SPX_GSTEP_MINB)
   p2 = block_fold<kGroupThreads>(p2);
   if (threadIdx.x == 0) {
     partials[blockIdx.x] = p;
-    partials[gridDim.x + blockIdx.x] = p2;
+    part1[blockIdx.x] = p2;
   }
+}
+
+// The step kernels of every group above 256 elements -- the CTA-per-group classes in `classes` and the warp kernel for
+// the others -- and, with `short_groups`, group_l2_step_kernel for the rest, on persistent grids capped so that their
+// CTAs together stay within kMaxPartials.  Kernel k writes slot 0 at d_partials + base_k and slot 1 at d_partials +
+// total + base_k, so finalize_partials(ctx, total, 2) folds them in a fixed order: two identical calls give identical
+// sums.  With a class present the kernels run on the context's side streams, as the plain prox! does (ragged 1..4096 on
+// a B200: 2.72 against 2.97 ms at 2^28 Float64 with every kernel on ctx->stream, 3.20 against 3.37 ms at 2^29 Float32).
+template <class R>
+static int32_t launch_step_groupl2(spx_ctx* ctx, bool short_groups, unsigned classes, R* s, R* xsy, const R* xk,
+                                   const R* sj, const R* grad, int64_t ngroups, const int64_t* offs, const R* lambda_g,
+                                   R nu, int* total) {
+  constexpr int kMidT = 128, kMidStages = SPX_L2_MID_STAGES, kCap = kMaxPartials / 4;
+  const size_t big_bytes = 3 * (size_t)bulk_plane<R>((int)kBigMax) * sizeof(R);
+  const size_t mid_bytes = kMidStages * 3 * (size_t)bulk_plane<R>((int)kBigMin) * sizeof(R);
+  auto big = group_l2_big_kernel<R, true, true, kGroupThreads, (int)kBigMin, kBigE / 2, kBigE, 1, true>;
+  auto mid = group_l2_big_kernel<R, true, true, kMidT, (int)kMidMin, 4, 8, kMidStages, true>;
+  auto lng = group_l2_kernel<R, true, 1, true, true>;
+  int gs = 0, gl = 0, gb = 0, gm = 0;
+  int32_t st = SPX_OK;
+  if (short_groups)
+    st = grid_for(ctx, (const void*)group_l2_step_kernel<R>, kGroupThreads, 0, warp_kernel_ctas(ngroups), kCap, true, &gs);
+  if (st == SPX_OK) st = grid_for(ctx, (const void*)lng, kGroupThreads, 0, warp_kernel_ctas(ngroups), kCap, true, &gl);
+  if (st == SPX_OK && (classes & 2u))
+    st = grid_for(ctx, (const void*)big, kGroupThreads, big_bytes, (ngroups + kGroupThreads - 1) / kGroupThreads, kCap,
+                  true, &gb);
+  if (st == SPX_OK && (classes & 1u))
+    st = grid_for(ctx, (const void*)mid, kMidT, mid_bytes, (ngroups + kMidT - 1) / kMidT, kCap, true, &gm);
+  if (st != SPX_OK) return st;
+  const int n_all = gs + gl + gb + gm;
+  Partial* const p0 = ctx->d_partials;
+  Partial* const p1 = ctx->d_partials + n_all;
+  const long long* const o = (const long long*)offs;
+  cudaStream_t s_big = ctx->stream, s_mid = ctx->stream, s_warp = ctx->stream;
+  if (classes != 0u) {
+    st = fork_side_streams(ctx);
+    if (st != SPX_OK) return st;
+    s_mid = ctx->pipe_streams[0];
+    s_warp = ctx->pipe_streams[1];
+  }
+  // the class (1024, 4096] first: it is the long pole of a ragged layout
+  if (gb > 0) big<<<gb, kGroupThreads, big_bytes, s_big>>>(s, xk, sj, grad, ngroups, o, lambda_g, nu, p0, xsy, -nu, p1);
+  if (gm > 0)
+    mid<<<gm, kMidT, mid_bytes, s_mid>>>(s, xk, sj, grad, ngroups, o, lambda_g, nu, p0 + gb, xsy, -nu, p1 + gb);
+  lng<<<gl, kGroupThreads, 0, s_warp>>>(s, xk, sj, grad, ngroups, o, lambda_g, nu, classes, p0 + gb + gm, xsy, -nu,
+                                        p1 + gb + gm);
+  if (gs > 0)
+    group_l2_step_kernel<R><<<gs, kGroupThreads, 0, s_warp>>>(s, xsy, xk, sj, grad, ngroups, o, lambda_g, nu, -nu,
+                                                               p0 + gb + gm + gl, p1 + gb + gm + gl, true);
+  SPX_CUDA(cudaGetLastError());
+  ctx->launches += 1 + (gs > 0) + (gb > 0) + (gm > 0);
+  *total = n_all;
+  if (classes != 0u) return join_side_streams(ctx);
+  return SPX_OK;
+}
+
+// The norm pass of prox_single_group with q formed from ∇f on the load, on the grid ew_launch gives SolSumSq over the
+// same operands (not its own: the instances' register counts, and with them the resident CTAs, may differ), so the
+// norm is summed in prox!'s order and s is bit for bit prox!'s
+template <class R> static int32_t sol_sumsq_grad_launch(spx_ctx* ctx, const SolSumSqGrad<R>& op, int64_t n, int* nb) {
+  constexpr int VECW = 16 / (int)sizeof(R), UNROLL = SolSumSq<R>::UNROLL;
+  const bool vec = aligned16(op);
+  const long long nvec = vec ? n / VECW : n, tile = (long long)kEwThreads * UNROLL;
+  const long long want = std::max(1LL, (nvec + tile - 1) / tile);
+  const int per_sm = vec ? ew_blocks_per_sm<VECW, UNROLL, SolSumSq<R>>() : ew_blocks_per_sm<1, UNROLL, SolSumSq<R>>();
+  *nb = (int)std::min(want, std::min((long long)ctx->sm_count * per_sm, (long long)kMaxPartials));
+  if (vec)
+    ew_kernel<VECW, UNROLL, SolSumSqGrad<R>><<<*nb, kEwThreads, 0, ctx->stream>>>(op, n, 0, ctx->d_partials);
+  else
+    ew_kernel<1, UNROLL, SolSumSqGrad<R>><<<*nb, kEwThreads, 0, ctx->stream>>>(op, n, 0, ctx->d_partials);
+  ctx->launches++;
+  SPX_CUDA(cudaGetLastError());
+  return SPX_OK;
+}
+
+// one group spanning the vector: that norm pass, then the scaling pass on step_kernel with xsy and the sums
+template <class R>
+static int32_t step_single_group(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad,
+                                 const R* lambda_g, R nu, double* out3) {
+  R lam;
+  SPX_CUDA(cudaMemcpyAsync(&lam, lambda_g, sizeof(R), cudaMemcpyDeviceToHost, ctx->stream));
+  SolSumSqGrad<R> ss;
+  set_in3(ss, xk, sj, grad);
+  ss.mnu = -nu;
+  int nb = 0;
+  int32_t st = sol_sumsq_grad_launch(ctx, ss, n, &nb);
+  if (st != SPX_OK) return st;
+  st = finalize_partials(ctx, nb, 1, false);  // synchronises: lam has arrived as well
+  if (st != SPX_OK) return st;
+  const R snorm = (R)std::sqrt(ctx->h_result[0].s2);
+  R alpha = R(1) - nu * lam / snorm;  // shiftedGroupNormL2.jl:70-77
+  alpha = (alpha != alpha) ? alpha : (alpha > R(0) ? alpha : R(0));
+  double v[3];
+  st = step_group_scale<R>(ctx, n, s, xsy, xk, sj, grad, nu, alpha, snorm == R(0), v);
+  if (st != SPX_OK) return st;
+  out3[0] = (double)(R)(double)(lam * (R)std::sqrt(v[0]));
+  out3[1] = v[2];
+  out3[2] = v[1];
+  return SPX_OK;
 }
 
 template <class R>
@@ -2601,29 +2755,50 @@ static int32_t step_groupl2(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, 
   SPX_REQUIRE(ngroups == 0 || n == 0 || (sj && offs && lambda_g), "null device vector");
   out3[0] = out3[1] = out3[2] = 0.0;
   if (ngroups == 0 || n == 0) return SPX_OK;
+  if (ngroups == 1 && n >= kSingleGroupMin) return step_single_group<R>(ctx, n, s, xsy, xk, sj, grad, lambda_g, (R)nu, out3);
   const spx_ctx::GroupCensus* census = find_census(ctx, offs, ngroups, n);
-  // a validated layout whose groups all have <= 256 elements (the packed warp rounds hold every group)
-  if (ngroups > 1 && census && census->classes == 0u) {
+  int32_t st = SPX_OK;
+  if (census && census->classes == 0u) {
+    // a validated layout whose groups all have <= 256 elements (the packed warp rounds hold every group)
     int grid = 0;
-    int32_t st = grid_for(ctx, (const void*)group_l2_step_kernel<R>, kGroupThreads, 0, warp_kernel_ctas(ngroups),
-                          kMaxPartials / 2, true, &grid);
+    st = grid_for(ctx, (const void*)group_l2_step_kernel<R>, kGroupThreads, 0, warp_kernel_ctas(ngroups),
+                  kMaxPartials / 2, true, &grid);
     if (st != SPX_OK) return st;
     group_l2_step_kernel<R><<<grid, kGroupThreads, 0, ctx->stream>>>(s, xsy, xk, sj, grad, ngroups, (const long long*)offs,
-                                                                    lambda_g, (R)nu, -(R)nu, ctx->d_partials);
+                                                                    lambda_g, (R)nu, -(R)nu, ctx->d_partials,
+                                                                    ctx->d_partials + grid, false);
     ctx->launches++;
     SPX_CUDA(cudaGetLastError());
     st = finalize_partials(ctx, grid, 2, false);
     if (st != SPX_OK) return st;
-    if (ctx->h_result[0].bad <= 0) {
-      out3[0] = (double)(R)ctx->h_result[0].s;
-      out3[1] = ctx->h_result[0].s2;
-      out3[2] = ctx->h_result[1].s;
-      return SPX_OK;
-    }  // else: the layout is not what the census recorded -- redo the call the long way
+    out3[0] = ctx->h_result[0].s;
+    out3[1] = ctx->h_result[0].s2;
+    out3[2] = ctx->h_result[1].s;
+    // The flag (folded with max: every rank of a sharded vector sees it) says the layout holds a group of more than 256
+    // elements after all -- it was rewritten after validation.  The kernel has written every other group; the
+    // long-group kernels take the rest, every class treated as present, and their sums are added to these.
+    if (ctx->h_result[0].bad > 0) {
+      int total = 0;
+      st = launch_step_groupl2<R>(ctx, false, 3u, s, xsy, xk, sj, grad, ngroups, offs, lambda_g, (R)nu, &total);
+      if (st == SPX_OK) st = finalize_partials(ctx, total, 2, false);
+      if (st != SPX_OK) return st;
+      out3[0] += ctx->h_result[0].s;
+      out3[1] += ctx->h_result[0].s2;
+      out3[2] += ctx->h_result[1].s;
+    }
+  } else {
+    // every other layout: the size classes the census records (all of them for a layout never validated)
+    int total = 0;
+    st = launch_step_groupl2<R>(ctx, true, census ? census->classes & 3u : 3u, s, xsy, xk, sj, grad, ngroups, offs,
+                                lambda_g, (R)nu, &total);
+    if (st == SPX_OK) st = finalize_partials(ctx, total, 2, false);
+    if (st != SPX_OK) return st;
+    out3[0] = ctx->h_result[0].s;
+    out3[1] = ctx->h_result[0].s2;
+    out3[2] = ctx->h_result[1].s;
   }
-  return step_composed<R>(ctx, n, s, xsy, xk, sj, grad, nu, [&](double* psi) {
-    return prox_group<R>(ctx, false, n, s, xk, sj, s, ngroups, offs, lambda_g, nu, 0.0, psi);
-  }, out3);
+  out3[0] = (double)(R)out3[0];  // the reference accumulates ψ in R: one rounding to R
+  return SPX_OK;
 }
 
 // ---- the solver step of ShiftedGroupNormL2Binf ---------------------------------------------------------------------

@@ -394,6 +394,30 @@ int32_t step_l1b2_finish(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, con
   return SPX_OK;
 }
 
+// The scaling pass of the ShiftedGroupNormL2 step on a single group spanning the vector (spx_group.cu): s = (zero ? 0 :
+// α sol) - (xk + sj) with sol = (q + xk) + sj, q = (-ν)∇f, xsy = (xk + sj) + s (xsy may be NULL), and
+// v = {Σ(xk + sj + s)², Σ∇f·s, Σs²}.
+template <class R>
+int32_t step_group_scale(spx_ctx* ctx, int64_t n, R* s, R* xsy, const R* xk, const R* sj, const R* grad, R nu, R alpha,
+                         bool zero, double* v) {
+  SolScaleStep<R> op;
+  op.in[0] = xk; op.in[1] = sj; op.in[2] = grad;
+  op.fill[0] = op.fill[1] = op.fill[2] = R(0);
+  op.y = s;
+  op.alpha = alpha;
+  op.zero = zero;
+  int32_t st = step_launch<false>(ctx, op, -nu, xsy, n);
+  if (st != SPX_OK) return st;
+  v[0] = ctx->h_result[0].s2;
+  v[1] = ctx->h_result[1].s;
+  v[2] = ctx->h_result[1].s2;
+  return SPX_OK;
+}
+
+template int32_t step_group_scale<double>(spx_ctx*, int64_t, double*, double*, const double*, const double*, const double*,
+                                          double, double, bool, double*);
+template int32_t step_group_scale<float>(spx_ctx*, int64_t, float*, float*, const float*, const float*, const float*,
+                                         float, float, bool, double*);
 template int32_t step_l1b2_finish<double>(spx_ctx*, int64_t, double*, double*, const double*, const double*,
                                           const double*, const double*, double, double, bool, double, double, double*);
 template int32_t step_l1b2_finish<float>(spx_ctx*, int64_t, float*, float*, const float*, const float*, const float*,

@@ -695,8 +695,8 @@ class ShiftedGroupNormL2(_GroupBase):
         return out.value
 
     def step_(self, s, grad, nu, xsy=None):
-        """spx_step_groupl2_*: the whole step in one pass when every group holds <= 256 elements (the C4 shape), the
-        two passes around prox! otherwise (decided in the library from the census of the validated layout)."""
+        """spx_step_groupl2_*: the whole step inside the passes of prox!'s own kernels on every layout -- one pass per
+        group of any size, two grid-wide passes for a single group spanning the vector (ψ built from NormL2)."""
         return self._lib_step("step_groupl2", (C.c_int64(self.n),), s, grad, xsy,
                               (C.c_int64(self.ngroups), _p(self._offs), _p(self._lam_g), C.c_double(nu)))
 

@@ -86,6 +86,24 @@ def main():
         print(f"{name:34s} {ms:9.3f} ms  {r['elements_per_s']:.3e} el/s  {gbs:8.1f} GB/s  "
               f"{100 * gbs / peak:5.1f}% of measured {peak:.0f}  {note}", flush=True)
 
+    def step_pair(name, psi, composed_transits, note):
+        # spx_step_groupl2 (5 vector transits; 8 on one group) against ShiftedProximableFunction.step_ of the same ψ:
+        # first whether both give the same s and xsy bit for bit, then both timed, alternated three times (q plays ∇f)
+        xsy_a, s_b, xsy_b = torch.empty_like(y), torch.empty_like(y), torch.empty_like(y)
+        _, r = sp.step_(y, psi, q, 0.3, xsy=xsy_a)
+        _, r2 = sp.ShiftedProximableFunction.step_(psi, s_b, q, 0.3, xsy=xsy_b)
+        same = torch.equal(y, s_b) and torch.equal(xsy_a, xsy_b)
+        print(f"{name} vs composed: s and xsy bit-identical: {same}; scalars {tuple(r)} vs {tuple(r2)}", flush=True)
+        del s_b, xsy_b
+        fused = 8 if name.endswith("_one") else 5
+        for _ in range(3):
+            timeit(name, lambda: sp.step_(y, psi, q, 0.3, xsy=xsy_a), fused * R,
+                   note=f"spx_step_groupl2, {note}; alg. bytes = {fused} transits")
+            timeit(f"{name}_composed", lambda: sp.ShiftedProximableFunction.step_(psi, y, q, 0.3, xsy=xsy_a),
+                   fused * R, note=f"step_pre, prox! in place + ψ, step_post ({composed_transits} transits); "
+                                  "alg. bytes as above")
+        del xsy_a
+
     def two(h, *a, **k):
         return sp.shifted(sp.shifted(h, xk, *a, **k), sj)
 
@@ -220,7 +238,8 @@ def main():
     for gname in ("g64", "ragged"):
         names = [f"prox_groupl2_{gname}", f"value_groupl2_{gname}", f"prox_groupl2binf_{gname}",
                  "prox_groupl2binf_g64_biglambda", "step_groupl2_g64", "step_groupl2binf_g64",
-                 "step_groupl2binf_g64_composed", "step_groupl2binf_g64_biglambda"]
+                 "step_groupl2binf_g64_composed", "step_groupl2binf_g64_biglambda", "step_groupl2_ragged",
+                 "step_groupl2_ragged_composed"]
         if not any(re.search(args.only, nm) for nm in names):
             continue
         if gname == "g64":
@@ -245,6 +264,11 @@ def main():
             timeit("step_groupl2_g64", lambda psi=psi: sp.step_(y, psi, q, 0.3, xsy=xsy_g), 5 * R,
                    note="spx_step_groupl2: one pass on this layout (groups <= 256); alg. bytes = 3 reads + 2 writes")
             del xsy_g
+        # the step on the ragged layout (groups of 1..4096: every size class) against the base-class composition of
+        # the same ψ (spx_step_pre, prox! in place with ψ, spx_step_post), alternated three times
+        if gname == "ragged" and any(re.search(args.only, nm) for nm in ("step_groupl2_ragged",
+                                                                            "step_groupl2_ragged_composed")):
+            step_pair("step_groupl2_ragged", psi, 11, f"{ng} groups")
         psib = sp.shifted(sp.shifted(h, xk, 0.5, sp.NormLinf(1.0)), sj)
         timeit(f"prox_groupl2binf_{gname}", lambda psi=psib: sp.prox_(y, psi, q, 0.3), 4 * R, note=f"{ng} groups")
         if gname == "g64":  # σλ_g >> ||sol_g||: the regime of a sparse solution (root next to the pole of c(n) at σλ)
@@ -272,6 +296,11 @@ def main():
                 timeit("step_groupl2binf_g64_biglambda", lambda: sp.step_(y, psil, q, 0.3, xsy=xsy_b), 5 * R,
                        note="lambda_g x 200")
                 del xsy_b
+    # the step on one group spanning the vector (ShiftedGroupNormL2 built from NormL2): norm pass (3R) and scaling
+    # pass (3R+2W) against the composition (step_pre 1R+1W, the prox!'s norm pass 3R and scaling pass 3R+1W with ψ,
+    # step_post 4R+1W), alternated three times
+    if any(re.search(args.only, nm) for nm in ("step_groupl2_one", "step_groupl2_one_composed")):
+        step_pair("step_groupl2_one", sp.shifted(sp.shifted(sp.NormL2(lam), xk), sj), 14, "one group")
     # top-r batch: problems of 65536, r = 1024
     if any(re.search(args.only, nm) for nm in ("prox_indballl0_batch", "prox_indballl0binf_batch", "prox_indballl0_single")):
         pn = 65536
