@@ -29,6 +29,80 @@ template <class Op> struct MinBlocks<Op, std::void_t<decltype(Op::MINB)>> { stat
 template <class Op, class = void> struct SplitNull { static constexpr bool value = false; };
 template <class Op> struct SplitNull<Op, std::void_t<decltype(Op::SPLIT_NULL)>> { static constexpr bool value = Op::SPLIT_NULL; };
 
+// Operators that declare `static constexpr bool PACKET = true` (and `int PREFETCH, L2_AHEAD`) are applied one 128-bit
+// packet at a time in the vector launches, in four parts (see ProxLhalfBox):
+//   bool selects_all()                       every element selected: the loop then holds no selection test at all
+//   bool pick_packet(x, o, hard)             the common path: o for every element, true if some element needs the slow path
+//   void exact_packet(x, o, hard)            the slow path, only when pick_packet returned true
+//   Pack finish_packet<ALL>(x, o, i0, acc)   the selection and the ψ terms
+// After the slow path the packet is loaded again rather than held across it: held, it pushes the common path's registers
+// to the stack.  With PREFETCH = 1 each thread also issues the loads of its next packet before it computes the
+// current one (NIN x 16 bytes more in registers).  With L2_AHEAD = k > 0 it asks L2 for the lines of its packet k
+// iterations ahead (`prefetch.global.L2`: no register, no shared memory), so its own loads later hit L2.
+template <class Op, class = void> struct Packet { static constexpr bool value = false; };
+template <class Op> struct Packet<Op, std::void_t<decltype(Op::PACKET)>> { static constexpr bool value = Op::PACKET; };
+
+template <int VEC, int NPTR, class Op>
+__device__ __forceinline__ void ew_load_packet(const Op& op, long long v, long long nvec,
+                                               Pack<typename Op::Real, VEC> (&x)[Op::NIN]) {
+#pragma unroll
+  for (int k = 0; k < Op::NIN; ++k) {
+    if (NPTR >= 0) {
+      if (k < NPTR) {
+        if (v < nvec) ld_stream(op.in[k] + v * VEC, x[k]);  // past the end: never used
+      } else {
+#pragma unroll
+        for (int e = 0; e < VEC; ++e) x[k].v[e] = op.fill[k];
+      }
+    } else if (op.in[k] != nullptr && v < nvec) {
+      ld_stream(op.in[k] + v * VEC, x[k]);
+    } else {
+#pragma unroll
+      for (int e = 0; e < VEC; ++e) x[k].v[e] = op.fill[k];
+    }
+  }
+}
+
+__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
+
+template <int VEC, int NPTR, bool ALL, class Op>
+__device__ __forceinline__ void ew_packet_loop(const Op& op, long long nvec, long long index_base, Partial& acc) {
+  using R = typename Op::Real;
+  const long long stride = (long long)gridDim.x * kEwThreads;
+  long long v = (long long)blockIdx.x * kEwThreads + threadIdx.x;
+  Pack<R, VEC> x[Op::NIN];
+  if (Op::PREFETCH > 0) ew_load_packet<VEC, NPTR>(op, v, nvec, x);
+  for (; v < nvec; v += stride) {
+    if (Op::L2_AHEAD > 0) {
+      const long long va = v + Op::L2_AHEAD * stride;
+      if (va < nvec) {
+#pragma unroll
+        for (int k = 0; k < Op::NIN; ++k)
+          if (NPTR >= 0 ? k < NPTR : op.in[k] != nullptr) prefetch_l2(op.in[k] + va * VEC);
+      }
+    }
+    Pack<R, VEC> nx[Op::NIN];
+    if (Op::PREFETCH > 0)
+      ew_load_packet<VEC, NPTR>(op, v + stride, nvec, nx);
+    else
+      ew_load_packet<VEC, NPTR>(op, v, nvec, x);
+    Pack<R, VEC> o;
+    bool hard[VEC];
+    if (op.pick_packet(x, o, hard)) {
+      op.exact_packet(x, o, hard);
+      // the same bytes: this thread stores packet v below and packet v + stride in its next iteration (y may alias q)
+      ew_load_packet<VEC, NPTR>(op, v, nvec, x);
+      if (Op::PREFETCH > 0) ew_load_packet<VEC, NPTR>(op, v + stride, nvec, nx);
+    }
+    const Pack<R, VEC> out = op.template finish_packet<ALL>(x, o, index_base + v * VEC, acc);
+    if (Op::OUT) st_stream(op.y + v * VEC, out);
+    if (Op::PREFETCH > 0) {
+#pragma unroll
+      for (int k = 0; k < Op::NIN; ++k) x[k] = nx[k];
+    }
+  }
+}
+
 template <int VEC, int UNROLL, class Op, int NPTR = -1>
 __global__ void __launch_bounds__(kEwThreads, MinBlocks<Op>::value)
     ew_kernel(const Op op, const long long n, const long long index_base, Partial* __restrict__ partials) {
@@ -41,41 +115,49 @@ __global__ void __launch_bounds__(kEwThreads, MinBlocks<Op>::value)
 
   const long long nvec = n / VEC;
   const long long tile = (long long)kEwThreads * UNROLL;
-  for (long long base = (long long)blockIdx.x * tile; base < nvec; base += (long long)gridDim.x * tile) {
-    Pack<R, VEC> reg[NIN][UNROLL];
+  if constexpr (Packet<Op>::value && VEC > 1) {
+    static_assert(UNROLL == 1, "the packet loop strides by one packet per thread");
+    if (op.selects_all())
+      ew_packet_loop<VEC, NPTR, true>(op, nvec, index_base, acc);
+    else
+      ew_packet_loop<VEC, NPTR, false>(op, nvec, index_base, acc);
+  } else {
+    for (long long base = (long long)blockIdx.x * tile; base < nvec; base += (long long)gridDim.x * tile) {
+      Pack<R, VEC> reg[NIN][UNROLL];
 #pragma unroll
-    for (int u = 0; u < UNROLL; ++u) {
-      const long long v = base + (long long)u * kEwThreads + threadIdx.x;
+      for (int u = 0; u < UNROLL; ++u) {
+        const long long v = base + (long long)u * kEwThreads + threadIdx.x;
 #pragma unroll
-      for (int k = 0; k < NIN; ++k) {
-        if (NPTR >= 0) {  // vector-ness known at compile time: no fill moves, no null tests
-          if (k < NPTR) {
-            if (v < nvec) ld_stream(op.in[k] + v * VEC, reg[k][u]);  // past the end: never used below
+        for (int k = 0; k < NIN; ++k) {
+          if (NPTR >= 0) {  // vector-ness known at compile time: no fill moves, no null tests
+            if (k < NPTR) {
+              if (v < nvec) ld_stream(op.in[k] + v * VEC, reg[k][u]);  // past the end: never used below
+            } else {
+#pragma unroll
+              for (int e = 0; e < VEC; ++e) reg[k][u].v[e] = op.fill[k];
+            }
+          } else if (op.in[k] != nullptr && v < nvec) {  // one predicate: keeps every load of the tile in one batch
+            ld_stream(op.in[k] + v * VEC, reg[k][u]);
           } else {
 #pragma unroll
             for (int e = 0; e < VEC; ++e) reg[k][u].v[e] = op.fill[k];
           }
-        } else if (op.in[k] != nullptr && v < nvec) {  // one predicate: keeps every load of the tile in one batch
-          ld_stream(op.in[k] + v * VEC, reg[k][u]);
-        } else {
-#pragma unroll
-          for (int e = 0; e < VEC; ++e) reg[k][u].v[e] = op.fill[k];
         }
       }
-    }
 #pragma unroll
-    for (int u = 0; u < UNROLL; ++u) {
-      const long long v = base + (long long)u * kEwThreads + threadIdx.x;
-      if (v < nvec) {
-        Pack<R, VEC> out;
+      for (int u = 0; u < UNROLL; ++u) {
+        const long long v = base + (long long)u * kEwThreads + threadIdx.x;
+        if (v < nvec) {
+          Pack<R, VEC> out;
 #pragma unroll
-        for (int e = 0; e < VEC; ++e) {
-          R x[NIN];
+          for (int e = 0; e < VEC; ++e) {
+            R x[NIN];
 #pragma unroll
-          for (int k = 0; k < NIN; ++k) x[k] = reg[k][u].v[e];
-          out.v[e] = op.apply(x, index_base + v * VEC + e, acc);
+            for (int k = 0; k < NIN; ++k) x[k] = reg[k][u].v[e];
+            out.v[e] = op.apply(x, index_base + v * VEC + e, acc);
+          }
+          if (Op::OUT) st_stream(op.y + v * VEC, out);
         }
-        if (Op::OUT) st_stream(op.y + v * VEC, out);
       }
     }
   }
